@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the calibration hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], the configuration the metric "calib images/sec (hist+KL)"
@@ -33,6 +33,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -121,6 +122,7 @@ class ClockSampler:
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait()
         self.thread.join(timeout=2)
         sm, mx, reasons, power = [], [], set(), []
         for r in self.rows[self.first:] or self.rows:
@@ -227,7 +229,7 @@ def ours(args):
     torch.backends.cudnn.benchmark = os.environ.get("PQ_BENCH_NO_AUTOTUNE") != "1"   # off under ncu
     _native.lib()
     net = build_model()
-    workdir = os.path.join("/tmp", "pq_bench_rank%d" % rank)
+    workdir = tempfile.mkdtemp(prefix="pq_bench_rank%d_" % rank)
     K, W = args.steps, max(args.warmup, 3)
 
     # warm-up: W steps through the same job shape (cuDNN autotune, allocator, kernels)
@@ -253,14 +255,18 @@ def ours(args):
     l0 = _native.LAUNCHES["total"]
     if rank == 0:
         sampler.mark()
-    secs, q = run_job(net, ShardedBatches(dev_batches, K * world, rank, world), K * world, workdir, rank, world)
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        secs, q = run_job(net, ShardedBatches(dev_batches, K * world, rank, world), K * world, workdir, rank, world)
+    finally:                               # nvidia-smi must not outlive a failed run
+        clocks = sampler.stop() if rank == 0 else None
     launches = _native.LAUNCHES["total"] - l0
     _native.set_profile(None)
     torch.cuda.synchronize()
     value = world * K * MICRO_BATCH / secs
     timings = dict(q.timings)
     bits_image = q.last_calibration["bits"]["image"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, q.last_calibration)
     del dev_batches
 
     def kernel_stats(name):
@@ -331,6 +337,18 @@ def ours(args):
         torch.distributed.destroy_process_group()
     return line
 
+
+
+def dump_outputs(out_dir, cal):
+    """What the timed job hands its caller (Quantity.last_calibration after the merge over ranks), as float64 arrays
+    whose rows follow the observed tensors in forward order ("image" first): <key>.npy of shape [71] for the
+    per-tensor scalars and distributions.npy of shape [71, 2048] for the histograms."""
+    os.makedirs(out_dir, exist_ok=True)
+    names = cal["top_feat_names"]
+    for key in ("max_vals", "intervals", "thresholds", "threshold_bins", "bits"):
+        np.save(os.path.join(out_dir, key + ".npy"), np.array([float(cal[key][n]) for n in names], np.float64))
+    np.save(os.path.join(out_dir, "distributions.npy"),
+            np.stack([np.asarray(cal["distributions"][n], np.float64) for n in names]))
 
 
 # ------------------------------------------------------------------------ extras (after the timed region)
@@ -691,13 +709,26 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=8)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip c3_full / recontest / reconmodel / c1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed job computed as DIR/<name>.npy (float64; the "
+                         "inputs are seeded, so two builds can be compared output for output).  cuDNN autotuning "
+                         "may pick other fp32 convolutions from run to run, which moves maxima and histograms in "
+                         "the last bits; PQ_BENCH_NO_AUTOTUNE=1 turns it off, so that cuDNN's heuristics choose "
+                         "the algorithms")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     # the drop-in classes print progress like the reference does; keep stdout to the ONE JSON line
     real_stdout = sys.stdout
     sys.stdout = sys.stderr
     try:
-        line = reference_arm(args) if args.impl == "reference" else ours(args)
+        with tempfile.TemporaryDirectory(prefix="pq_bench_") as tmp:
+            tempfile.tempdir = tmp          # every work directory of the run lives here and goes with it
+            line = reference_arm(args) if args.impl == "reference" else ours(args)
     finally:
+        tempfile.tempdir = None
         sys.stdout = real_stdout
     if line is not None:
         print(json.dumps(line), flush=True)
