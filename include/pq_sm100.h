@@ -34,6 +34,10 @@ extern "C" {
 
 typedef void *pq_stream_t; /* cudaStream_t */
 
+/* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
+ * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
+#define PQ_VERSION 200
+
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
 #define PQ_EUNSUPPORTED (-2) /* shape / alignment the kernels do not implement */
@@ -46,7 +50,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 #define PQ_KL_CANDIDATES (PQ_HIST_BINS - PQ_KL_TARGET_BIN)
 #define PQ_MAX_SEGMENTS 256 /* tensors per multi-tensor launch */
 
-int pq_version(void);
+int pq_version(void); /* PQ_VERSION */
 const char *pq_error_string(int code);
 
 /* ---- a1: DistributionCollector.refresh_max_val, common/quantity/distribution_collector.py:70-78
@@ -143,7 +147,7 @@ int pq_quantize_im2col_s8(const float *x, int8_t *a, int N, int C, int H, int W,
  * desc.C must be 8; weights are [K][R][64] int8 = 8 tap slots x 8 channel slots per filter row, zero
  * where s >= S or c >= C.  Requires S <= 8, even stride_w, Hp % stride_h == 0,
  * Hp >= max((P-1)*stride_h + R, H + pad_h), Wp even, Wp >= max((Q-1)*stride_w + 8, W + pad_w).
- * Epilogue and outputs as pq_conv2d_s8_ex. */
+ * desc.dil_h / dil_w must be 1 (else PQ_EUNSUPPORTED).  Epilogue, flags and outputs as pq_conv2d_s8. */
 int pq_quantize_nchw_to_padded_nhwc8_s8(const float *x, int8_t *q, int N, int C, int H, int W, int pad_h,
                                         int pad_w, int Hp, int Wp, int ib, pq_stream_t stream);
 
@@ -156,27 +160,28 @@ int pq_quantize_nchw_to_padded_nhwc8_s8(const float *x, int8_t *q, int N, int C,
  * pq_gemm_s8: a is [M][K] row-major int8 (NHWC activations of a 1x1/stride-1 conv, or the
  * input of a Linear), w is [N][K] row-major int8, K % 16 == 0, 16-byte aligned rows.
  * Outputs (either may be NULL): out_f32 written as NCHW fp32 with `hw` pixels per image
- * (hw = 1 gives the plain [M][N] row-major layout of a Linear); out_s8 written [M][N]. */
+ * (hw = 1 gives the plain [M][N] row-major layout of a Linear); out_s8 written [M][N].
+ * pq_conv2d_s8: the same on an NHWC image, filter tap (r, s) reading input pixel
+ * (p*stride_h - pad_h + r*dil_h, q*stride_w - pad_w + s*dil_w).  Dilated filters (nn.Conv2d(dilation=...) wrapped by
+ * NewConv2d; the reference's weight path zero-stuffs such kernels for its target hardware,
+ * tools/pytorch_quantizer.py:626-629,679-693) take the im2col-TMA path with the dilation as tap offsets, so no
+ * multiply is wasted on stuffed zeros; a 1x1 filter ignores the dilation. */
 typedef struct pq_conv_desc {
     int N, H, W, C;          /* input NHWC, C = padded channel count (multiple of 16) */
     int K;                   /* output channels */
     int R, S;                /* filter height / width; weights are [K][R][S][C] int8 */
     int stride_h, stride_w, pad_h, pad_w;
-    int P, Q;                /* output height / width */
+    int P, Q;                /* output height / width: (H + 2*pad_h - ((R-1)*dil_h + 1)) / stride_h + 1, Q alike */
     int rs;                  /* weight_bit + input_bit - output_bit, any sign */
     int ob;                  /* output_bit */
+    int dil_h, dil_w;        /* dilation, >= 1 */
 } pq_conv_desc;
 
-int pq_gemm_s8(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K,
-               int rs, int ob, int hw, float *out_f32, int8_t *out_s8, pq_stream_t stream);
-int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                 const pq_conv_desc *desc_host, float *out_f32_nchw, int8_t *out_s8_nhwc,
-                 pq_stream_t stream);
-
-/* ---- SURVEY 8(f) n1, the int8 inter-layer pipeline (no reference counterpart as separate ops; the
- * composition is bit-identical to the reference's fp32-boundary chain because a layer's input_bit is
- * its producer's output_bit in feat.table, tools/pytorch_quantizer.py:468-485).
- * PQ_FLAG_RELU fuses a following nn.ReLU into the GEMM / conv epilogue: y = max(y, 0). */
+/* flags of the GEMM / conv entry points (0: the layer as above).
+ * PQ_FLAG_RELU fuses a following nn.ReLU into the GEMM / conv epilogue: y = max(y, 0).  It serves SURVEY 8(f) n1, the
+ * int8 inter-layer pipeline (no reference counterpart as separate ops; the composition is bit-identical to the
+ * reference's fp32-boundary chain because a layer's input_bit is its producer's output_bit in feat.table,
+ * tools/pytorch_quantizer.py:468-485). */
 #define PQ_FLAG_RELU 1
 /* PQ_FLAG_BIAS_FOLDED: bias_q points to int32 [3][N] written by pq_bias_fold_s32 for the SAME rs (N % 16 == 0):
  *   [0] bias   [1] 2^(rs-1) + (bias << rs)
@@ -189,26 +194,17 @@ int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias
  * (the composition Sp(Sp(r) + b) is monotone in r and constant beyond the int8 range of r).  Same integers either way.
  * Ignored unless 1 <= rs <= 20 and N % 16 == 0. */
 #define PQ_FLAG_BIAS_FOLDED 2
-/* PQ_FLAG_NO_WINDOWS (pq_conv2d_s8_ex): take the im2col-TMA path even where the patch-window path applies (3x3,
+/* PQ_FLAG_NO_WINDOWS (conv only): take the im2col-TMA path even where the patch-window path applies (3x3,
  * stride 1, pad 1, C = 64 / 128, one tile of output channels); both are bit-identical, the flag exists for A/B tests. */
 #define PQ_FLAG_NO_WINDOWS 4
+
+int pq_gemm_s8(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs, int ob, int hw,
+               int flags, float *out_f32, int8_t *out_s8, pq_stream_t stream);
+int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
+                 int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, pq_stream_t stream);
+
 /* out: int32 [3 * n] (rows [0], [1], [2] above; n even). */
 int pq_bias_fold_s32(const int32_t *bias_q, int n, int rs, int32_t *out, pq_stream_t stream);
-int pq_gemm_s8_ex(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs,
-                  int ob, int hw, int flags, float *out_f32, int8_t *out_s8, pq_stream_t stream);
-int pq_conv2d_s8_ex(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                    const pq_conv_desc *desc_host, int flags, float *out_f32_nchw, int8_t *out_s8_nhwc,
-                    pq_stream_t stream);
-
-/* Dilated convolution (nn.Conv2d(dilation=...) wrapped by NewConv2d, new_quantity_op.py:104-133; the reference's
- * weight path zero-stuffs such kernels for its target hardware, tools/pytorch_quantizer.py:626-629,679-693).
- * Same contract as pq_conv2d_s8_ex with filter tap (r, s) reading input pixel
- * (p*stride_h - pad_h + r*dil_h, q*stride_w - pad_w + s*dil_w); desc->P / Q must be the dilated output size
- * (H + 2*pad_h - ((R-1)*dil_h + 1)) / stride_h + 1.  The taps are im2col-TMA offsets, so no multiply is wasted
- * on stuffed zeros.  A 1x1 filter ignores the dilation. */
-int pq_conv2d_s8_dil(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                     const pq_conv_desc *desc_host, int dil_h, int dil_w, int flags, float *out_f32_nchw,
-                     int8_t *out_s8_nhwc, pq_stream_t stream);
 
 /* Space-to-depth form of the same input for stride-2 convolutions with C <= 4: 2 x 2 pixel blocks of the zero-padded
  * image as 16-byte pixels, q[n][i][j][(dy * 2 + dx) * 4 + c] = Quantity(ib)(x[n][c][2i + dy - pad_t][2j + dx - pad_l])
@@ -243,14 +239,11 @@ int pq_maxpool_nhwc_s8(const int8_t *x, int8_t *y, int N, int H, int W, int C, i
  *                                                           a_relu / b_relu apply max(.,0) on load
  *   out16 = s * 2^o_bit (int16, o_bit = max(a_bit, b_bit), exact)      -> the identity shortcut of the next add
  *   out8  = clamp(round_half_even(s * 2^q_bit), -128, 127) (int8)      -> Quantity(q_bit) of the consuming convs
+ * flags & PQ_FLAG_RELU: the nn.ReLU that follows the Eltwise is applied to s before both outputs
+ * (max(.,0) commutes with the monotone quantiser, so out8 equals Quantity(q_bit)(relu(s))).
  * Either output may be NULL.  Requires 0 <= o_bit - min(a_bit, b_bit) <= 7 and |q_bit - o_bit| <= 15. */
 int pq_add_requant(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16, int b_bit,
-                   int b_relu, size_t n, int16_t *out16, int8_t *out8, int q_bit, pq_stream_t stream);
-/* flags & PQ_FLAG_RELU: the nn.ReLU that follows the Eltwise is applied to s before both outputs
- * (max(.,0) commutes with the monotone quantiser, so out8 equals Quantity(q_bit)(relu(s))). */
-int pq_add_requant_ex(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16, int b_bit,
-                      int b_relu, size_t n, int flags, int16_t *out16, int8_t *out8, int q_bit,
-                      pq_stream_t stream);
+                   int b_relu, size_t n, int flags, int16_t *out16, int8_t *out8, int q_bit, pq_stream_t stream);
 
 /* Concat (fabu_layer.py:14-20, left in place by tools/reconstruction.py:219-238) followed by the
  * consumer's input quantiser Quantity(q_bit) (new_quantity_op.py:48-58), on quantised operands: source i is
@@ -272,7 +265,7 @@ int pq_concat_requant_s8(const pq_concat_src *srcs_host, int k, size_t pixels, i
                          int8_t *out, pq_stream_t stream);
 
 /* NewConv2d + NewAdd (+ the nn.ReLU after the Eltwise) in ONE kernel: the conv / GEMM epilogue adds the
- * shortcut operand and writes the exact int16 sum and its int8 requantisation, exactly as pq_add_requant_ex
+ * shortcut operand and writes the exact int16 sum and its int8 requantisation, exactly as pq_add_requant
  * would on the conv's int8 result (which is never written to memory).  conv operand: y at bit `ob` of the
  * conv descriptor; shortcut: int8 or int16 [M][N] row-major (NHWC) at bit shortcut_bit.  N % 16 == 0. */
 typedef struct pq_add_desc {
@@ -283,14 +276,10 @@ typedef struct pq_add_desc {
     int16_t *out16;          /* exact sum at o_bit = max(ob, shortcut_bit); may be NULL */
     int8_t *out8;            /* required */
 } pq_add_desc;
-int pq_gemm_s8_add(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs, int ob,
-                   const pq_add_desc *add_host, pq_stream_t stream);
-int pq_conv2d_s8_add(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                     const pq_conv_desc *desc_host, const pq_add_desc *add_host, pq_stream_t stream);
-/* the same with flags: PQ_FLAG_BIAS_FOLDED (bias_q as written by pq_bias_fold_s32); PQ_FLAG_RELU is rejected
+/* flags: PQ_FLAG_BIAS_FOLDED (bias_q as written by pq_bias_fold_s32); PQ_FLAG_RELU is rejected with PQ_EINVAL
  * (the ReLU of a fused add is add_host->out_relu). */
-int pq_conv2d_s8_add_ex(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                        const pq_conv_desc *desc_host, const pq_add_desc *add_host, int flags, pq_stream_t stream);
+int pq_conv2d_s8_add(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
+                     const pq_add_desc *add_host, int flags, pq_stream_t stream);
 
 #ifdef __cplusplus
 }

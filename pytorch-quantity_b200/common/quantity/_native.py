@@ -19,6 +19,7 @@ HIST_BINS_MAX = 8192
 KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
+PQ_VERSION = 200             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -42,32 +43,26 @@ SYMBOLS = {
     "pq_quantize_nchw_to_padded_nhwc8_s8": (_i, [_vp, _vp] + [_i] * 9 + [_vp]),
     "pq_conv2d_smallc_s8": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "pq_quantize_nchw_to_s2d16_s8": (_i, [_vp, _vp] + [_i] * 9 + [_vp]),
-    "pq_gemm_s8": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
-    "pq_conv2d_s8": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "pq_gemm_s8_ex": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
-    "pq_conv2d_s8_ex": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
-    "pq_conv2d_s8_dil": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
-    "pq_gemm_s8_add": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp]),
-    "pq_conv2d_s8_add": (_i, [_vp, _vp, _vp, _vp, _vp, _vp]),
-    "pq_conv2d_s8_add_ex": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "pq_gemm_s8": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "pq_conv2d_s8": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "pq_conv2d_s8_add": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "pq_relu_s8": (_i, [_vp, _vp, _sz, _vp]),
     "pq_maxpool_nhwc_s8": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "pq_avgpool_global_nhwc_f32": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
-    "pq_add_requant": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _sz, _vp, _vp, _i, _vp]),
-    "pq_add_requant_ex": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _sz, _i, _vp, _vp, _i, _vp]),
+    "pq_add_requant": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _sz, _i, _vp, _vp, _i, _vp]),
     "pq_concat_requant_s8": (_i, [_vp, _i, _sz, _i, _i, _vp, _vp]),
     "pq_bias_fold_s32": (_i, [_vp, _i, _i, _vp, _vp]),
 }
 FLAG_RELU = 1
 FLAG_BIAS_FOLDED = 2
-FLAG_NO_WINDOWS = 4          # pq_conv2d_s8_ex: force the im2col-TMA path (A/B tests of the patch-window path)
+FLAG_NO_WINDOWS = 4          # pq_conv2d_s8: force the im2col-TMA path (A/B tests of the patch-window path)
 
 
 class ConvDesc(ctypes.Structure):
     """struct pq_conv_desc"""
     _fields_ = [(n, ctypes.c_int) for n in
                 ("N", "H", "W", "C", "K", "R", "S", "stride_h", "stride_w", "pad_h", "pad_w",
-                 "P", "Q", "rs", "ob")]
+                 "P", "Q", "rs", "ob", "dil_h", "dil_w")]
 
 
 class AddDesc(ctypes.Structure):
@@ -129,6 +124,11 @@ def lib():
                 "libpq_sm100.so not found at %s -- build it with `python __graft_entry__.py` "
                 "(or `make -C pytorch-quantity_b200/csrc`).  This package has no CPU fallback." % LIB_PATH)
         handle = ctypes.CDLL(LIB_PATH)
+        handle.pq_version.restype, handle.pq_version.argtypes = SYMBOLS["pq_version"]
+        if handle.pq_version() != PQ_VERSION:
+            raise ImportError(
+                "%s is version %d, this package needs %d -- rebuild with `python __graft_entry__.py`"
+                % (LIB_PATH, handle.pq_version(), PQ_VERSION))
         for name, (res, args) in SYMBOLS.items():
             fn = getattr(handle, name)          # AttributeError if the .so lacks a declared symbol
             fn.restype, fn.argtypes = res, args
@@ -252,6 +252,18 @@ def bias_fold(bias_i32, rs):
     return out
 
 
+def conv_out_size(in_hw, kernel, stride, padding, dilation=(1, 1)):
+    """(P, Q): output height and width of a convolution, as nn.Conv2d computes them."""
+    return ((in_hw[0] + 2 * padding[0] - (kernel[0] - 1) * dilation[0] - 1) // stride[0] + 1,
+            (in_hw[1] + 2 * padding[1] - (kernel[1] - 1) * dilation[1] - 1) // stride[1] + 1)
+
+
+def _conv_desc(N, H, W, C, K, kernel, stride, padding, rs, ob, dilation=(1, 1)):
+    P, Q = conv_out_size((H, W), kernel, stride, padding, dilation)
+    return ConvDesc(N, H, W, C, K, kernel[0], kernel[1], stride[0], stride[1], padding[0], padding[1], P, Q,
+                    int(rs), int(ob), dilation[0], dilation[1])
+
+
 def _bias_flags(bias_q, n, relu):
     return (FLAG_RELU if relu else 0) | (FLAG_BIAS_FOLDED if bias_q.numel() == 3 * n else 0)
 
@@ -317,8 +329,7 @@ def quantize_im2col_s8(x, ib, kernel, stride, padding, kp):
     xc = x.contiguous()
     N, C, H, W = xc.shape
     R, S = kernel
-    P = (H + 2 * padding[0] - R) // stride[0] + 1
-    Q = (W + 2 * padding[1] - S) // stride[1] + 1
+    P, Q = conv_out_size((H, W), kernel, stride, padding)
     a = torch.empty((N * P * Q, kp), dtype=torch.int8, device=x.device)
     with _Timed("quantize_s8", 1, xc.numel() * 4 + a.numel(), xc.device):
         check(lib().pq_quantize_im2col_s8(xc.data_ptr(), a.data_ptr(), N, C, H, W, R, S, stride[0], stride[1],
@@ -361,11 +372,9 @@ def conv2d_smallc_s8(xp, w_krs8, bias_q, in_hw, kernel, stride, padding, rs, ob,
     require_cuda(xp, "conv2d_smallc_s8")
     N, Hp, Wp, _ = xp.shape
     K = w_krs8.shape[0]
-    H, W = in_hw
     R, S = kernel
-    P = (H + 2 * padding[0] - R) // stride[0] + 1
-    Q = (W + 2 * padding[1] - S) // stride[1] + 1
-    d = ConvDesc(N, H, W, 8, K, R, S, stride[0], stride[1], padding[0], padding[1], P, Q, int(rs), int(ob))
+    d = _conv_desc(N, in_hw[0], in_hw[1], 8, K, kernel, stride, padding, rs, ob)
+    P, Q = d.P, d.Q
     out_f32 = torch.empty((N, K, P, Q), dtype=torch.float32, device=xp.device) if want_f32 else None
     out_s8 = torch.empty((N, P, Q, K), dtype=torch.int8, device=xp.device) if want_s8 else None
     with _Timed("conv_s8", 1, ops or 2 * N * P * Q * K * R * S * (c_real or 8), xp.device):        # int8 ops
@@ -387,9 +396,9 @@ def gemm_s8(a, w, bias_q, rs, ob, hw=1, want_f32=True, want_s8=False, k_real=Non
     if want_s8:
         out_s8 = torch.empty((M, N), dtype=torch.int8, device=a.device)
     with _Timed("gemm_s8", 1, 2 * M * N * (k_real or K), a.device):      # "bytes" field carries int8 ops here
-        check(lib().pq_gemm_s8_ex(a.data_ptr(), w.data_ptr(), bias_q.data_ptr(), M, N, K, int(rs), int(ob), hw,
-                                  _bias_flags(bias_q, N, relu), out_f32.data_ptr() if want_f32 else None,
-                                  out_s8.data_ptr() if want_s8 else None, _stream(a)), "pq_gemm_s8")
+        check(lib().pq_gemm_s8(a.data_ptr(), w.data_ptr(), bias_q.data_ptr(), M, N, K, int(rs), int(ob), hw,
+                               _bias_flags(bias_q, N, relu), out_f32.data_ptr() if want_f32 else None,
+                               out_s8.data_ptr() if want_s8 else None, _stream(a)), "pq_gemm_s8")
     return out_f32, out_s8
 
 
@@ -399,24 +408,16 @@ def conv2d_s8(x_nhwc, w_krsc, bias_q, stride, padding, rs, ob, want_f32=True, wa
     N, H, W, C = x_nhwc.shape
     K, R, S, C2 = w_krsc.shape
     assert C == C2
-    dh, dw = (int(dilation[0]), int(dilation[1])) if (R, S) != (1, 1) else (1, 1)
-    P = (H + 2 * padding[0] - ((R - 1) * dh + 1)) // stride[0] + 1
-    Q = (W + 2 * padding[1] - ((S - 1) * dw + 1)) // stride[1] + 1
-    d = ConvDesc(N, H, W, C, K, R, S, stride[0], stride[1], padding[0], padding[1], P, Q, int(rs), int(ob))
+    dilation = (int(dilation[0]), int(dilation[1])) if (R, S) != (1, 1) else (1, 1)
+    d = _conv_desc(N, H, W, C, K, (R, S), stride, padding, rs, ob, dilation)
+    P, Q = d.P, d.Q
     out_f32 = torch.empty((N, K, P, Q), dtype=torch.float32, device=x_nhwc.device) if want_f32 else None
     out_s8 = torch.empty((N, P, Q, K), dtype=torch.int8, device=x_nhwc.device) if want_s8 else None
     with _Timed("conv_s8", 1, 2 * N * P * Q * K * R * S * (c_real or C), x_nhwc.device):   # int8 ops
-        if (dh, dw) == (1, 1):
-            check(lib().pq_conv2d_s8_ex(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
-                                        _bias_flags(bias_q, K, relu) | (0 if windows else FLAG_NO_WINDOWS),
-                                        out_f32.data_ptr() if want_f32 else None,
-                                        out_s8.data_ptr() if want_s8 else None, _stream(x_nhwc)), "pq_conv2d_s8")
-        else:
-            check(lib().pq_conv2d_s8_dil(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
-                                         dh, dw, _bias_flags(bias_q, K, relu),
-                                         out_f32.data_ptr() if want_f32 else None,
-                                         out_s8.data_ptr() if want_s8 else None, _stream(x_nhwc)),
-                  "pq_conv2d_s8_dil (dilation %dx%d)" % (dh, dw))
+        check(lib().pq_conv2d_s8(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
+                                 _bias_flags(bias_q, K, relu) | (0 if windows else FLAG_NO_WINDOWS),
+                                 out_f32.data_ptr() if want_f32 else None,
+                                 out_s8.data_ptr() if want_s8 else None, _stream(x_nhwc)), "pq_conv2d_s8")
     return out_f32, out_s8
 
 
@@ -428,19 +429,18 @@ def conv2d_s8_add(x_nhwc, w_krsc, bias_q, stride, padding, rs, ob, shortcut, sho
     N, H, W, C = x_nhwc.shape
     K, R, S, C2 = w_krsc.shape
     assert C == C2
-    P = (H + 2 * padding[0] - R) // stride[0] + 1
-    Q = (W + 2 * padding[1] - S) // stride[1] + 1
+    d = _conv_desc(N, H, W, C, K, (R, S), stride, padding, rs, ob)
+    P, Q = d.P, d.Q
     assert tuple(shortcut.shape) == (N, P, Q, K) and shortcut.is_contiguous()
-    d = ConvDesc(N, H, W, C, K, R, S, stride[0], stride[1], padding[0], padding[1], P, Q, int(rs), int(ob))
     out16 = torch.empty((N, P, Q, K), dtype=torch.int16, device=x_nhwc.device) if want16 else None
     out8 = torch.empty((N, P, Q, K), dtype=torch.int8, device=x_nhwc.device)
     add = AddDesc(shortcut.data_ptr(), 1 if shortcut.dtype == torch.int16 else 0, int(shortcut_bit),
                   1 if shortcut_relu else 0, 1 if out_relu else 0, int(q_bit),
                   out16.data_ptr() if want16 else None, out8.data_ptr())
     with _Timed("conv_add_s8", 1, 2 * N * P * Q * K * R * S * (c_real or C), x_nhwc.device):        # int8 ops
-        check(lib().pq_conv2d_s8_add_ex(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
-                                        ctypes.byref(add), _bias_flags(bias_q, K, False), _stream(x_nhwc)),
-              "pq_conv2d_s8_add_ex")
+        check(lib().pq_conv2d_s8_add(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
+                                     ctypes.byref(add), _bias_flags(bias_q, K, False), _stream(x_nhwc)),
+              "pq_conv2d_s8_add")
     return out16, out8
 
 
@@ -456,8 +456,7 @@ def relu_s8(x):
 def maxpool_nhwc_s8(x, k, stride, pad, relu=False):
     require_cuda(x, "maxpool_nhwc_s8")
     N, H, W, C = x.shape
-    P = (H + 2 * pad - k) // stride + 1
-    Q = (W + 2 * pad - k) // stride + 1
+    P, Q = conv_out_size((H, W), (k, k), (stride, stride), (pad, pad))
     y = torch.empty((N, P, Q, C), dtype=torch.int8, device=x.device)
     with _Timed("maxpool_s8", 1, x.numel() + y.numel(), x.device):
         check(lib().pq_maxpool_nhwc_s8(x.data_ptr(), y.data_ptr(), N, H, W, C, k, stride, pad, 1 if relu else 0,
@@ -489,11 +488,11 @@ def add_requant(a, a_bit, a_relu, b, b_bit, b_relu, q_bit, want16=True, want8=Tr
     out8 = torch.empty(a.shape, dtype=torch.int8, device=a.device) if want8 else None
     nbytes = a.numel() * (a.element_size() + b.element_size() + (2 if want16 else 0) + (1 if want8 else 0))
     with _Timed("add_requant", 1, nbytes, a.device):
-        check(lib().pq_add_requant_ex(a.data_ptr(), 1 if a.dtype == torch.int16 else 0, int(a_bit),
-                                      1 if a_relu else 0, b.data_ptr(), 1 if b.dtype == torch.int16 else 0,
-                                      int(b_bit), 1 if b_relu else 0, a.numel(), FLAG_RELU if out_relu else 0,
-                                      out16.data_ptr() if want16 else None, out8.data_ptr() if want8 else None,
-                                      int(q_bit), _stream(a)), "pq_add_requant_ex")
+        check(lib().pq_add_requant(a.data_ptr(), 1 if a.dtype == torch.int16 else 0, int(a_bit),
+                                   1 if a_relu else 0, b.data_ptr(), 1 if b.dtype == torch.int16 else 0,
+                                   int(b_bit), 1 if b_relu else 0, a.numel(), FLAG_RELU if out_relu else 0,
+                                   out16.data_ptr() if want16 else None, out8.data_ptr() if want8 else None,
+                                   int(q_bit), _stream(a)), "pq_add_requant")
     return out16, out8
 
 

@@ -26,8 +26,8 @@ import torch.nn.functional as F
 from . import _native
 
 
-# NewConv2d + NewAdd (+ ReLU) in one kernel (pq_conv2d_s8_add_ex): the convolution's int8 result never touches
-# memory.  Bit-identical to conv followed by pq_add_requant_ex; on ResNet-50 batch 512 the 16 fused launches take
+# NewConv2d + NewAdd (+ ReLU) in one kernel (pq_conv2d_s8_add): the convolution's int8 result never touches
+# memory.  Bit-identical to conv followed by pq_add_requant; on ResNet-50 batch 512 the 16 fused launches take
 # 3.02 ms against 1.19 + 2.52 ms for the separate kernels (forward 6.83 -> 6.19 ms), so it is on by default.
 # PQ_FUSE_ADD=0 switches it off (A/B measurements).
 import os as _os
@@ -45,8 +45,8 @@ class _LazyConv:
     values, exactly like the fp32-boundary model.  If the only consumer is a NewAdd, the add (and the ReLU after
     it) can run inside the conv's epilogue and the conv result never touches memory."""
 
-    def __init__(self, mod, run, q=None):
-        self.mod, self.run, self.q = mod, run, q       # q: int8 NHWC operand (kept for the fused conv+add kernel)
+    def __init__(self, mod, operand):
+        self.mod, self.operand = mod, operand          # the NewConv2d and its operand (see NewConv2d._quantize)
         self.out = {}                                  # relu -> int8 NHWC payload
 
     def get(self, relu):
@@ -54,7 +54,7 @@ class _LazyConv:
             if relu and False in self.out:             # both asked for (rare): ReLU of the payload already there
                 self.out[True] = _native.relu_s8(self.out[False])
             else:
-                self.out[relu] = self.run(relu)
+                self.out[relu] = self.mod._run(self.operand, False, True, relu)[1]
         return self.out[relu]
 
 
@@ -78,8 +78,7 @@ class _LazyAdd:
     @staticmethod
     def _fusable(t):
         lc = t._lazy_conv
-        return FUSE_ADD_INTO_CONV and lc is not None and lc.q is not None and not lc.out and not t.relu_pending \
-            and lc.mod.Conv.out_channels % 16 == 0 and getattr(lc.mod, "_dilation", (1, 1)) == (1, 1)
+        return FUSE_ADD_INTO_CONV and lc is not None and lc.mod._fuses_add and not lc.out and not t.relu_pending
 
     def get(self, relu, kind):
         """kind: "s16" (exact sum) or "q8" (Quantity(q_bit) of it).  Returns the dict of payloads held."""
@@ -96,11 +95,8 @@ class _LazyAdd:
                 x, y = y, x
             if self._fusable(x):                       # conv + add (+ relu) in one kernel (always writes int8)
                 lc = x._lazy_conv
-                mod, conv = lc.mod, lc.mod.Conv
                 sc, sc_bit, sc_relu = _operand(y)
-                s16, q8 = _native.conv2d_s8_add(lc.q, mod._w_krsc, mod._bias_i32, conv.stride, conv.padding,
-                                                mod.rs_bit, mod.output_bit, sc, sc_bit, sc_relu, self.q_bit,
-                                                relu, want16=want16, c_real=conv.in_channels)
+                s16, q8 = lc.mod._run_add(lc.operand, sc, sc_bit, sc_relu, self.q_bit, relu, want16)
             else:
                 (a, abit, arelu), (b, bbit, brelu) = _operand(x), _operand(y)
                 s16, q8 = _native.add_requant(a, abit, arelu, b, bbit, brelu, self.q_bit, want16=want16,
@@ -339,57 +335,24 @@ def _avgpool(x, kernel_size, stride=None, padding=0, ceil_mode=False, count_incl
 
 
 def conv_forward(mod, x):
-    """NewConv2d.forward in pipeline mode."""
-    conv = mod.Conv
-    cat = isinstance(x, QTensor) and x._lazy_cat is not None
-    if cat:
-        usable = (not mod._explicit_im2col and not getattr(mod, "_smallc", False)
-                  and x.channels <= mod._c_pad and x._lazy_cat.supported(mod.input_bit))
-        if not usable:
+    """NewConv2d.forward in pipeline mode: the operand is the producer's int8 payload, the lazy concatenation at this
+    layer's input bit, or else the layer's own quantiser applied to the de-quantised input."""
+    c = mod._payload_channels
+    operand = None
+    if isinstance(x, QTensor):
+        if x._lazy_cat is not None:
+            if c is not None and x.channels <= c and x._lazy_cat.supported(mod.input_bit):
+                operand = x._lazy_cat.get(mod.input_bit, c, x.relu_pending and not x.nonneg)  # Concat + Quantity(ib)
+        elif c is not None and x.has_q8() and x.q8_bit == mod.input_bit and x.channels == c:
+            operand = x.int8_payload()                           # Quantity(ib) is the identity here
+    if operand is None:
+        if isinstance(x, QTensor):
             x = x.dequantize()
-    elif isinstance(x, QTensor):
-        usable = (not mod._explicit_im2col and not getattr(mod, "_smallc", False) and x.has_q8()
-                  and x.q8_bit == mod.input_bit and x.channels == mod._c_pad)
-        if not usable:
-            x = x.dequantize()
-    if isinstance(x, QTensor) and cat:
-        q = x._lazy_cat.get(mod.input_bit, mod._c_pad, x.relu_pending and not x.nonneg)   # Concat + Quantity(ib)
-    elif isinstance(x, QTensor):
-        q = x.int8_payload()                                     # Quantity(ib) is the identity here
-    elif getattr(mod, "_smallc", False):
-        N, _, H, W = x.shape
-        (R, S), (sh, sw), (ph, pw) = conv.kernel_size, conv.stride, conv.padding
-        P, Q = (H + 2 * ph - R) // sh + 1, (W + 2 * pw - S) // sw + 1
-
-        def run_smallc(relu, x=x):
-            return mod._smallc_forward(x, want_f32=False, want_s8=True, relu=relu)[1]
-        return QTensor((N, conv.out_channels, P, Q), x.device, q8_bit=mod.output_bit,
-                       lazy_conv=_LazyConv(mod, run_smallc))
-    elif mod._explicit_im2col:
-        a, (N, P, Q) = _native.quantize_im2col_s8(x, mod.input_bit, conv.kernel_size, conv.stride,
-                                                  conv.padding, mod._k_pad)
-
-        def run_gemm(relu, a=a):
-            _, out8 = _native.gemm_s8(a, mod._w_nk, mod._bias_i32, mod.rs_bit, mod.output_bit, hw=1,
-                                      want_f32=False, want_s8=True, relu=relu,
-                                      k_real=conv.in_channels * conv.kernel_size[0] * conv.kernel_size[1])
-            return out8.view(N, P, Q, conv.out_channels)
-        return QTensor((N, conv.out_channels, P, Q), a.device, q8_bit=mod.output_bit,
-                       lazy_conv=_LazyConv(mod, run_gemm))
+        operand, device = mod._quantize(x), x.device
     else:
-        q = _native.quantize_nchw_to_nhwc_s8(x, mod.input_bit, mod._c_pad)
-    N, H, W, _ = q.shape
-    (R, S), (sh, sw), (ph, pw) = conv.kernel_size, conv.stride, conv.padding
-    dh, dw = getattr(mod, "_dilation", (1, 1))
-    P, Q = (H + 2 * ph - ((R - 1) * dh + 1)) // sh + 1, (W + 2 * pw - ((S - 1) * dw + 1)) // sw + 1
-
-    def run_conv(relu, q=q):
-        return _native.conv2d_s8(q, mod._w_krsc, mod._bias_i32, conv.stride, conv.padding, mod.rs_bit,
-                                 mod.output_bit, want_f32=False, want_s8=True, c_real=conv.in_channels,
-                                 relu=relu, dilation=getattr(mod, "_dilation", (1, 1)))[1]
+        device = operand.device
     # deferred: the ReLU that may follow is fused on demand, and a NewAdd consumer can absorb the whole convolution
-    return QTensor((N, conv.out_channels, P, Q), q.device, q8_bit=mod.output_bit,
-                   lazy_conv=_LazyConv(mod, run_conv, q))
+    return QTensor(mod._out_shape(operand), device, q8_bit=mod.output_bit, lazy_conv=_LazyConv(mod, operand))
 
 
 def _operand(t):
@@ -425,8 +388,6 @@ def enable_int8_pipeline(model, enabled=True):
     for m in model.modules():
         if isinstance(m, (NewConv2d, NewAdd)):
             m.int8_pipeline = enabled
-        if isinstance(m, NewConv2d):
-            m._fuse_relu = False                       # kept for models pickled by earlier versions; unused
     return model
 
 

@@ -177,20 +177,29 @@ class _IntSimBase(nn.Module):
         layer.weight = nn.Parameter(wq)
         layer.bias = nn.Parameter(torch.zeros(out_features, device=w.device))
         self.register_buffer("quantized_bias", bq)                      # fp32, integer-valued
-        # [N] bias, followed (when N % 4 == 0 and 1 <= rs <= 20) by the folded constants of the int8 epilogue
+        # [N] bias, followed (when N % 16 == 0 and 1 <= rs <= 20) by the folded constants of the int8 epilogue
         self.register_buffer("_bias_i32", _native.bias_fold(bq.to(torch.int32), self.rs_bit))
         return wq
 
 
 class NewConv2d(_IntSimBase):
-    """Integer-simulated convolution (new_quantity_op.py:104-163)."""
+    """Integer-simulated convolution (new_quantity_op.py:104-163).
+
+    quantity() picks the kernel for the layer's shape and builds the weights that kernel reads:
+      _payload_channels set   int8 NHWC image with that many (padded) channels -> pq_conv2d_s8 (implicit GEMM)
+      _smallc                 <= 8 channels: zero-padded image of 8-byte pixels -> pq_conv2d_smallc_s8 (one TMA
+                              per filter row); with _s2d the same kernel on the space-to-depth image (stride 2,
+                              <= 4 channels)
+      _explicit_im2col        other convolutions with <= 8 channels: explicit im2col matrix -> pq_gemm_s8
+      _group_convs            groups > 1: one NewConv2d per group
+    Only this class reads these flags: forward() and the int8 pipeline run the layer through _quantize / _run /
+    _run_add."""
 
     def __init__(self, conv_module, quantize_infor):
         super().__init__()
         self._read_info(quantize_infor)
         self.Conv = conv_module
         self.int8_pipeline = False      # see int8_pipeline.enable_int8_pipeline
-        self._fuse_relu = False
         self.quantity()
 
     def quantity(self):
@@ -203,19 +212,28 @@ class NewConv2d(_IntSimBase):
         wq = self._quantize_params(conv, conv.out_channels)
         K, C, R, S = wq.shape
         self._dilation = tuple(int(d) for d in conv.dilation) if (R, S) != (1, 1) else (1, 1)
-        dilated = self._dilation != (1, 1)
+        # channel count of the int8 NHWC operand, None when the layer's kernel reads another layout
+        self._payload_channels = None
+        # whether _run_add can fuse a following NewAdd into this convolution's epilogue
+        self._fuses_add = False
         self._group_convs = None
+        self._smallc = self._s2d = self._explicit_im2col = False
         if conv.groups != 1:
             self._build_groups(conv, wq)
             return
         # im2col TMA fetches channel blocks of 32 / 64 / 128 bytes; a 1x1 stride-1 conv is a plain GEMM
         plain = (R, S) == (1, 1) and tuple(conv.stride) == (1, 1) and tuple(conv.padding) == (0, 0)
-        # very few input channels (the ResNet stem): instead of padding C to 32, either the windowed
-        # small-channel kernel (8-byte pixels, one TMA per filter row) or explicit im2col + GEMM
-        # (a dilated filter always takes the im2col-TMA kernel: its taps are TMA offsets)
-        self._smallc = (not plain) and not dilated and C <= 8 and S <= 8 and conv.stride[1] % 2 == 0
-        self._explicit_im2col = (not plain) and not dilated and C <= 8 and not self._smallc
-        if self._smallc:
+        if plain or C > 8 or self._dilation != (1, 1):
+            # (a dilated filter always takes the im2col-TMA kernel: its taps are TMA offsets)
+            self._payload_channels = _pad16(C) if plain else _pad32(C)
+            self._fuses_add = self._dilation == (1, 1) and K % 16 == 0
+            w_krsc = torch.zeros((K, R, S, self._payload_channels), dtype=torch.int8, device=wq.device)
+            w_krsc[..., :C] = wq.permute(0, 2, 3, 1).to(torch.int8)
+            self.register_buffer("_w_krsc", w_krsc.contiguous())
+        elif S <= 8 and conv.stride[1] % 2 == 0:
+            # very few input channels (the ResNet stem): instead of padding C to 32, the windowed small-channel
+            # kernel over 8-byte pixels
+            self._smallc = True
             w = torch.zeros((K, R, 8, 8), dtype=torch.int8, device=wq.device)       # [K][R][tap slot][channel slot]
             w[:, :, :S, :C] = wq.permute(0, 2, 3, 1).to(torch.int8)
             self.register_buffer("_w_krs8", w.view(K, R, 64).contiguous())
@@ -227,17 +245,13 @@ class NewConv2d(_IntSimBase):
             self._s2d = S2D_STEM and tuple(conv.stride) == (2, 2) and C <= 4 and R <= 7 and S <= 7
             if self._s2d:
                 self.register_buffer("_w_s2d", s2d_filter(wq, conv.padding), persistent=False)
-            return
-        if self._explicit_im2col:
+        else:
+            # the small-channel kernel does not apply (odd stride, wide filter): explicit im2col + GEMM
+            self._explicit_im2col = True
             self._k_pad = (R * S * C + 63) // 64 * 64
             w_nk = torch.zeros((K, self._k_pad), dtype=torch.int8, device=wq.device)
             w_nk[:, :R * S * C] = wq.permute(0, 2, 3, 1).reshape(K, -1).to(torch.int8)
             self.register_buffer("_w_nk", w_nk.contiguous())
-            return
-        self._c_pad = _pad16(C) if plain else _pad32(C)
-        w_krsc = torch.zeros((K, R, S, self._c_pad), dtype=torch.int8, device=wq.device)
-        w_krsc[..., :C] = wq.permute(0, 2, 3, 1).to(torch.int8)
-        self.register_buffer("_w_krsc", w_krsc.contiguous())
 
     def _build_groups(self, conv, wq):
         """groups > 1 (the reference wraps any nn.Conv2d, new_quantity_op.py:104-133): one integer convolution per
@@ -255,7 +269,6 @@ class NewConv2d(_IntSimBase):
             subs.append(NewConv2d(sub, {"weight_bit": self.weight_bit, "bias_bit": self.bias_bit,
                                         "input_bit": self.input_bit, "output_bit": self.output_bit}))
         self._group_convs = nn.ModuleList(subs)
-        self._smallc = self._explicit_im2col = False
 
     def _grouped_forward(self, input):
         x = input.dequantize() if hasattr(input, "dequantize") else input
@@ -266,51 +279,85 @@ class NewConv2d(_IntSimBase):
     def forward(self, input):
         if CHECK_ACC_RANGE:
             self._check_acc(input, self.Conv)
-        if getattr(self, "_group_convs", None) is not None:
+        if self._group_convs is not None:
             return self._grouped_forward(input)
-        if getattr(self, "int8_pipeline", False):
+        if self.int8_pipeline:
             from .int8_pipeline import conv_forward
             return conv_forward(self, input)
+        return self._run(self._quantize(input), True, False, False)[0]   # Quan, Conv+RightShift+BiasAdd+Sp+DeQuan
+
+    # ---- the layer's launch path (not for grouped layers).  An operand is what _quantize returns: the int8 NHWC image
+    # [N][H][W][_payload_channels] when _payload_channels is set (a producer's int8 payload at input_bit is one, too),
+    # otherwise (int8 tensor in the kernel's layout, (N, H, W) of the input).
+
+    def _quantize(self, x):
+        """Quantity(input_bit) of fp32 NCHW x into the operand this layer's kernel reads."""
         conv = self.Conv
-        if getattr(self, "_smallc", False):
-            out, _ = self._smallc_forward(input, want_f32=True, want_s8=False, relu=False)
-            return out
+        if self._payload_channels is not None:
+            return _native.quantize_nchw_to_nhwc_s8(x, self.input_bit, self._payload_channels)
+        N, _, H, W = x.shape
         if self._explicit_im2col:
-            a, (N, P, Q) = _native.quantize_im2col_s8(input, self.input_bit, conv.kernel_size, conv.stride,
-                                                      conv.padding, self._k_pad)       # Quan + im2col
-            out, _ = _native.gemm_s8(a, self._w_nk, self._bias_i32, self.rs_bit, self.output_bit, hw=P * Q,
-                                     k_real=conv.in_channels * conv.kernel_size[0] * conv.kernel_size[1])
-            return out.view(N, conv.out_channels, P, Q)
-        q = _native.quantize_nchw_to_nhwc_s8(input, self.input_bit, self._c_pad)        # Quan
-        out, _ = _native.conv2d_s8(q, self._w_krsc, self._bias_i32, conv.stride, conv.padding,
-                                   self.rs_bit, self.output_bit, c_real=conv.in_channels,
-                                   dilation=getattr(self, "_dilation", (1, 1)))   # Conv+RightShift+BiasAdd+Sp+DeQuan
-        return out
-
-
-    def _smallc_forward(self, input, want_f32, want_s8, relu):
-        """Quan into a zero-padded 8-byte-pixel NHWC image, then the windowed small-channel convolution."""
-        conv = self.Conv
+            a, _ = _native.quantize_im2col_s8(x, self.input_bit, conv.kernel_size, conv.stride, conv.padding,
+                                              self._k_pad)
+            return a, (N, H, W)
         (R, S), (sh, sw), (ph, pw) = conv.kernel_size, conv.stride, conv.padding
-        H, W = input.shape[2], input.shape[3]
-        P, Q = (H + 2 * ph - R) // sh + 1, (W + 2 * pw - S) // sw + 1
-        if getattr(self, "_s2d", False):
-            ra = self._w_s2d.shape[1]
-            hp2, wp2 = P + ra - 1, Q + 3                       # blocks the 64-byte row windows of every output touch
-            xs = _native.quantize_s2d16_s8(input, self.input_bit, (ph + (ph & 1), pw + (pw & 1)), hp2, wp2)
-            # the same bytes as an 8-byte-pixel image of twice the width: filter of ra rows x 8 slots, stride (1, 2)
-            return _native.conv2d_smallc_s8(xs.view(xs.shape[0], hp2, 2 * wp2, 8), self._w_s2d, self._bias_i32,
-                                            (hp2, 2 * wp2), (ra, 8), (1, 2), (0, 0), self.rs_bit, self.output_bit,
-                                            want_f32=want_f32, want_s8=want_s8, relu=relu,
-                                            ops=2 * input.shape[0] * P * Q * conv.out_channels * R * S * conv.in_channels)
+        P, Q = _native.conv_out_size((H, W), conv.kernel_size, conv.stride, conv.padding)
+        if self._s2d:
+            hp2, wp2 = P + self._w_s2d.shape[1] - 1, Q + 3      # blocks the 64-byte row windows of every output touch
+            xs = _native.quantize_s2d16_s8(x, self.input_bit, (ph + (ph & 1), pw + (pw & 1)), hp2, wp2)
+            # the same bytes as an 8-byte-pixel image of twice the width
+            return xs.view(N, hp2, 2 * wp2, 8), (N, H, W)
         Hp = max((P - 1) * sh + R, H + ph)
         Hp = (Hp + sh - 1) // sh * sh
         Wp = max((Q - 1) * sw + 8, W + pw)
         Wp += Wp & 1
-        xp = _native.quantize_pad_nhwc8_s8(input, self.input_bit, (ph, pw), Hp, Wp)
-        return _native.conv2d_smallc_s8(xp, self._w_krs8, self._bias_i32, (H, W), (R, S), (sh, sw), (ph, pw),
-                                        self.rs_bit, self.output_bit, want_f32=want_f32, want_s8=want_s8,
-                                        c_real=conv.in_channels, relu=relu)
+        return _native.quantize_pad_nhwc8_s8(x, self.input_bit, (ph, pw), Hp, Wp), (N, H, W)
+
+    def _out_shape(self, operand):
+        """(N, K, P, Q) of the layer's output for this operand."""
+        conv = self.Conv
+        N, H, W = operand.shape[:3] if self._payload_channels is not None else operand[1]
+        P, Q = _native.conv_out_size((H, W), conv.kernel_size, conv.stride, conv.padding, self._dilation)
+        return N, conv.out_channels, P, Q
+
+    def _run(self, operand, want_f32, want_s8, relu):
+        """Conv + RightShift + BiasAdd + Sp (+ the nn.ReLU after the layer when relu) on an operand.  Returns
+        (fp32 NCHW after DeQuantity or None, int8 NHWC [N][P][Q][K] or None)."""
+        conv = self.Conv
+        if self._payload_channels is not None:
+            return _native.conv2d_s8(operand, self._w_krsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
+                                     self.output_bit, want_f32=want_f32, want_s8=want_s8, c_real=conv.in_channels,
+                                     relu=relu, dilation=self._dilation)
+        t = operand[0]
+        N, K, P, Q = self._out_shape(operand)
+        if self._explicit_im2col:
+            f32, s8 = _native.gemm_s8(t, self._w_nk, self._bias_i32, self.rs_bit, self.output_bit, hw=P * Q,
+                                      want_f32=want_f32, want_s8=want_s8, relu=relu,
+                                      k_real=conv.in_channels * conv.kernel_size[0] * conv.kernel_size[1])
+            return (f32.view(N, K, P, Q) if want_f32 else None), (s8.view(N, P, Q, K) if want_s8 else None)
+        if self._s2d:
+            # filter of ra rows x 8 slots, stride (1, 2) over the 8-byte-pixel view
+            (R, S), ra = conv.kernel_size, self._w_s2d.shape[1]
+            return _native.conv2d_smallc_s8(t, self._w_s2d, self._bias_i32, t.shape[1:3], (ra, 8), (1, 2), (0, 0),
+                                            self.rs_bit, self.output_bit, want_f32=want_f32, want_s8=want_s8,
+                                            relu=relu, ops=2 * N * P * Q * K * R * S * conv.in_channels)
+        return _native.conv2d_smallc_s8(t, self._w_krs8, self._bias_i32, operand[1][1:], conv.kernel_size,
+                                        conv.stride, conv.padding, self.rs_bit, self.output_bit, want_f32=want_f32,
+                                        want_s8=want_s8, c_real=conv.in_channels, relu=relu)
+
+    def _smallc_forward(self, input, want_f32, want_s8, relu):
+        """Quan + the small-channel convolution from fp32 NCHW input, in the form _s2d selects (the space-to-depth
+        image or the 8-byte-pixel image; both give the same integers).  Returns what _run returns."""
+        return self._run(self._quantize(input), want_f32, want_s8, relu)
+
+    def _run_add(self, operand, shortcut, shortcut_bit, shortcut_relu, q_bit, relu, want16):
+        """This layer and the NewAdd of its int8 output with `shortcut` (int8 / int16 NHWC at shortcut_bit), plus the
+        nn.ReLU after the add when relu, in one kernel (only where _fuses_add).  Returns (int16 exact sum or None,
+        int8 Quantity(q_bit) of it), both NHWC."""
+        conv = self.Conv
+        return _native.conv2d_s8_add(operand, self._w_krsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
+                                     self.output_bit, shortcut, shortcut_bit, shortcut_relu, q_bit, relu,
+                                     want16=want16, c_real=conv.in_channels)
 
 
 def s2d_filter(wq, padding):

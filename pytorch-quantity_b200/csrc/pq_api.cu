@@ -1,7 +1,7 @@
 // pq_api.cu -- library identity and error strings.
 #include "pq_common.cuh"
 
-extern "C" int pq_version(void) { return 100; }   // 0.1.0
+extern "C" int pq_version(void) { return PQ_VERSION; }
 
 extern "C" const char *pq_error_string(int code)
 {

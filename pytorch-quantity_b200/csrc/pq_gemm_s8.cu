@@ -1483,12 +1483,12 @@ int encode_nd(CUtensorMap *map, const void *base, int rank, const cuuint64_t *di
     return r == CUDA_SUCCESS ? PQ_OK : PQ_EUNSUPPORTED;
 }
 
-int encode_im2col(CUtensorMap *map, const void *base, const pq_conv_desc &d, int bk, int dil_h, int dil_w)
+int encode_im2col(CUtensorMap *map, const void *base, const pq_conv_desc &d, int bk)
 {
     cuuint64_t dims[4] = {(cuuint64_t)d.C, (cuuint64_t)d.W, (cuuint64_t)d.H, (cuuint64_t)d.N};
     cuuint64_t strides[3] = {(cuuint64_t)d.C, (cuuint64_t)d.W * d.C, (cuuint64_t)d.H * d.W * d.C};
     int lower[2] = {-d.pad_w, -d.pad_h};
-    int upper[2] = {d.pad_w - (d.S - 1) * dil_w, d.pad_h - (d.R - 1) * dil_h};
+    int upper[2] = {d.pad_w - (d.S - 1) * d.dil_w, d.pad_h - (d.R - 1) * d.dil_h};
     cuuint32_t estr[4] = {1, (cuuint32_t)d.stride_w, (cuuint32_t)d.stride_h, 1};
     CUresult r = g_encode_im2col(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, const_cast<void *>(base), dims, strides,
                                  lower, upper, (cuuint32_t)bk, (cuuint32_t)pq::kBM, estr,
@@ -1530,19 +1530,27 @@ int launch_pdl(void (*kern)(KArgs...), int grid, size_t smem, cudaStream_t s, Ar
     return (int)cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
 
-template <int BN, int BK, int STAGES, int BSLOTS = STAGES>
-int launch_cfg(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, cudaStream_t s)
+// one gemm_s8_kernel instance (opted in to its shared memory on first use) on a persistent grid: one CTA per SM
+template <int BN, int BK, int STAGES, bool ADDK, int BSLOTS>
+int launch_gemm(const CUtensorMap &ta, const CUtensorMap &tb, const CUtensorMap &to, const CUtensorMap &tsc,
+                const CUtensorMap &to16, const pq::GemmParams &p, cudaStream_t s)
 {
-    using Cfg = pq::GemmSmem<BN, BK, STAGES, false, BSLOTS>;
+    using Cfg = pq::GemmSmem<BN, BK, STAGES, ADDK, BSLOTS>;
     static_assert(Cfg::kTotal <= 227 * 1024, "shared memory budget");
-    auto kern = pq::gemm_s8_kernel<BN, BK, STAGES, false, BSLOTS>;
+    auto kern = pq::gemm_s8_kernel<BN, BK, STAGES, ADDK, BSLOTS>;
     static bool attr = false;
     if (!attr) {
         PQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kTotal));
         attr = true;
     }
     const long long tiles = (long long)((p.M + pq::kBM - 1) / pq::kBM) * ((p.N + BN - 1) / BN);
-    const int grid = (int)(tiles < num_sms() ? tiles : num_sms());     // persistent: one CTA per SM
+    const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
+    return launch_pdl(kern, grid, Cfg::kTotal, s, ta, tb, to, tsc, to16, p);
+}
+
+template <int BN, int BK, int STAGES, int BSLOTS = STAGES>
+int launch_cfg(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, cudaStream_t s)
+{
     p.b_resident = (p.a_im2col != 2 && p.N <= BN && p.num_kb <= BSLOTS) ? 1 : 0;
     if (BSLOTS != STAGES && !p.b_resident) return PQ_EUNSUPPORTED;      // deep-A configurations need the resident B
     // int8 output tile: [128 rows][min(BN, 128) bytes] boxes of the row-major [M][N] result
@@ -1565,7 +1573,7 @@ int launch_cfg(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, 
         p.stage_s8 = 1;
     }
     const CUtensorMap none = {};
-    return launch_pdl(kern, grid, Cfg::kTotal, s, ta, tb, to, none, none, p);
+    return launch_gemm<BN, BK, STAGES, false, BSLOTS>(ta, tb, to, none, none, p, s);
 }
 
 // fused NewConv2d + NewAdd kernels (ADDK): int8 result, shortcut and int16 sum travel as [32 rows][32 channels]
@@ -1573,16 +1581,6 @@ int launch_cfg(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, 
 template <int BN, int BK, int STAGES>
 int launch_cfg_add(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, cudaStream_t s)
 {
-    using Cfg = pq::GemmSmem<BN, BK, STAGES, true>;
-    static_assert(Cfg::kTotal <= 227 * 1024, "shared memory budget");
-    auto kern = pq::gemm_s8_kernel<BN, BK, STAGES, true>;
-    static bool attr = false;
-    if (!attr) {
-        PQ_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kTotal));
-        attr = true;
-    }
-    const long long tiles = (long long)((p.M + pq::kBM - 1) / pq::kBM) * ((p.N + BN - 1) / BN);
-    const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
     p.b_resident = (p.N <= BN && p.num_kb <= STAGES) ? 1 : 0;
     CUtensorMap to = {}, tsc = {}, to16 = {};
     int rc;
@@ -1593,7 +1591,7 @@ int launch_cfg_add(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams 
     if (rc != PQ_OK) return rc;
     if (p.out16 && (rc = encode_2d(&to16, p.out16, 2 * N, M, 2 * N, 2 * pq::kAddSlab, 32)) != PQ_OK) return rc;
     p.stage_s8 = 1;
-    return launch_pdl(kern, grid, Cfg::kTotal, s, ta, tb, to, tsc, to16, p);
+    return launch_gemm<BN, BK, STAGES, true, STAGES>(ta, tb, to, tsc, to16, p, s);
 }
 
 // stage counts: fill ~192 KB of shared memory, at most 8 stages
@@ -1644,14 +1642,18 @@ int launch(const CUtensorMap &ta, const CUtensorMap &tb, pq::GemmParams &p, int 
 }  // namespace
 
 namespace {
-// validates a fused-add request and copies it into the kernel parameters
-// PQ_FLAG_BIAS_FOLDED: bias_q is int32 [2][N] = bias | 2^(rs-1) + (bias << rs)   (pq_bias_fold_s32)
-void apply_bias_fold(pq::GemmParams &p, const int32_t *bias_q, int flags, int N, int rs)
+// the epilogue half of GemmParams (RightShift, BiasAdd, Sp, DeQuantity, the fused ReLU and the outputs); p.N must be set.
+// PQ_FLAG_BIAS_FOLDED: bias_q is int32 [3][N] as written by pq_bias_fold_s32
+void set_epilogue(pq::GemmParams &p, const int32_t *bias_q, int rs, int ob, int hw, int flags, float *out_f32,
+                  int8_t *out_s8)
 {
-    p.bias_c = ((flags & PQ_FLAG_BIAS_FOLDED) && rs >= 1 && rs <= 20 && (N & 15) == 0) ? bias_q + N : nullptr;
-    p.bias_hl = p.bias_c ? reinterpret_cast<const uint32_t *>(bias_q + 2 * N) : nullptr;
+    p.rs = rs; p.ob = ob; p.hw = hw; p.bias = bias_q; p.out_f32 = out_f32; p.out_s8 = out_s8;
+    p.relu = flags & PQ_FLAG_RELU;
+    p.bias_c = ((flags & PQ_FLAG_BIAS_FOLDED) && rs >= 1 && rs <= 20 && (p.N & 15) == 0) ? bias_q + p.N : nullptr;
+    p.bias_hl = p.bias_c ? reinterpret_cast<const uint32_t *>(bias_q + 2 * p.N) : nullptr;
 }
 
+// validates a fused-add request and copies it into the kernel parameters
 int apply_add(pq::GemmParams &p, const pq_add_desc *add, int conv_ob)
 {
     if (!add) return PQ_OK;
@@ -1667,30 +1669,7 @@ int apply_add(pq::GemmParams &p, const pq_add_desc *add, int conv_ob)
     p.out16 = add->out16; p.out_s8 = add->out8;
     return PQ_OK;
 }
-int gemm_impl(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs, int ob, int hw,
-              int flags, float *out_f32, int8_t *out_s8, const pq_add_desc *add, pq_stream_t stream);
-}  // namespace
 
-extern "C" int pq_gemm_s8(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs,
-                          int ob, int hw, float *out_f32, int8_t *out_s8, pq_stream_t stream)
-{
-    return pq_gemm_s8_ex(a, w, bias_q, M, N, K, rs, ob, hw, 0, out_f32, out_s8, stream);
-}
-
-extern "C" int pq_gemm_s8_ex(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs,
-                             int ob, int hw, int flags, float *out_f32, int8_t *out_s8, pq_stream_t stream)
-{
-    return gemm_impl(a, w, bias_q, M, N, K, rs, ob, hw, flags, out_f32, out_s8, nullptr, stream);
-}
-
-extern "C" int pq_gemm_s8_add(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs,
-                              int ob, const pq_add_desc *add_host, pq_stream_t stream)
-{
-    if (!add_host) return PQ_EINVAL;
-    return gemm_impl(a, w, bias_q, M, N, K, rs, ob, 1, 0, nullptr, add_host->out8, add_host, stream);
-}
-
-namespace {
 int gemm_impl(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs, int ob, int hw,
               int flags, float *out_f32, int8_t *out_s8, const pq_add_desc *add, pq_stream_t stream)
 {
@@ -1709,67 +1688,19 @@ int gemm_impl(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, in
     if ((rc = encode_2d(&tb, w, K, N, K, bk, bn)) != PQ_OK) return rc;
     pq::GemmParams p = {};
     p.M = M; p.N = N; p.num_kb = (K + bk - 1) / bk; p.a_im2col = 0;
-    p.rs = rs; p.ob = ob; p.hw = hw; p.bias = bias_q; p.out_f32 = out_f32; p.out_s8 = out_s8;
-    p.relu = flags & PQ_FLAG_RELU;
-    apply_bias_fold(p, bias_q, flags, N, rs);
+    set_epilogue(p, bias_q, rs, ob, hw, flags, out_f32, out_s8);
     if ((rc = apply_add(p, add, ob)) != PQ_OK) return rc;
     return launch(ta, tb, p, bk, bn, (cudaStream_t)stream);
 }
-}  // namespace
 
-extern "C" int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                            const pq_conv_desc *desc_host, float *out_f32_nchw, int8_t *out_s8_nhwc,
-                            pq_stream_t stream)
-{
-    return pq_conv2d_s8_ex(x_nhwc, w_krsc, bias_q, desc_host, 0, out_f32_nchw, out_s8_nhwc, stream);
-}
-
-namespace {
 int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
-              int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, const pq_add_desc *add, pq_stream_t stream,
-              int dil_h = 1, int dil_w = 1);
-}
-
-extern "C" int pq_conv2d_s8_dil(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                                const pq_conv_desc *desc_host, int dil_h, int dil_w, int flags, float *out_f32_nchw,
-                                int8_t *out_s8_nhwc, pq_stream_t stream)
-{
-    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, flags, out_f32_nchw, out_s8_nhwc, nullptr, stream, dil_h,
-                     dil_w);
-}
-
-extern "C" int pq_conv2d_s8_ex(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                               const pq_conv_desc *desc_host, int flags, float *out_f32_nchw,
-                               int8_t *out_s8_nhwc, pq_stream_t stream)
-{
-    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, flags, out_f32_nchw, out_s8_nhwc, nullptr, stream);
-}
-
-extern "C" int pq_conv2d_s8_add(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                                const pq_conv_desc *desc_host, const pq_add_desc *add_host, pq_stream_t stream)
-{
-    if (!add_host) return PQ_EINVAL;
-    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, 0, nullptr, add_host->out8, add_host, stream);
-}
-
-extern "C" int pq_conv2d_s8_add_ex(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
-                                   const pq_conv_desc *desc_host, const pq_add_desc *add_host, int flags,
-                                   pq_stream_t stream)
-{
-    if (!add_host || (flags & PQ_FLAG_RELU)) return PQ_EINVAL;   // the ReLU of a fused add is add_host->out_relu
-    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, flags, nullptr, add_host->out8, add_host, stream);
-}
-
-namespace {
-int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
-              int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, const pq_add_desc *add, pq_stream_t stream,
-              int dil_h, int dil_w)
+              int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, const pq_add_desc *add, pq_stream_t stream)
 {
     if (!x_nhwc || !w_krsc || !bias_q || !desc_host || (!out_f32_nchw && !out_s8_nhwc)) return PQ_EINVAL;
     const pq_conv_desc &d = *desc_host;
     if (d.N <= 0 || d.H <= 0 || d.W <= 0 || d.C <= 0 || d.K <= 0 || d.R <= 0 || d.S <= 0) return PQ_EINVAL;
-    if (d.stride_h <= 0 || d.stride_w <= 0 || d.pad_h < 0 || d.pad_w < 0 || dil_h <= 0 || dil_w <= 0) return PQ_EINVAL;
-    const int r_eff = (d.R - 1) * dil_h + 1, s_eff = (d.S - 1) * dil_w + 1;       // footprint of the dilated filter
+    if (d.stride_h <= 0 || d.stride_w <= 0 || d.pad_h < 0 || d.pad_w < 0 || d.dil_h <= 0 || d.dil_w <= 0) return PQ_EINVAL;
+    const int r_eff = (d.R - 1) * d.dil_h + 1, s_eff = (d.S - 1) * d.dil_w + 1;   // footprint of the dilated filter
     if (d.H + 2 * d.pad_h < r_eff || d.W + 2 * d.pad_w < s_eff) return PQ_EINVAL;
     if (d.P != (d.H + 2 * d.pad_h - r_eff) / d.stride_h + 1 || d.Q != (d.W + 2 * d.pad_w - s_eff) / d.stride_w + 1)
         return PQ_EINVAL;
@@ -1789,7 +1720,7 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
     // windows (GemmParams, a_im2col == 3).  The im2col gather re-reads every input byte nine times out of L2 and bounds
     // these layers at ~9.5 TB/s of L2 -> SM traffic; the window box is read (TH + 2) / TH times.
     if (!add && !(flags & PQ_FLAG_NO_WINDOWS) && d.R == 3 && d.S == 3 && d.stride_h == 1 && d.stride_w == 1 &&
-        d.pad_h == 1 && d.pad_w == 1 && dil_h == 1 && dil_w == 1 &&
+        d.pad_h == 1 && d.pad_w == 1 && d.dil_h == 1 && d.dil_w == 1 &&
         ((d.C == 64 && d.K <= 64) || (d.C == 128 && d.K > 64 && d.K <= 128)) && d.W + 2 <= 64) {
         const int tw_shift = d.W + 2 <= 16 ? 4 : (d.W + 2 <= 32 ? 5 : 6);
         const int TW = 1 << tw_shift, TH = pq::kBM / TW;
@@ -1813,9 +1744,7 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
             p.P = d.P; p.Q = d.Q; p.stride_h = 1; p.stride_w = 1; p.pad_h = 1; p.pad_w = 1; p.dil_h = 1; p.dil_w = 1;
             p.tw_shift = tw_shift; p.TW = TW; p.TH = TH; p.tiles_q = 1; p.tiles_p = (d.P + TH - 1) / TH;
             p.win_slot_bytes = slot; p.win_slots = slots;
-            p.rs = d.rs; p.ob = d.ob; p.hw = d.P * d.Q; p.bias = bias_q; p.out_f32 = out_f32_nchw; p.out_s8 = out_s8_nhwc;
-            p.relu = flags & PQ_FLAG_RELU;
-            apply_bias_fold(p, bias_q, flags, d.K, d.rs);
+            set_epilogue(p, bias_q, d.rs, d.ob, d.P * d.Q, flags, out_f32_nchw, out_s8_nhwc);
             return d.C == 64 ? launch_cfg<64, 64, 18, 9>(ta, tb, p, (cudaStream_t)stream)
                              : launch_cfg<128, 128, 3, 9>(ta, tb, p, (cudaStream_t)stream);
         }
@@ -1824,7 +1753,7 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
     int bn = pick_bn(M, d.K);
     if (add && bn < 64) bn = 64;                 // the fused-add pass works on 64-column slabs
     CUtensorMap ta, tb;
-    if ((rc = encode_im2col(&ta, x_nhwc, d, bk, dil_h, dil_w)) != PQ_OK) return rc;
+    if ((rc = encode_im2col(&ta, x_nhwc, d, bk)) != PQ_OK) return rc;
     const uint64_t ktot = (uint64_t)d.R * d.S * d.C;
     pq::GemmParams p = {};
     p.M = (int)M; p.N = d.K; p.a_im2col = 1;
@@ -1841,14 +1770,33 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
         if ((rc = encode_nd(&tb, w_krsc, 3, bdims, bstr, bbox, bk)) != PQ_OK) return rc;
     }
     p.P = d.P; p.Q = d.Q; p.stride_h = d.stride_h; p.stride_w = d.stride_w; p.pad_h = d.pad_h; p.pad_w = d.pad_w;
-    p.dil_h = dil_h; p.dil_w = dil_w;
-    p.rs = d.rs; p.ob = d.ob; p.hw = d.P * d.Q; p.bias = bias_q; p.out_f32 = out_f32_nchw; p.out_s8 = out_s8_nhwc;
-    p.relu = flags & PQ_FLAG_RELU;
-    apply_bias_fold(p, bias_q, flags, d.K, d.rs);
+    p.dil_h = d.dil_h; p.dil_w = d.dil_w;
+    set_epilogue(p, bias_q, d.rs, d.ob, d.P * d.Q, flags, out_f32_nchw, out_s8_nhwc);
     if ((rc = apply_add(p, add, d.ob)) != PQ_OK) return rc;
     return launch(ta, tb, p, bk, bn, (cudaStream_t)stream);
 }
 }  // namespace
+
+extern "C" int pq_gemm_s8(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs,
+                          int ob, int hw, int flags, float *out_f32, int8_t *out_s8, pq_stream_t stream)
+{
+    return gemm_impl(a, w, bias_q, M, N, K, rs, ob, hw, flags, out_f32, out_s8, nullptr, stream);
+}
+
+extern "C" int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
+                            const pq_conv_desc *desc_host, int flags, float *out_f32_nchw, int8_t *out_s8_nhwc,
+                            pq_stream_t stream)
+{
+    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, flags, out_f32_nchw, out_s8_nhwc, nullptr, stream);
+}
+
+extern "C" int pq_conv2d_s8_add(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
+                                const pq_conv_desc *desc_host, const pq_add_desc *add_host, int flags,
+                                pq_stream_t stream)
+{
+    if (!add_host || (flags & PQ_FLAG_RELU)) return PQ_EINVAL;   // the ReLU of a fused add is add_host->out_relu
+    return conv_impl(x_nhwc, w_krsc, bias_q, desc_host, flags, nullptr, add_host->out8, add_host, stream);
+}
 
 // Convolution with <= 8 input channels over a zero-padded NHWC image with 8-byte pixels (see GemmParams):
 // xp is [N][Hp][Wp][8] int8 as written by pq_quantize_nchw_to_padded_nhwc8_s8 (image pixel (h, w) at
@@ -1862,6 +1810,7 @@ extern "C" int pq_conv2d_smallc_s8(const int8_t *xp, const int8_t *w_krs8, const
     const pq_conv_desc &d = *desc_host;
     if (d.N <= 0 || d.H <= 0 || d.W <= 0 || d.K <= 0 || d.R <= 0 || d.S <= 0) return PQ_EINVAL;
     if (d.stride_h <= 0 || d.stride_w <= 0 || d.pad_h < 0 || d.pad_w < 0) return PQ_EINVAL;
+    if (d.dil_h != 1 || d.dil_w != 1) return PQ_EUNSUPPORTED;
     if (d.P != (d.H + 2 * d.pad_h - d.R) / d.stride_h + 1 || d.Q != (d.W + 2 * d.pad_w - d.S) / d.stride_w + 1)
         return PQ_EINVAL;
     constexpr int kPix = 8, kBK = 64;
@@ -1882,9 +1831,7 @@ extern "C" int pq_conv2d_smallc_s8(const int8_t *xp, const int8_t *w_krs8, const
     p.M = (int)(patches * pq::kBM); p.N = d.K; p.num_kb = d.R;
     p.R = d.R; p.S = d.S; p.C = kPix; p.P = d.P; p.Q = d.Q;
     p.stride_h = d.stride_h; p.stride_w = d.stride_w; p.pad_h = d.pad_h; p.pad_w = d.pad_w;
-    p.rs = d.rs; p.ob = d.ob; p.hw = d.P * d.Q; p.bias = bias_q; p.out_f32 = out_f32_nchw; p.out_s8 = out_s8_nhwc;
-    p.relu = flags & PQ_FLAG_RELU;
-    apply_bias_fold(p, bias_q, flags, d.K, d.rs);
+    set_epilogue(p, bias_q, d.rs, d.ob, d.P * d.Q, flags, out_f32_nchw, out_s8_nhwc);
     // Preferred: the row kernel (stride_w == 2: GEMM rows 16 bytes apart == an un-swizzled core matrix)
     if (d.stride_w == 2 && d.R <= 8) {
         const int n_tiles = (d.K + 63) / 64;

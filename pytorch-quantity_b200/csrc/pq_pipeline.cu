@@ -469,14 +469,8 @@ extern "C" int pq_avgpool_global_nhwc_f32(const void *x, int is16, int bit, int 
 }
 
 extern "C" int pq_add_requant(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16, int b_bit,
-                              int b_relu, size_t n, int16_t *out16, int8_t *out8, int q_bit, pq_stream_t stream)
-{
-    return pq_add_requant_ex(a, a_is16, a_bit, a_relu, b, b_is16, b_bit, b_relu, n, 0, out16, out8, q_bit, stream);
-}
-
-extern "C" int pq_add_requant_ex(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16,
-                                 int b_bit, int b_relu, size_t n, int flags, int16_t *out16, int8_t *out8,
-                                 int q_bit, pq_stream_t stream)
+                              int b_relu, size_t n, int flags, int16_t *out16, int8_t *out8, int q_bit,
+                              pq_stream_t stream)
 {
     if (n == 0) return PQ_OK;
     if (!a || !b || (!out16 && !out8)) return PQ_EINVAL;

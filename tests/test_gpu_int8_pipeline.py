@@ -67,8 +67,8 @@ FUSED_ADD_CASES = [(2, 64, 14, 14, 256, 1, 1, 0, 4, 5, 4, True), (3, 32, 9, 11, 
 
 @pytest.mark.parametrize("case", FUSED_ADD_CASES, ids=["c%d_%dx%d_o%d_k%d" % (c[1], c[2], c[3], c[4], c[5]) for c in FUSED_ADD_CASES])
 def test_conv_add_fused_equals_conv_then_add(case):
-    """pq_conv2d_s8_add / pq_gemm_s8_add (NewConv2d + NewAdd + ReLU in one epilogue) against the two separate
-    kernels, which are pinned to the reference elsewhere."""
+    """pq_conv2d_s8_add (NewConv2d + NewAdd + ReLU in one epilogue; 1x1 stride-1 layers take its GEMM form) against
+    the two separate kernels, which are pinned to the reference elsewhere."""
     from common.quantity import _native
     B, Cin, H, W, Cout, k, stride, pad, ob, sbit, qbit, s16 = case
     g = torch.Generator(device="cuda").manual_seed(Cin + Cout)

@@ -258,8 +258,9 @@ def test_accumulator_range_debug_check():
 @pytest.mark.parametrize("case", gg.INTSIM_EXT_CASES, ids=[c[0] for c in gg.INTSIM_EXT_CASES])
 @pytest.mark.parametrize("pipeline", [False, True])
 def test_newconv2d_dilation_and_groups_vs_golden(oracle, case, pipeline):
-    """Dilation = im2col-TMA tap offsets (pq_conv2d_s8_dil), groups = one tensor-core convolution per group; against
-    the reference's NewConv2d around the same dilated / grouped nn.Conv2d (intsim_ext.npz) and the oracle."""
+    """Dilation = im2col-TMA tap offsets (pq_conv2d_s8 with pq_conv_desc.dil_h / dil_w), groups = one tensor-core
+    convolution per group; against the reference's NewConv2d around the same dilated / grouped nn.Conv2d
+    (intsim_ext.npz) and the oracle."""
     import common.quantity as cq
     g = load_golden("intsim_ext.npz")
     name, B, Cin, H, W, Cout, k, stride, pad, dil, groups = case[:11]

@@ -11,18 +11,42 @@ import pytest
 from conftest import GOLDEN, REPO, golden_json, load_golden
 
 
+def _header():
+    return open(os.path.join(REPO, "include", "pq_sm100.h")).read()
+
+
 def test_library_exports_every_declared_symbol():
     from common.quantity import _native
-    header = open(os.path.join(REPO, "include", "pq_sm100.h")).read()
+    header = _header()
     declared = set(re.findall(r"\b(pq_[a-z0-9_]+)\s*\(", header))
     assert declared, "no declarations parsed"
     assert declared == set(_native.SYMBOLS), declared ^ set(_native.SYMBOLS)
     lib = _native.lib()
     for name in declared:
         assert hasattr(lib, name), name
-    assert lib.pq_version() >= 100
+    version = int(re.search(r"#define PQ_VERSION (\d+)", header).group(1))
+    assert lib.pq_version() == version == _native.PQ_VERSION
     assert b"PQ_EINVAL" in lib.pq_error_string(-1)
     assert lib.pq_kl_workspace_doubles() >= 2048 + 2 * 1920
+
+
+def test_ctypes_signatures_match_the_header():
+    """ctypes passes surplus arguments through without complaint, so a stale argtypes list or struct layout would
+    misbind silently: every SYMBOLS entry must take as many parameters as the header declares, and the ctypes
+    structures must have the header structs' fields in the same order."""
+    from common.quantity import _native
+    header = re.sub(r"/\*.*?\*/", "", _header(), flags=re.S)
+    decls = re.findall(r"^[a-z_0-9 ]+\**\s*\**(pq_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", header, flags=re.M)
+    assert {name for name, _ in decls} == set(_native.SYMBOLS)
+    for name, params in decls:
+        params = params.strip()
+        count = 0 if params in ("", "void") else params.count(",") + 1
+        assert len(_native.SYMBOLS[name][1]) == count, name
+    for struct, cls in (("pq_conv_desc", _native.ConvDesc), ("pq_add_desc", _native.AddDesc),
+                        ("pq_concat_src", _native.ConcatSrc)):
+        body = re.search(r"typedef struct %s \{(.*?)\}" % struct, header, flags=re.S).group(1)
+        fields = [re.findall(r"\w+", part)[-1] for decl in body.split(";") if decl.strip() for part in decl.split(",")]
+        assert fields == [f[0] for f in cls._fields_], struct
 
 
 def test_product_never_imports_oracle():
