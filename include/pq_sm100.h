@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 200
+#define PQ_VERSION 201
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -69,6 +69,21 @@ int pq_absmax_multi_f32(const float *const *xs_host, const uint64_t *ns_host, in
  * Requires channels <= 8192, inner < 2^31 - 2^14 and outer * channels < 2^31. */
 int pq_absmax_per_channel_f32(const float *x, uint64_t outer, int channels, uint64_t inner,
                               uint32_t *max_bits, pq_stream_t stream);
+
+/* ---- the elementwise glue of the fp32 calibration forward (tools/pytorch_quantizer.py fuses it during
+ * Quantity.activation_quantize), each in ONE pass, bit for bit what the unfused PyTorch forward computes:
+ * the IEEE fp32 add of ATen's `a + 1 * b`, nn.ReLU as ATen's clamp_min (NaN passes, else max(v, 0)), and the max
+ * as pq_absmax_multi_f32 takes it.
+ * pq_conv_epilogue_f32: nn.Conv2d's bias add after cuDNN, in place on a contiguous fp32 NCHW y [N][C][hw]:
+ *   y += bias[c];  relu_out = relu(y) when relu_out != NULL;  *max_slot = max(*max_slot, bits(max |y|)) when
+ *   max_slot != NULL (one slot of a pq_absmax_multi_f32 max_bits array).
+ *   y and relu_out 16-byte aligned; N * C < 2^31, hw < 2^31, N * C * hw < 2^33 (hw % 4 != 0: < 2^31).
+ * pq_eltwise_add_f32: Eltwise (fabu_layer.py:5-11), z = a + b out of place over n elements, relu_out and max_slot
+ *   as above.  a, b, z, relu_out 16-byte aligned, z and relu_out alias nothing; n < 2^33. */
+int pq_conv_epilogue_f32(float *y, const float *bias, int N, int C, uint64_t hw, float *relu_out,
+                         uint32_t *max_slot, pq_stream_t stream);
+int pq_eltwise_add_f32(const float *a, const float *b, float *z, size_t n, float *relu_out, uint32_t *max_slot,
+                       pq_stream_t stream);
 
 /* ---- a3: DistributionCollector._add_to_distribution, distribution_collector.py:127-135
  * for every x != 0:  hist[i][min((int)trunc(fl32(|x| / interval_i)), 2047)] += 1

@@ -19,7 +19,7 @@ HIST_BINS_MAX = 8192
 KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
-PQ_VERSION = 200             # the header's PQ_VERSION: the entry points below match a library built from it
+PQ_VERSION = 201             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -28,6 +28,8 @@ SYMBOLS = {
     "pq_error_string": (ctypes.c_char_p, [_i]),
     "pq_absmax_multi_f32": (_i, [_vp, _vp, _i, _vp, _vp]),
     "pq_absmax_per_channel_f32": (_i, [_vp, ctypes.c_uint64, _i, ctypes.c_uint64, _vp, _vp]),
+    "pq_conv_epilogue_f32": (_i, [_vp, _vp, _i, _i, ctypes.c_uint64, _vp, _vp, _vp]),
+    "pq_eltwise_add_f32": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp]),
     "pq_hist2048_multi_f32": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "pq_kl_workspace_doubles": (_sz, []),
     "pq_kl_search_f64": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
@@ -200,6 +202,46 @@ def absmax_per_channel(x, max_bits, channel_dim=1):
     with _Timed("absmax_channel", 1, 4 * xc.numel(), xc.device):
         check(lib().pq_absmax_per_channel_f32(xc.data_ptr() if xc.numel() else None, outer, C, inner,
                                               max_bits.data_ptr(), _stream(xc)), "pq_absmax_per_channel_f32")
+
+
+def _require_f32_contiguous(tensors, what):
+    """The fused calibration kernels address fp32 elements of contiguous tensors on one CUDA device."""
+    dev = tensors[0].device
+    for t in tensors:
+        require_cuda(t, what)
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev:
+            raise RuntimeError("%s needs contiguous fp32 tensors on %s, got %s %s on %s"
+                               % (what, dev, t.dtype, "contiguous" if t.is_contiguous() else "strided", t.device))
+
+
+def conv_epilogue(y, bias, relu=False, max_slot=None):
+    """nn.Conv2d's bias add after a bias-less cuDNN convolution, in place on y (contiguous fp32 CUDA [N][C][H][W]):
+    y += bias[c].  Returns relu(y) as a new tensor when `relu`, else None.  max_slot: device address of one int32 of
+    an absmax_multi max_bits array that takes max |y|, or None.  Launched on y's current stream."""
+    _require_f32_contiguous((y, bias), "conv_epilogue")
+    N, C, H, W = y.shape
+    if bias.numel() != C:
+        raise RuntimeError("conv_epilogue: %d bias values for %d channels" % (bias.numel(), C))
+    r = torch.empty_like(y) if relu else None
+    with _Timed("conv_epilogue", 1, y.numel() * (12 if relu else 8), y.device):
+        check(lib().pq_conv_epilogue_f32(y.data_ptr(), bias.data_ptr(), N, C, H * W, r.data_ptr() if relu else None,
+                                         max_slot, _stream(y)), "pq_conv_epilogue_f32")
+    return r
+
+
+def eltwise_add(a, b, relu=False, max_slot=None):
+    """Eltwise: a + b for contiguous fp32 CUDA tensors of one shape.  Returns (sum, relu(sum) or None); max_slot as in
+    conv_epilogue."""
+    _require_f32_contiguous((a, b), "eltwise_add")
+    if a.shape != b.shape:
+        raise RuntimeError("eltwise_add: shapes %s and %s differ" % (tuple(a.shape), tuple(b.shape)))
+    z = torch.empty_like(a)
+    r = torch.empty_like(a) if relu else None
+    with _Timed("eltwise", 1, a.numel() * (16 if relu else 12), a.device):
+        check(lib().pq_eltwise_add_f32(a.data_ptr(), b.data_ptr(), z.data_ptr(), a.numel(),
+                                       r.data_ptr() if relu else None, max_slot, _stream(a)),
+              "pq_eltwise_add_f32")
+    return z, r
 
 
 def hist_multi(tensors, intervals, hist):

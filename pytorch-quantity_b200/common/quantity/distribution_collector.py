@@ -61,10 +61,13 @@ class DistributionCollector:
         self._max_bits = torch.zeros(n, dtype=torch.int32, device=self._device)
         self._hist = torch.zeros((n, self._interval_num), dtype=torch.int64, device=self._device)
 
-    def _gather(self, tensors):
+    def _gather(self, tensors, skip=()):
+        """The tensors as flat fp32 device tensors in tensor_list order; those named in `skip` as empty ones."""
         first = next(iter(tensors.values())) if len(tensors) else None
         self._ensure_state(first)
-        return [_native.to_device_f32(tensors[name], self._device) for name in self._tensor_list]
+        empty = torch.empty(0, device=self._device) if skip else None
+        return [empty if name in skip else _native.to_device_f32(tensors[name], self._device)
+                for name in self._tensor_list]
 
     # ------------------------------------------------------------------- reference API
     @property
@@ -104,10 +107,20 @@ class DistributionCollector:
 
     def refresh_max_val(self, tensors):
         """Pass 1: running max |x| of every tensor (distribution_collector.py:70-78)."""
+        self._refresh_max_val_except(tensors, ())
+
+    def _refresh_max_val_except(self, tensors, reduced):
+        """refresh_max_val for the tensors not named in `reduced`: those already went into their max_bits slots
+        (max_slot) while they were computed, the fused ops of the calibration forward.  They stay in the one
+        absmax_multi launch as empty segments."""
         self._max_vals_refreshed_flag = True
-        flat = self._gather(tensors)
-        _native.absmax_multi(flat, self._max_bits)
+        _native.absmax_multi(self._gather(tensors, reduced), self._max_bits)
         self._max_dirty = True
+
+    def _max_slot(self, name):
+        """Device address of the int32 max_bits slot of tensor `name`: the max_slot of a fused op."""
+        self._ensure_state(None)
+        return self._max_bits.data_ptr() + 4 * self._tensor_list.index(name)
 
     def add_to_distributions(self, tensors):
         """Pass 2: accumulate the 2048-bin |x| histograms (distribution_collector.py:80-135)."""

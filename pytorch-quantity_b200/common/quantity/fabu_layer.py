@@ -3,8 +3,8 @@
 The calibration tracer only sees ``nn.Module`` calls, so a model that wants its residual
 adds, concatenations and flattens observed (and later replaced, e.g. Eltwise -> NewAdd)
 must express them with these modules instead of ``+`` / ``torch.cat`` / ``.view``.
-They stay ordinary PyTorch ops on purpose: during calibration they are part of the user's
-fp32 forward, which is library time outside the rebuilt hot path."""
+They stay ordinary PyTorch ops; during calibration Quantity.activation_quantize runs Eltwise (and the
+nn.ReLU after it) as one native kernel with the same result (tools/pytorch_quantizer.py, plan_calibration_fusion)."""
 import torch
 from torch import nn
 

@@ -99,6 +99,65 @@ extern "C" int pq_absmax_per_channel_f32(const float *x, uint64_t outer, int cha
     return (int)cudaGetLastError();
 }
 
+namespace {
+bool aligned16(const void *p) { return (((unsigned long long)p) & 15ull) == 0; }
+
+int launch_epilogue(pq::EpiArgs &p, int mode, cudaStream_t stream)
+{
+    const unsigned long long nvec = p.n >> 2;
+    if (nvec >= (1ull << 31) || (mode == pq::EPI_BIAS1 && p.n >= (1ull << 31))) return PQ_EUNSUPPORTED;
+    magic31(p.hw, &p.m_hw, &p.s_hw);
+    magic31(p.channels, &p.m_chan, &p.s_chan);
+    unsigned long long blocks = (nvec / pq::kEpiUnroll + pq::kStatThreads - 1) / pq::kStatThreads;
+    if (blocks > (unsigned long long)pq::kNumSMs * 8) blocks = (unsigned long long)pq::kNumSMs * 8;
+    if (blocks == 0) blocks = 1;
+    const unsigned int g = (unsigned int)blocks;
+    if (mode == pq::EPI_BIAS4) pq::epilogue_kernel<pq::EPI_BIAS4><<<g, pq::kStatThreads, 0, stream>>>(p);
+    else if (mode == pq::EPI_BIAS1) pq::epilogue_kernel<pq::EPI_BIAS1><<<g, pq::kStatThreads, 0, stream>>>(p);
+    else pq::epilogue_kernel<pq::EPI_ADD><<<g, pq::kStatThreads, 0, stream>>>(p);
+    return (int)cudaGetLastError();
+}
+}  // namespace
+
+extern "C" int pq_conv_epilogue_f32(float *y, const float *bias, int N, int C, uint64_t hw, float *relu_out,
+                                    uint32_t *max_slot, pq_stream_t stream)
+{
+    if (N < 0 || C <= 0) return PQ_EINVAL;
+    if (N == 0 || hw == 0) return PQ_OK;
+    if (!y || !bias || relu_out == y) return PQ_EINVAL;
+    if (!aligned16(y) || !aligned16(relu_out) || (((unsigned long long)bias) & 3ull)) return PQ_EALIGN;
+    if (hw >= (1ull << 31) || (uint64_t)N * (uint64_t)C >= (1ull << 31)) return PQ_EUNSUPPORTED;
+    pq::EpiArgs p = {};
+    p.a = y;
+    p.b = bias;
+    p.out = y;
+    p.relu_out = relu_out;
+    p.max_slot = max_slot;
+    p.n = (uint64_t)N * (uint64_t)C * hw;
+    p.channels = (unsigned int)C;
+    const int mode = (hw & 3) == 0 ? pq::EPI_BIAS4 : pq::EPI_BIAS1;
+    p.hw = (unsigned int)(mode == pq::EPI_BIAS4 ? hw / 4 : hw);
+    return launch_epilogue(p, mode, (cudaStream_t)stream);
+}
+
+extern "C" int pq_eltwise_add_f32(const float *a, const float *b, float *z, size_t n, float *relu_out,
+                                  uint32_t *max_slot, pq_stream_t stream)
+{
+    if (n == 0) return PQ_OK;
+    if (!a || !b || !z || z == a || z == b || relu_out == a || relu_out == b || relu_out == z) return PQ_EINVAL;
+    if (!aligned16(a) || !aligned16(b) || !aligned16(z) || !aligned16(relu_out)) return PQ_EALIGN;
+    pq::EpiArgs p = {};
+    p.a = a;
+    p.b = b;
+    p.out = z;
+    p.relu_out = relu_out;
+    p.max_slot = max_slot;
+    p.n = n;
+    p.hw = 1;
+    p.channels = 1;
+    return launch_epilogue(p, pq::EPI_ADD, (cudaStream_t)stream);
+}
+
 extern "C" int pq_hist2048_multi_f32(const float *const *xs_host, const uint64_t *ns_host,
                                      const float *intervals_host, int k, long long *hist,
                                      pq_stream_t stream)

@@ -53,6 +53,21 @@ __host__ __device__ inline unsigned int seg_num_chunks(const float *p, unsigned 
 // ------------------------------------------------------------------------------ absmax
 __device__ __forceinline__ unsigned int absbits(float v) { return __float_as_uint(v) & 0x7fffffffu; }
 
+// Publish the CTA's maximum of the per-thread values m into *dst: warp redux, ONE atomic per CTA.  Every thread of
+// the kStatThreads-wide CTA must call it; s_warp is [kStatThreads / 32] shared words, free again on return.
+__device__ __forceinline__ void block_max_publish(unsigned int m, unsigned int *s_warp, unsigned int *dst)
+{
+    m = __reduce_max_sync(0xffffffffu, m);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = m;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        unsigned int w = threadIdx.x < kStatThreads / 32 ? s_warp[threadIdx.x] : 0u;
+        w = __reduce_max_sync(0xffffffffu, w);
+        if (threadIdx.x == 0 && w != 0) atomicMax(dst, w);
+    }
+    __syncthreads();
+}
+
 __global__ void __launch_bounds__(kStatThreads)
 absmax_multi_kernel(const __grid_constant__ SegTable tab, unsigned int *__restrict__ max_bits)
 {
@@ -90,16 +105,7 @@ absmax_multi_kernel(const __grid_constant__ SegTable tab, unsigned int *__restri
                 if (threadIdx.x < g.tail) m = max(m, absbits(g.p[g.n - g.tail + threadIdx.x]));
             }
         }
-        // publish this CTA's maximum for the segment: warp redux, one atomic per CTA
-        m = __reduce_max_sync(0xffffffffu, m);
-        if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = m;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            unsigned int w = threadIdx.x < kStatThreads / 32 ? s_warp[threadIdx.x] : 0u;
-            w = __reduce_max_sync(0xffffffffu, w);
-            if (threadIdx.x == 0 && w != 0) atomicMax(max_bits + seg, w);
-        }
-        __syncthreads();
+        block_max_publish(m, s_warp, max_bits + seg);      // this CTA's maximum for the segment
         m = 0;
         ++seg;
     }
@@ -268,6 +274,113 @@ absmax_periodic_kernel(const float4 *__restrict__ x, unsigned int vec_per_img, u
         const unsigned int m = s_cmax[i];
         if (m) atomicMax(max_bits + ch_base + i, m);
     }
+}
+
+// ------------------------------------------------------------- calibration forward epilogues
+// The elementwise glue around the convolutions of the fp32 calibration forward, one pass each instead of ATen's two
+// or three (bias add, ReLU) plus the pass-1 re-read of absmax_multi_kernel:
+//   out = a + (bias[channel] or b[i]),   relu_out = relu(out) (optional),   *max_slot = max(*max_slot, bits(max |out|))
+// Bit for bit what the unfused forward computes: one IEEE fp32 add (ATen's a + 1 * b), ReLU as ATen's clamp_min
+// (NaN passes, else max(v, 0)), and absmax_multi_kernel's order-free integer max over |out| bit patterns.
+//   EPI_BIAS4 : the conv epilogue in place (out == a), plane size H*W % 4 == 0: a float4 never leaves its plane, so
+//               its channel is two multiply-shift divisions of the float4 index (hw = float4 per plane)
+//   EPI_BIAS1 : the same for any plane size (7x7): the channel is found for the first element of the float4 and
+//               stepped for the other three (hw = elements per plane)
+//   EPI_ADD   : Eltwise, out = a + b out of place
+// Grid-stride over float4 with kEpiUnroll float4 per operand in flight per thread; n % 4 tail scalars in CTA 0.
+enum EpiMode { EPI_BIAS4 = 0, EPI_BIAS1 = 1, EPI_ADD = 2 };
+constexpr int kEpiUnroll = 4;
+
+struct EpiArgs {
+    const float *a;             // EPI_BIAS*: the conv output, == out
+    const float *b;             // EPI_BIAS*: bias [channels]; EPI_ADD: second addend [n]
+    float *out;
+    float *relu_out;            // may be null
+    unsigned int *max_slot;     // may be null
+    unsigned long long n;       // elements; n / 4 < 2^31 (EPI_BIAS1: n < 2^31)
+    unsigned int hw, channels;
+    unsigned int m_hw, m_chan;  // magic31 multipliers of hw and channels
+    int s_hw, s_chan;
+};
+
+// ATen's clamp_min(v, 0) (launch_clamp_scalar): NaN propagates, otherwise max(v, 0)
+__device__ __forceinline__ float relu_aten(float v) { return isnan(v) ? v : fmaxf(v, 0.0f); }
+
+template <int MODE>
+__device__ __forceinline__ float4 epi_load_a(const EpiArgs &p, unsigned int i)
+{
+    // in place: a coherent streaming load (the same thread overwrites the float4 right after)
+    return MODE == EPI_ADD ? ld_stream_f4(reinterpret_cast<const float4 *>(p.a) + i)
+                           : __ldcs(reinterpret_cast<const float4 *>(p.a) + i);
+}
+
+template <int MODE>
+__device__ __forceinline__ float4 epi_load_b(const EpiArgs &p, unsigned int i)
+{
+    if (MODE == EPI_ADD) return ld_stream_f4(reinterpret_cast<const float4 *>(p.b) + i);
+    if (MODE == EPI_BIAS4) {
+        const unsigned int plane = magic_div(i, p.m_hw, p.s_hw);
+        const unsigned int c = plane - magic_div(plane, p.m_chan, p.s_chan) * p.channels;
+        const float v = __ldg(p.b + c);
+        return make_float4(v, v, v, v);
+    }
+    const unsigned int e = 4u * i;
+    const unsigned int plane = magic_div(e, p.m_hw, p.s_hw);
+    unsigned int rem = e - plane * p.hw;
+    unsigned int c = plane - magic_div(plane, p.m_chan, p.s_chan) * p.channels;
+    float v[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        v[j] = __ldg(p.b + c);
+        if (++rem == p.hw) {
+            rem = 0;
+            if (++c == p.channels) c = 0;
+        }
+    }
+    return make_float4(v[0], v[1], v[2], v[3]);
+}
+
+__device__ __forceinline__ void epi_store(const EpiArgs &p, unsigned int i, const float4 &a, const float4 &b,
+                                          unsigned int &m)
+{
+    const float4 o = make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+    __stcs(reinterpret_cast<float4 *>(p.out) + i, o);
+    if (p.relu_out)
+        reinterpret_cast<float4 *>(p.relu_out)[i] = make_float4(relu_aten(o.x), relu_aten(o.y), relu_aten(o.z),
+                                                                relu_aten(o.w));
+    m = max(max(m, max(absbits(o.x), absbits(o.y))), max(absbits(o.z), absbits(o.w)));
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(kStatThreads)
+epilogue_kernel(const EpiArgs p)
+{
+    __shared__ unsigned int s_warp[kStatThreads / 32];
+    const unsigned int nvec = (unsigned int)(p.n >> 2);
+    const unsigned int stride = gridDim.x * kStatThreads;
+    unsigned int i = blockIdx.x * kStatThreads + threadIdx.x;
+    unsigned int m = 0;
+    for (; i + (kEpiUnroll - 1) * stride < nvec; i += kEpiUnroll * stride) {
+        float4 a[kEpiUnroll], b[kEpiUnroll];
+#pragma unroll
+        for (int u = 0; u < kEpiUnroll; ++u) a[u] = epi_load_a<MODE>(p, i + u * stride);
+#pragma unroll
+        for (int u = 0; u < kEpiUnroll; ++u) b[u] = epi_load_b<MODE>(p, i + u * stride);
+#pragma unroll
+        for (int u = 0; u < kEpiUnroll; ++u) epi_store(p, i + u * stride, a[u], b[u], m);
+    }
+    for (; i < nvec; i += stride) epi_store(p, i, epi_load_a<MODE>(p, i), epi_load_b<MODE>(p, i), m);
+    const unsigned long long t = ((unsigned long long)nvec << 2) + blockIdx.x * kStatThreads + threadIdx.x;
+    if (t < p.n) {                                         // the n % 4 tail: threads 0..2 of CTA 0
+        float b;
+        if (MODE == EPI_ADD) b = p.b[t];
+        else b = __ldg(p.b + (unsigned int)((t / (MODE == EPI_BIAS4 ? 4ull * p.hw : p.hw)) % p.channels));
+        const float o = __fadd_rn(p.a[t], b);
+        p.out[t] = o;
+        if (p.relu_out) p.relu_out[t] = relu_aten(o);
+        m = max(m, absbits(o));
+    }
+    if (p.max_slot) block_max_publish(m, s_warp, p.max_slot);
 }
 
 // --------------------------------------------------------------------------- histogram

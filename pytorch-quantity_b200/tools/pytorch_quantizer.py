@@ -14,19 +14,23 @@ What is different from the reference, by design (B200-first):
     maxima merge with all_reduce(MAX) and the integer histograms with all_reduce(SUM), so the
     tables are bit-identical for any rank count;
   * the KL threshold search for all tensors is one GPU launch sequence;
+  * during calibration the bias add after every cuDNN convolution, each Eltwise and the out-of-place nn.ReLU that
+    follows either run as one native kernel that also takes the pass-1 max-abs (plan_calibration_fusion), with
+    bit-identical results;
   * producer/consumer links are traced by tensor identity instead of a value hash.
 """
 import json
 import math
 import os
 import time
-from collections import OrderedDict
+from collections import Counter, OrderedDict
 
 import numpy as np
 import torch
 import torch.nn as nn
+import torch.nn.functional as F
 
-from common.quantity import DistributionCollector, Quantizer, _native
+from common.quantity import DistributionCollector, Eltwise, Quantizer, _native
 
 from ._config import load_tool_config, load_user_config
 from ._jsonio import dump_int_array
@@ -45,6 +49,152 @@ def _barrier():
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         dist.barrier()
+
+
+def plan_calibration_fusion(net, modules, inplace_modified):
+    """Which modules the calibration forward runs as fused native ops, decided from one trace of
+    Quantity.build_net_structure (``net``: tracer name -> {"inputs", "type"}, ``modules``: tracer name -> module).
+
+    Returns {tracer name: (module, relu)} for every module that fired exactly once, whose output no later op modifies
+    in place, and that is
+      * an nn.Conv2d with the plain nn.Conv2d forward, an fp32 bias and zero padding: cuDNN convolves without the bias
+        and pq_conv_epilogue_f32 adds it, or
+      * an Eltwise: pq_eltwise_add_f32.
+    ``relu`` is the output's only traced nn.ReLU consumer when that ReLU is out of place, has the plain forward and
+    fired once (the fused op then writes its output too), else None.  Without torch's backend selector the fused
+    convolution could not tell whether cuDNN would run it, so no convolution is planned (Eltwise does not depend on
+    it).  What depends on the call (grad mode, autocast, contiguous fp32 tensors on the device, the cuDNN backend)
+    the fused forwards check every time.  Modules outside CARE_OP_TYPE are planned too; their fused ops take no
+    max-abs, since the collector does not observe their outputs."""
+    calls = Counter(id(m) for m in modules.values())
+    consumers = {}
+    for name, info in net.items():
+        for src in info["inputs"]:
+            consumers.setdefault(src, []).append(name)
+
+    def once(m):
+        return calls[id(m)] == 1 and "forward" not in vars(m)
+
+    can_select = hasattr(torch._C, "_select_conv_backend")
+    plan = OrderedDict()
+    for name, m in modules.items():
+        if not once(m) or name in inplace_modified:
+            continue
+        conv = (can_select and isinstance(m, nn.Conv2d) and type(m).forward is nn.Conv2d.forward
+                and type(m)._conv_forward is nn.Conv2d._conv_forward and m.bias is not None
+                and m.bias.dtype == torch.float32 and m.padding_mode == "zeros" and not isinstance(m.padding, str))
+        if not (conv or type(m) is Eltwise):
+            continue
+        relus = [modules[c] for c in consumers.get(name, ()) if isinstance(modules[c], nn.ReLU)]
+        relu = relus[0] if len(relus) == 1 else None
+        if relu is not None and (type(relu).forward is not nn.ReLU.forward or relu.inplace or not once(relu)):
+            relu = None
+        plan[name] = (m, relu)
+    return plan
+
+
+class _CalibrationFusion:
+    """The fused forwards of a plan (plan_calibration_fusion) for one activation_quantize call: install() sets them as
+    instance attributes, remove() restores the modules.
+
+    Each fused op is one native launch on the stream current at the call.  While ``collect`` is set (pass 1) a fused
+    op whose output the collector observes (``slots``: tensor name -> its max_bits slot) also takes the max |x| of
+    that output into the slot, provided it runs at its traced position in the forward (the calibration hooks' count),
+    and adds the name to ``reduced``; refresh_max_val then skips those tensors.  A fused op that also computed its
+    consumer ReLU's output hands it over only if that ReLU is called with the very tensor, unmodified; any other
+    call runs the ReLU's own forward."""
+
+    def __init__(self, plan, hook_state, slots, device):
+        self.collect = False
+        self.reduced = set()
+        self._state = hook_state
+        self._device = device
+        self._forwards = []         # (module, fused forward), all built before any module is touched
+        for name, (m, relu) in plan.items():
+            stash = [None] if relu is not None else None
+            pos = int(name.rsplit("_", 1)[1])
+            make = self._conv if isinstance(m, nn.Conv2d) else self._eltwise
+            self._forwards.append((m, make(m, name, pos, slots.get(name), stash)))
+            if relu is not None:
+                self._forwards.append((relu, self._relu(relu, stash)))
+        self._patched = []
+
+    def install(self):
+        for m, forward in self._forwards:
+            m.forward = forward
+            self._patched.append(m)
+
+    def remove(self):
+        for m in self._patched:
+            del m.forward
+        self._patched = []
+
+    def _fusable(self, t):
+        return (isinstance(t, torch.Tensor) and t.device == self._device and t.dtype == torch.float32
+                and t.is_contiguous() and t.data_ptr() % 16 == 0)
+
+    def _slot(self, name, pos, slot):
+        if slot is not None and self.collect and self._state["idx"] == pos - 1:
+            self.reduced.add(name)
+            return slot
+        return None
+
+    def _conv(self, m, name, pos, slot, stash):
+        own = m.forward
+        cudnn = {}                  # input shape -> does cuDNN run this convolution (bias included)?
+
+        def on_cudnn(x):
+            # only on the cuDNN backend is the bias a separate add after the convolution (ATen's
+            # output.add_(bias)); the slow and depthwise kernels accumulate it.  A selector that cannot be asked
+            # (a changed private signature) means: not fused.
+            try:
+                return torch._C._select_conv_backend(x, m.weight, m.bias, m.stride, m.padding, m.dilation, False,
+                                                     (0, 0), m.groups) == torch._C._ConvBackend.Cudnn
+            except (TypeError, RuntimeError):
+                return False
+
+        def forward(x):
+            # under autocast the convolution runs in 16 bits with the bias cast alongside: the module's own forward
+            if (torch.is_grad_enabled() or torch.is_autocast_enabled(self._device.type) or not self._fusable(x)
+                    or x.dim() != 4):
+                return own(x)
+            ok = cudnn.get(x.shape)
+            if ok is None:
+                ok = cudnn[x.shape] = on_cudnn(x)
+            if not ok:
+                return own(x)
+            y = F.conv2d(x, m.weight, None, m.stride, m.padding, m.dilation, m.groups)
+            if y.dtype != torch.float32 or not y.is_contiguous():     # (a channels_last weight) ATen's own bias add
+                return y.add_(m.bias.reshape(1, -1, 1, 1))
+            r = _native.conv_epilogue(y, m.bias, stash is not None, self._slot(name, pos, slot))
+            if stash is not None:
+                stash[0] = (y, y._version, r)
+            return y
+        return forward
+
+    def _eltwise(self, m, name, pos, slot, stash):
+        own = m.forward
+
+        def forward(a, b):
+            # (torch.add is not an autocast op: fp32 operands give the fp32 sum with autocast on or off)
+            if torch.is_grad_enabled() or not (self._fusable(a) and self._fusable(b)) or a.shape != b.shape:
+                return own(a, b)
+            z, r = _native.eltwise_add(a, b, stash is not None, self._slot(name, pos, slot))
+            if stash is not None:
+                stash[0] = (z, z._version, r)
+            return z
+        return forward
+
+    @staticmethod
+    def _relu(relu, stash):
+        own = relu.forward
+
+        def forward(x):
+            st, stash[0] = stash[0], None
+            if st is not None and x is st[0] and x._version == st[1]:
+                return st[2]
+            return own(x)
+        return forward
 
 
 class Quantity(object):
@@ -84,6 +234,7 @@ class Quantity(object):
         self.cache_bytes = cache_bytes
         self._begin_forward = lambda: None
         self._inplace_modified = set()
+        self._fuse_calibration = True      # False: the calibration forward runs the model's own forwards only
         self.net_info = self.build_net_structure(self.model, self.input_size, self.device)
         self.cared_op_layer_names = self.get_cared_op_names(self.model)
         self._DKL_weight = False
@@ -106,6 +257,7 @@ class Quantity(object):
         hooks = []
         orphan = []
         observed = []               # (tracer name, tensor, version at hook time): what calibration will record
+        modules = OrderedDict()     # tracer name -> the module that fired
 
         def _hook(m, inputs, output):
             kind = type(m).__name__
@@ -125,6 +277,7 @@ class Quantity(object):
             if not net and inputs and isinstance(inputs[0], torch.Tensor):
                 observed.append(("image", inputs[0], inputs[0]._version))
             net[name] = {"inputs": srcs, "type": kind}
+            modules[name] = m
             producer_of[id(output)] = name    # in-place / pass-through ops take over the tensor
             keep_alive.append((inputs, output))
             if isinstance(output, torch.Tensor):
@@ -145,6 +298,7 @@ class Quantity(object):
         # pre-modification values; the calibration hooks below keep device references and therefore clone
         # exactly these tensors (and only these) to record the same values.
         self._inplace_modified = {n for n, t, v in observed if t._version != v}
+        self._fusion_plan = plan_calibration_fusion(net, modules, self._inplace_modified)
         keep = [n for n, info in net.items() if info["type"] in self._cared_op_type]
         return self.prune_net_info(net, keep)
 
@@ -278,6 +432,7 @@ class Quantity(object):
         versions = {}
         clone = self._inplace_modified
         self._feat_versions = versions
+        self._feat_state = state
 
         def _begin():
             state["idx"] = 0
@@ -352,52 +507,63 @@ class Quantity(object):
 
         t0 = time.perf_counter()
         n_mine = 0
-        for i, img in self._device_batches(images_files):                    # pass 1  (:379-390)
-            self._forward_device(self.model, img)
-            self._check_unmodified(named_feats)
-            feats = {n: named_feats[n] for n in top_feat_names}
-            collector.refresh_max_val(feats)
-            nbytes = sum(t.numel() * t.element_size() for t in feats.values())
-            if cached_bytes + nbytes <= budget:
-                cache[i] = feats
-                cached_bytes += nbytes
-                n_cached += 1
-            n_mine += 1
-        if n_mine == 0:
-            collector.refresh_max_val({n: torch.zeros(0, device=self.cuda_device) for n in top_feat_names})
-        collector.all_reduce_max()
-        self._log("max_vals", collector.max_vals)
-        distribution_intervals = collector.distribution_intervals
-        t1 = time.perf_counter()
-
-        def group_has_eltwise(names):
-            return any(self.net_info[n]["type"] == "Eltwise" for n in names)
-
-        for names in merge_groups:                                           # (:396-411)
-            assert len(names) > 1
-            if group_has_eltwise(names):
-                continue
-            widest = 0
-            for n in names:
-                widest = max(widest, distribution_intervals[n])
-            for n in names:
-                distribution_intervals[n] = widest
-
-        self._log("Collect histograms of activations:")
-        for i, img in self._device_batches(images_files, skip=lambda i: i in cache):   # pass 2  (:415-426)
-            if img is None:
-                feats = cache.pop(i)
-            else:
+        plan = self._fusion_plan if self._fuse_calibration else {}
+        # max slots only for the tensors the collector observes (CARE_OP_TYPE); the other fused ops take no max
+        slots = {n: collector._max_slot(n) for n in plan if n in top_feat_names}
+        fusion = _CalibrationFusion(plan, self._feat_state, slots, self.cuda_device)
+        try:
+            fusion.install()
+            fusion.collect = True
+            for i, img in self._device_batches(images_files):                    # pass 1  (:379-390)
+                fusion.reduced.clear()
                 self._forward_device(self.model, img)
                 self._check_unmodified(named_feats)
                 feats = {n: named_feats[n] for n in top_feat_names}
-            collector.add_to_distributions(feats)
-        if n_mine == 0:
-            collector.add_to_distributions({n: torch.zeros(0, device=self.cuda_device) for n in top_feat_names})
-        cache.clear()
-        collector.all_reduce_hist()
-        for h in hooks:
-            h.remove()
+                collector._refresh_max_val_except(feats, fusion.reduced)
+                nbytes = sum(t.numel() * t.element_size() for t in feats.values())
+                if cached_bytes + nbytes <= budget:
+                    cache[i] = feats
+                    cached_bytes += nbytes
+                    n_cached += 1
+                n_mine += 1
+            if n_mine == 0:
+                collector.refresh_max_val({n: torch.zeros(0, device=self.cuda_device) for n in top_feat_names})
+            collector.all_reduce_max()
+            self._log("max_vals", collector.max_vals)
+            distribution_intervals = collector.distribution_intervals
+            t1 = time.perf_counter()
+
+            def group_has_eltwise(names):
+                return any(self.net_info[n]["type"] == "Eltwise" for n in names)
+
+            for names in merge_groups:                                           # (:396-411)
+                assert len(names) > 1
+                if group_has_eltwise(names):
+                    continue
+                widest = 0
+                for n in names:
+                    widest = max(widest, distribution_intervals[n])
+                for n in names:
+                    distribution_intervals[n] = widest
+
+            self._log("Collect histograms of activations:")
+            fusion.collect = False
+            for i, img in self._device_batches(images_files, skip=lambda i: i in cache):   # pass 2  (:415-426)
+                if img is None:
+                    feats = cache.pop(i)
+                else:
+                    self._forward_device(self.model, img)
+                    self._check_unmodified(named_feats)
+                    feats = {n: named_feats[n] for n in top_feat_names}
+                collector.add_to_distributions(feats)
+            if n_mine == 0:
+                collector.add_to_distributions({n: torch.zeros(0, device=self.cuda_device) for n in top_feat_names})
+            cache.clear()
+            collector.all_reduce_hist()
+        finally:
+            fusion.remove()
+            for h in hooks:
+                h.remove()
         named_feats.clear()                # the last forward's activations (4.3 GB for ResNet-50 at batch 64) go back to the pool
         distributions = collector.distributions
         t2 = time.perf_counter()
