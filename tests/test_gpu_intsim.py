@@ -144,7 +144,8 @@ def test_smallc_conv_vs_oracle_and_im2col(oracle, shape, relu, s2d):
                                    (300, 512, 128), (130, 1024, 64), (64, 2048, 512), (5000, 80, 96)])
 def test_gemm_s8_staged_int8_store(oracle, M, N, K):
     """int8 output through the swizzled shared-memory tile + TMA store (N % 16 == 0), every tile width and ragged
-    M / N edges, with and without the fused ReLU; sentinel bytes around the output must survive."""
+    M / N edges, with and without the fused ReLU.  (Writes outside the output are checked with sentinel-filled
+    buffers in test_gpu_epilogue_matrix.py.)"""
     from common.quantity import _native
     rng = np.random.default_rng(M + N + K)
     a = rng.integers(-128, 128, size=(M, K), dtype=np.int8)
