@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 201
+#define PQ_VERSION 202
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -217,6 +217,17 @@ int pq_gemm_s8(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, i
                int flags, float *out_f32, int8_t *out_s8, pq_stream_t stream);
 int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
                  int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, pq_stream_t stream);
+
+/* ---- a13 + a14 for depthwise convolutions (nn.Conv2d with groups == in_channels == out_channels, wrapped by
+ * NewConv2d): the chain of pq_conv2d_s8 per channel, out[c] = requant(sum_{r,s} x[c] * w[r][s][c]).
+ * x_nhwc is int8 [N][H][W][C], desc.C = padded channel count (C % 16 == 0), desc.K = real channel count (K <= C);
+ * w_rsc is int8 [R][S][C], channel-fastest, zero in channels >= K; bias_q is [K], or [3K] with PQ_FLAG_BIAS_FOLDED.
+ * Flags PQ_FLAG_RELU / PQ_FLAG_BIAS_FOLDED as for pq_conv2d_s8.  Outputs (either may be NULL, not both): fp32 NCHW
+ * [N][K][P][Q], int8 NHWC [N][P][Q][K].  Supports 1 <= R, S <= 7, stride 1 or 2 and dilation 1 or 2 in each
+ * dimension, 0 <= pad <= (R - 1) * dil; anything else is PQ_EUNSUPPORTED (and nothing is written).  x, w_rsc and
+ * out_s8_nhwc 16-byte aligned. */
+int pq_conv2d_dw_s8(const int8_t *x_nhwc, const int8_t *w_rsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
+                    int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, pq_stream_t stream);
 
 /* out: int32 [3 * n] (rows [0], [1], [2] above; n even). */
 int pq_bias_fold_s32(const int32_t *bias_q, int n, int rs, int32_t *out, pq_stream_t stream);

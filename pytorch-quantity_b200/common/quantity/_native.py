@@ -19,7 +19,7 @@ HIST_BINS_MAX = 8192
 KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
-PQ_VERSION = 201             # the header's PQ_VERSION: the entry points below match a library built from it
+PQ_VERSION = 202             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -48,6 +48,7 @@ SYMBOLS = {
     "pq_gemm_s8": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "pq_conv2d_s8": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "pq_conv2d_s8_add": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "pq_conv2d_dw_s8": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "pq_relu_s8": (_i, [_vp, _vp, _sz, _vp]),
     "pq_maxpool_nhwc_s8": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "pq_avgpool_global_nhwc_f32": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
@@ -460,6 +461,42 @@ def conv2d_s8(x_nhwc, w_krsc, bias_q, stride, padding, rs, ob, want_f32=True, wa
                                  _bias_flags(bias_q, K, relu) | (0 if windows else FLAG_NO_WINDOWS),
                                  out_f32.data_ptr() if want_f32 else None,
                                  out_s8.data_ptr() if want_s8 else None, _stream(x_nhwc)), "pq_conv2d_s8")
+    return out_f32, out_s8
+
+
+def conv2d_dw_s8(x_nhwc, w_rsc, bias_q, stride, padding, rs, ob, want_f32=True, want_s8=False, relu=False,
+                 dilation=(1, 1), channels=None):
+    """Depthwise convolution (groups == channels): x_nhwc int8 [N][H][W][C_pad], w_rsc int8 [R][S][C_pad] (zero in the
+    padded channels), bias_q int32 [K] or the folded [3K] of bias_fold -> fp32 NCHW [N][K][P][Q] and / or int8 NHWC
+    [N][P][Q][K].  K, the real channel count, is `channels`; by default the bias length when it is <= C_pad, else a
+    third of it (a folded buffer, which NewConv2d's C_pad = _pad16(K) < 3K always tells apart)."""
+    require_cuda(x_nhwc, "conv2d_dw_s8")
+    for t, dt, what in ((x_nhwc, torch.int8, "x_nhwc"), (w_rsc, torch.int8, "w_rsc"), (bias_q, torch.int32, "bias_q")):
+        if t.device != x_nhwc.device or t.dtype != dt or not t.is_contiguous():
+            raise RuntimeError("conv2d_dw_s8: %s must be a contiguous %s tensor on %s, got %s %s on %s"
+                               % (what, dt, x_nhwc.device, "contiguous" if t.is_contiguous() else "strided", t.dtype,
+                                  t.device))
+    if x_nhwc.dim() != 4 or w_rsc.dim() != 3 or bias_q.dim() != 1:
+        raise RuntimeError("conv2d_dw_s8: x_nhwc [N][H][W][C], w_rsc [R][S][C] and a 1-D bias_q expected, got %s, %s, %s"
+                           % (tuple(x_nhwc.shape), tuple(w_rsc.shape), tuple(bias_q.shape)))
+    N, H, W, C = x_nhwc.shape
+    R, S, C2 = w_rsc.shape
+    if C2 != C:
+        raise RuntimeError("conv2d_dw_s8: %d weight channels for %d input channels" % (C2, C))
+    n_bias = bias_q.numel()
+    K = int(channels) if channels is not None else (n_bias if n_bias <= C else n_bias // 3)
+    if not 0 < K <= C or n_bias not in (K, 3 * K):
+        raise RuntimeError("conv2d_dw_s8: %d bias values for %d (padded) channels" % (n_bias, C))
+    d = _conv_desc(N, H, W, C, K, (R, S), stride, padding, rs, ob, (int(dilation[0]), int(dilation[1])))
+    P, Q = d.P, d.Q
+    out_f32 = torch.empty((N, K, P, Q), dtype=torch.float32, device=x_nhwc.device) if want_f32 else None
+    out_s8 = torch.empty((N, P, Q, K), dtype=torch.int8, device=x_nhwc.device) if want_s8 else None
+    # HBM-bound: the algorithmic bytes (input image once, weights, outputs)
+    nbytes = x_nhwc.numel() + w_rsc.numel() + N * P * Q * K * ((4 if want_f32 else 0) + (1 if want_s8 else 0))
+    with _Timed("conv_dw_s8", 1, nbytes, x_nhwc.device):
+        check(lib().pq_conv2d_dw_s8(x_nhwc.data_ptr(), w_rsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
+                                    _bias_flags(bias_q, K, relu), out_f32.data_ptr() if want_f32 else None,
+                                    out_s8.data_ptr() if want_s8 else None, _stream(x_nhwc)), "pq_conv2d_dw_s8")
     return out_f32, out_s8
 
 

@@ -191,9 +191,14 @@ class NewConv2d(_IntSimBase):
                               per filter row); with _s2d the same kernel on the space-to-depth image (stride 2,
                               <= 4 channels)
       _explicit_im2col        other convolutions with <= 8 channels: explicit im2col matrix -> pq_gemm_s8
-      _group_convs            groups > 1: one NewConv2d per group
+      _depthwise              groups == in_channels == out_channels inside the kernel's limits: int8 NHWC image with
+                              _payload_channels (padded) channels -> pq_conv2d_dw_s8
+      _group_convs            other groups > 1: one NewConv2d per group
     Only this class reads these flags: forward() and the int8 pipeline run the layer through _quantize / _run /
     _run_add."""
+
+    # class-level default: a model pickled before the depthwise kernel existed has _group_convs set and no _depthwise
+    _depthwise = False
 
     def __init__(self, conv_module, quantize_infor):
         super().__init__()
@@ -217,8 +222,17 @@ class NewConv2d(_IntSimBase):
         # whether _run_add can fuse a following NewAdd into this convolution's epilogue
         self._fuses_add = False
         self._group_convs = None
-        self._smallc = self._s2d = self._explicit_im2col = False
+        self._smallc = self._s2d = self._explicit_im2col = self._depthwise = False
         if conv.groups != 1:
+            if _depthwise_fits(conv):
+                # one stencil kernel over the int8 NHWC image; weights [R][S][C_pad], channel-fastest
+                self._depthwise = True
+                self._dilation = tuple(int(d) for d in conv.dilation)
+                self._payload_channels = _pad16(K)
+                w_rsc = torch.zeros((R, S, self._payload_channels), dtype=torch.int8, device=wq.device)
+                w_rsc[..., :K] = wq[:, 0].permute(1, 2, 0).to(torch.int8)
+                self.register_buffer("_w_rsc", w_rsc.contiguous())
+                return
             self._build_groups(conv, wq)
             return
         # im2col TMA fetches channel blocks of 32 / 64 / 128 bytes; a 1x1 stride-1 conv is a plain GEMM
@@ -286,9 +300,9 @@ class NewConv2d(_IntSimBase):
             return conv_forward(self, input)
         return self._run(self._quantize(input), True, False, False)[0]   # Quan, Conv+RightShift+BiasAdd+Sp+DeQuan
 
-    # ---- the layer's launch path (not for grouped layers).  An operand is what _quantize returns: the int8 NHWC image
-    # [N][H][W][_payload_channels] when _payload_channels is set (a producer's int8 payload at input_bit is one, too),
-    # otherwise (int8 tensor in the kernel's layout, (N, H, W) of the input).
+    # ---- the layer's launch path (not for layers on the per-group path).  An operand is what _quantize returns: the
+    # int8 NHWC image [N][H][W][_payload_channels] when _payload_channels is set (a producer's int8 payload at input_bit
+    # is one, too), otherwise (int8 tensor in the kernel's layout, (N, H, W) of the input).
 
     def _quantize(self, x):
         """Quantity(input_bit) of fp32 NCHW x into the operand this layer's kernel reads."""
@@ -324,6 +338,10 @@ class NewConv2d(_IntSimBase):
         """Conv + RightShift + BiasAdd + Sp (+ the nn.ReLU after the layer when relu) on an operand.  Returns
         (fp32 NCHW after DeQuantity or None, int8 NHWC [N][P][Q][K] or None)."""
         conv = self.Conv
+        if self._depthwise:
+            return _native.conv2d_dw_s8(operand, self._w_rsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
+                                        self.output_bit, want_f32=want_f32, want_s8=want_s8, relu=relu,
+                                        dilation=self._dilation, channels=conv.out_channels)
         if self._payload_channels is not None:
             return _native.conv2d_s8(operand, self._w_krsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
                                      self.output_bit, want_f32=want_f32, want_s8=want_s8, c_real=conv.in_channels,
@@ -358,6 +376,14 @@ class NewConv2d(_IntSimBase):
         return _native.conv2d_s8_add(operand, self._w_krsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
                                      self.output_bit, shortcut, shortcut_bit, shortcut_relu, q_bit, relu,
                                      want16=want16, c_real=conv.in_channels)
+
+
+def _depthwise_fits(conv):
+    """A depthwise convolution (channel multiplier 1) of a shape pq_conv2d_dw_s8 implements: R, S <= 7, stride and
+    dilation 1 or 2, 0 <= pad <= (R - 1) * dilation (zero padding is checked by quantity())."""
+    (R, S), (sh, sw), (ph, pw), (dh, dw) = conv.kernel_size, conv.stride, conv.padding, conv.dilation
+    return (conv.groups == conv.in_channels == conv.out_channels and R <= 7 and S <= 7 and sh in (1, 2)
+            and sw in (1, 2) and dh in (1, 2) and dw in (1, 2) and 0 <= ph <= (R - 1) * dh and 0 <= pw <= (S - 1) * dw)
 
 
 def s2d_filter(wq, padding):

@@ -26,6 +26,7 @@
 #include <cstdlib>
 
 #include "pq_common.cuh"
+#include "pq_requant.cuh"
 
 namespace pq {
 
@@ -230,33 +231,11 @@ __device__ __forceinline__ void sts_u4(uint32_t addr, uint32_t a, uint32_t b, ui
 {
     asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
-// Programmatic dependent launch: every kernel here is launched with programmaticStreamSerializationAllowed, lets its
-// successor start as soon as this grid's CTAs have been scheduled (launch_dependents) and touches global memory only
-// after its predecessor has completed and flushed (wait).  A CTA of the next kernel lands on an SM as soon as this
-// kernel's CTA there has exited (one CTA per SM: shared memory), so its barrier / TMEM / tensor-map set-up overlaps the
-// tail of this kernel instead of following the launch latency.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void epi_bar_sync(int threads)
 {
     asm volatile("bar.sync 1, %0;" ::"r"(threads) : "memory");
-}
-// sat_s8(y0) | sat_s8(y1) << 8 | sat_s8(y2) << 16 | sat_s8(y3) << 24   (two I2IP.S8.S32.SAT)
-__device__ __forceinline__ uint32_t pack4_sat_s8(int y0, int y1, int y2, int y3)
-{
-    uint32_t t, w;
-    asm("cvt.pack.sat.s8.s32.b32 %0, %1, %2, %3;" : "=r"(t) : "r"(y3), "r"(y2), "r"(0));
-    asm("cvt.pack.sat.s8.s32.b32 %0, %1, %2, %3;" : "=r"(w) : "r"(y1), "r"(y0), "r"(t));
-    return w;
-}
-// byte permute with sign replication (selector nibble bit 3): sign-extends one packed int8 / int16 lane
-__device__ __forceinline__ int prmt_sx(uint32_t w, uint32_t sel)
-{
-    uint32_t d;
-    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(w), "r"(0u), "r"(sel));
-    return (int)d;
 }
 __device__ __forceinline__ uint4 ldg_nc_u4(const void *p)
 {
@@ -384,42 +363,12 @@ struct GemmParams {
     int8_t *out_s8;            // optional, [M][N]
 };
 
-// RightShift (round half away from zero, saturate) + BiasAdd + Sp, all in integers, branch-free:
-//   rs >= 1:  round_half_away(acc / 2^rs) = (acc + 2^(rs-1) - (acc < 0)) >> rs   (arithmetic shift)
-//   rs <= 0:  acc * 2^-rs, saturated first (the shift is monotone)
-struct Requant {
-    int half, sh, mul, lo;     // rs >= 1: half = 2^(rs-1), sh = rs, mul unused; rs <= 0: mul = 2^-rs
-    bool pos;
-};
-__device__ __forceinline__ Requant make_requant(int rs, int relu)
-{
-    Requant q;
-    q.lo = relu ? 0 : -128;
-    q.pos = rs >= 1;
-    q.half = rs >= 1 ? (1 << (rs - 1)) : 0;
-    q.sh = rs >= 1 ? rs : 0;
-    q.mul = rs >= 1 ? 1 : (1 << (-rs));
-    return q;
-}
-// result is saturated from below (q.lo = -128, or 0 when a ReLU is fused) but NOT from above: callers
-// finish with min(., 127) or with the saturating pack
-__device__ __forceinline__ int requant_nohi(int acc, const Requant &q, int bias)
-{
-    int r;
-    if (q.pos) r = (acc + q.half + (acc >> 31)) >> q.sh;
-    else r = max(-128, min(127, acc)) * q.mul;
-    r = max(-128, min(127, r));
-    return __viaddmax_s32(r, bias, q.lo);           // max(r + bias, lo) in one VIADDMNMX
-}
-__device__ __forceinline__ int requant(int acc, const Requant &q, int bias)
-{
-    return min(127, requant_nohi(acc, q, bias));
-}
-
 // Accumulator stages in TMEM (<= 512 columns) == groups of epilogue warps working on different tiles.
 // FAST (int8-only, staged) epilogues are instruction-bound: 2-4 tiles in flight, one warp per (tile, lane
 // quadrant[, column half]).  The generic epilogue (fp32 NCHW stores, unstaged int8) is store-bound and
 // does best when all 16 warps drain ONE tile at a time (its 128 x BN x 4 bytes leave as one burst).
+// (the RightShift -> BiasAdd -> Sp chain itself, Requant / requant_t / requant_folded, is in pq_requant.cuh: the
+// depthwise kernel of pq_depthwise.cu shares it)
 template <int BN, bool FAST = true> struct EpiCfg {
     static constexpr int kAcc = (FAST && BN < 256) ? 4 : 2;            // TMEM accumulator stages
     static constexpr int kGroups = FAST ? kAcc : (BN >= 64 ? 1 : 2);   // warp groups on different tiles
@@ -461,33 +410,6 @@ struct GemmSmem {
 // and either de-quantise to fp32 NCHW (the module boundary of the reference, lanes = consecutive pixels)
 // and / or pack to int8 and leave through a swizzled shared-memory tile + TMA store (full 128-byte lines;
 // the TMA clips rows >= M and columns >= N).
-template <bool POS>
-__device__ __forceinline__ int requant_t(int acc, const Requant &q, int bias)
-{
-    int r;
-    if (POS) r = (acc + q.half + (acc >> 31)) >> q.sh;        // VIADD, LEA.HI.SX32, SHF
-    else r = max(-128, min(127, acc)) * q.mul;
-    r = max(-128, min(127, r));                               // first saturation (RightShift)
-    return __viaddmax_s32(r, bias, q.lo);                     // max(r + bias, lo); callers saturate from above
-}
-
-// The same chain with BiasAdd folded into the rounding add (PQ_FLAG_BIAS_FOLDED, rs >= 1): b << rs is a multiple
-// of 2^rs, so with the per-channel constant c = 2^(rs-1) + (b << rs)
-//   (acc + c + (acc >> 31)) >> rs  ==  round_half_away(acc / 2^rs) + b,
-// and because the rounding is monotone the first saturation can be applied to the accumulator instead, with
-// channel-independent bounds:  clamp(r, -128, 127) == r(clamp(acc, -128 * 2^rs - 2^(rs-1) + 1, 127 * 2^rs + 2^(rs-1) - 1)).
-// The second saturation is the packing instruction's.  With a fused ReLU the lower bound is redundant (anything
-// below it ends at 0 either way).  5 ALU operations per element instead of 6, with the same single per-channel
-// constant vector as the classic chain; the CPU test suite checks the identities over every (rs, b) and the
-// accumulators around both bounds.
-template <bool RELU>
-__device__ __forceinline__ int requant_folded(int acc, int sh, int a_lo, int a_hi, int c)
-{
-    const int a = RELU ? min(acc, a_hi) : max(min(acc, a_hi), a_lo);
-    const int t = (a + c + (a >> 31)) >> sh;
-    return RELU ? max(t, 0) : t;
-}
-
 // Round 2: the saturations of the folded chain move BEHIND the shift, onto packed 16-bit pairs.  With
 //   t = (acc + c + (acc >> 31)) >> rs = r + b        (r = round_half_away(acc / 2^rs), NOT saturated)
 // the reference's  Sp(Sp(r) + b)  is  clamp(t, l, h)  with the per-channel bounds  h = 127 + min(b, 0),
@@ -1514,22 +1436,6 @@ int num_sms()
     return n;
 }
 
-// cudaLaunchKernelEx with programmatic stream serialisation (see pdl_wait); PQ_NO_PDL=1 in the environment turns the
-// attribute off (the kernels' griddepcontrol instructions are then no-ops)
-template <typename... KArgs, typename... Args>
-int launch_pdl(void (*kern)(KArgs...), int grid, size_t smem, cudaStream_t s, Args &&...args)
-{
-    static const bool no_pdl = [] { const char *e = getenv("PQ_NO_PDL"); return e && e[0] == '1'; }();
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)pq::kGemmThreads);
-    cfg.dynamicSmemBytes = smem; cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = no_pdl ? 0 : 1;
-    return (int)cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
-}
-
 // one gemm_s8_kernel instance (opted in to its shared memory on first use) on a persistent grid: one CTA per SM
 template <int BN, int BK, int STAGES, bool ADDK, int BSLOTS>
 int launch_gemm(const CUtensorMap &ta, const CUtensorMap &tb, const CUtensorMap &to, const CUtensorMap &tsc,
@@ -1545,7 +1451,7 @@ int launch_gemm(const CUtensorMap &ta, const CUtensorMap &tb, const CUtensorMap 
     }
     const long long tiles = (long long)((p.M + pq::kBM - 1) / pq::kBM) * ((p.N + BN - 1) / BN);
     const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
-    return launch_pdl(kern, grid, Cfg::kTotal, s, ta, tb, to, tsc, to16, p);
+    return launch_pdl(kern, dim3((unsigned)grid), pq::kGemmThreads, Cfg::kTotal, s, ta, tb, to, tsc, to16, p);
 }
 
 template <int BN, int BK, int STAGES, int BSLOTS = STAGES>
@@ -1870,7 +1776,7 @@ extern "C" int pq_conv2d_smallc_s8(const int8_t *xp, const int8_t *w_krs8, const
             }
             const long long tiles = tiles_m * n_tiles;
             const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
-            return launch_pdl(pq::conv_rows_s8_kernel, grid, smem, (cudaStream_t)stream, tb, to, q, rp);
+            return launch_pdl(pq::conv_rows_s8_kernel, dim3((unsigned)grid), pq::kGemmThreads, smem, (cudaStream_t)stream, tb, to, q, rp);
         }
     }
     // A: (byte in window, output column, row group, row phase, image); the column step overlaps the windows
