@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 202
+#define PQ_VERSION 203
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -180,16 +180,28 @@ int pq_quantize_nchw_to_padded_nhwc8_s8(const float *x, int8_t *q, int N, int C,
  * (p*stride_h - pad_h + r*dil_h, q*stride_w - pad_w + s*dil_w).  Dilated filters (nn.Conv2d(dilation=...) wrapped by
  * NewConv2d; the reference's weight path zero-stuffs such kernels for its target hardware,
  * tools/pytorch_quantizer.py:626-629,679-693) take the im2col-TMA path with the dilation as tap offsets, so no
- * multiply is wasted on stuffed zeros; a 1x1 filter ignores the dilation. */
+ * multiply is wasted on stuffed zeros; a 1x1 filter ignores the dilation.
+ *
+ * Grouped convolutions (desc.groups = G > 1; nn.Conv2d(groups=G) wrapped by NewConv2d), Cg = C / G input and
+ * Kg = K / G output channels per group, run in the same single launch: output-channel tile t of B = group_block
+ * channels reads only the contiguous input-channel window [(t*B / Kg) * Cg, + Wb) of the groups it covers,
+ * Wb = Cg * max(1, B / Kg).  The weights are int8 [K][R][S][Wb]: row k holds its group's Cg channels at that group's
+ * offset inside its tile's window (k / Kg * Cg - window origin) and zeros elsewhere, so the tensor cores issue
+ * max(1, B / Kg) times the useful work.  Requires G | C, G | K, desc.C == C (no channel padding),
+ * B in {32, 64, 128, 256} a multiple or a divisor of Kg, K % B == 0 and Wb % 16 == 0 for the 1x1 stride-1 GEMM path,
+ * Wb % 32 == 0 otherwise (else PQ_EUNSUPPORTED; G not dividing C or K, or groups < 0: PQ_EINVAL).
+ * pq_conv2d_s8_add does not take grouped layers (PQ_EUNSUPPORTED). */
 typedef struct pq_conv_desc {
     int N, H, W, C;          /* input NHWC, C = padded channel count (multiple of 16) */
     int K;                   /* output channels */
-    int R, S;                /* filter height / width; weights are [K][R][S][C] int8 */
+    int R, S;                /* filter height / width; weights are [K][R][S][C] int8 (grouped: [K][R][S][Wb]) */
     int stride_h, stride_w, pad_h, pad_w;
     int P, Q;                /* output height / width: (H + 2*pad_h - ((R-1)*dil_h + 1)) / stride_h + 1, Q alike */
     int rs;                  /* weight_bit + input_bit - output_bit, any sign */
     int ob;                  /* output_bit */
     int dil_h, dil_w;        /* dilation, >= 1 */
+    int groups;              /* 0 or 1: a dense layer; G > 1: a grouped convolution (above) */
+    int group_block;         /* grouped: output channels of one tile (B above); ignored for a dense layer */
 } pq_conv_desc;
 
 /* flags of the GEMM / conv entry points (0: the layer as above).

@@ -19,7 +19,7 @@ HIST_BINS_MAX = 8192
 KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
-PQ_VERSION = 202             # the header's PQ_VERSION: the entry points below match a library built from it
+PQ_VERSION = 203             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -65,7 +65,7 @@ class ConvDesc(ctypes.Structure):
     """struct pq_conv_desc"""
     _fields_ = [(n, ctypes.c_int) for n in
                 ("N", "H", "W", "C", "K", "R", "S", "stride_h", "stride_w", "pad_h", "pad_w",
-                 "P", "Q", "rs", "ob", "dil_h", "dil_w")]
+                 "P", "Q", "rs", "ob", "dil_h", "dil_w", "groups", "group_block")]
 
 
 class AddDesc(ctypes.Structure):
@@ -301,10 +301,16 @@ def conv_out_size(in_hw, kernel, stride, padding, dilation=(1, 1)):
             (in_hw[1] + 2 * padding[1] - (kernel[1] - 1) * dilation[1] - 1) // stride[1] + 1)
 
 
-def _conv_desc(N, H, W, C, K, kernel, stride, padding, rs, ob, dilation=(1, 1)):
+def _conv_desc(N, H, W, C, K, kernel, stride, padding, rs, ob, dilation=(1, 1), groups=1, group_block=0):
     P, Q = conv_out_size((H, W), kernel, stride, padding, dilation)
     return ConvDesc(N, H, W, C, K, kernel[0], kernel[1], stride[0], stride[1], padding[0], padding[1], P, Q,
-                    int(rs), int(ob), dilation[0], dilation[1])
+                    int(rs), int(ob), dilation[0], dilation[1], int(groups), int(group_block))
+
+
+def group_window(C, K, groups, group_block):
+    """Wb: the input channels one output-channel tile of a grouped convolution reads (include/pq_sm100.h)."""
+    Cg, Kg = C // groups, K // groups
+    return Cg * max(1, group_block // Kg)
 
 
 def _bias_flags(bias_q, n, relu):
@@ -446,17 +452,40 @@ def gemm_s8(a, w, bias_q, rs, ob, hw=1, want_f32=True, want_s8=False, k_real=Non
 
 
 def conv2d_s8(x_nhwc, w_krsc, bias_q, stride, padding, rs, ob, want_f32=True, want_s8=False, c_real=None,
-              relu=False, dilation=(1, 1), windows=True):
+              relu=False, dilation=(1, 1), windows=True, groups=1, group_block=0):
+    """x_nhwc int8 [N][H][W][C], w_krsc int8 [K][R][S][C] (groups > 1: [K][R][S][Wb] as grouped_filter builds it for
+    group_block), bias_q int32 [K] or the folded [3K] of bias_fold -> fp32 NCHW [N][K][P][Q] and / or int8 NHWC
+    [N][P][Q][K]."""
     require_cuda(x_nhwc, "conv2d_s8")
     N, H, W, C = x_nhwc.shape
     K, R, S, C2 = w_krsc.shape
-    assert C == C2
+    groups = int(groups)
+    if groups > 1:
+        # the kernel addresses by the descriptor alone: reject what it would misread
+        for t, dt, what in ((x_nhwc, torch.int8, "x_nhwc"), (w_krsc, torch.int8, "w_krsc"),
+                            (bias_q, torch.int32, "bias_q")):
+            if t.device != x_nhwc.device or t.dtype != dt or not t.is_contiguous():
+                raise RuntimeError("conv2d_s8: %s must be a contiguous %s tensor on %s, got %s %s on %s"
+                                   % (what, dt, x_nhwc.device, "contiguous" if t.is_contiguous() else "strided",
+                                      t.dtype, t.device))
+        if C % groups or K % groups or (c_real is not None and c_real != C):
+            raise RuntimeError("conv2d_s8: %d groups need unpadded input channels (C = %d, c_real = %s) and K = %d "
+                               "divisible by them" % (groups, C, c_real, K))
+        wb = group_window(C, K, groups, group_block)
+        if C2 != wb or bias_q.numel() not in (K, 3 * K):
+            raise RuntimeError("conv2d_s8: grouped weights [K][R][S][%d] and %d or %d bias values expected for "
+                               "group_block %d, got %s and %d" % (wb, K, 3 * K, group_block, tuple(w_krsc.shape),
+                                                                  bias_q.numel()))
+        ops = 2 * N * K * R * S * (C // groups)          # times P * Q below: the useful work, not the window
+    else:
+        assert C == C2
+        ops = 2 * N * K * R * S * (c_real or C)
     dilation = (int(dilation[0]), int(dilation[1])) if (R, S) != (1, 1) else (1, 1)
-    d = _conv_desc(N, H, W, C, K, (R, S), stride, padding, rs, ob, dilation)
+    d = _conv_desc(N, H, W, C, K, (R, S), stride, padding, rs, ob, dilation, groups, group_block)
     P, Q = d.P, d.Q
     out_f32 = torch.empty((N, K, P, Q), dtype=torch.float32, device=x_nhwc.device) if want_f32 else None
     out_s8 = torch.empty((N, P, Q, K), dtype=torch.int8, device=x_nhwc.device) if want_s8 else None
-    with _Timed("conv_s8", 1, 2 * N * P * Q * K * R * S * (c_real or C), x_nhwc.device):   # int8 ops
+    with _Timed("conv_s8", 1, ops * P * Q, x_nhwc.device):   # int8 ops
         check(lib().pq_conv2d_s8(x_nhwc.data_ptr(), w_krsc.data_ptr(), bias_q.data_ptr(), ctypes.byref(d),
                                  _bias_flags(bias_q, K, relu) | (0 if windows else FLAG_NO_WINDOWS),
                                  out_f32.data_ptr() if want_f32 else None,

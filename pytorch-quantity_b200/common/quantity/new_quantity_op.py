@@ -193,12 +193,18 @@ class NewConv2d(_IntSimBase):
       _explicit_im2col        other convolutions with <= 8 channels: explicit im2col matrix -> pq_gemm_s8
       _depthwise              groups == in_channels == out_channels inside the kernel's limits: int8 NHWC image with
                               _payload_channels (padded) channels -> pq_conv2d_dw_s8
-      _group_convs            other groups > 1: one NewConv2d per group
+      _group_block            other groups > 1 where _grouped_fits (>= 2 input channels per group): int8 NHWC image
+                              of in_channels (unpadded) channels -> pq_conv2d_s8 with groups, one launch, output-channel
+                              tiles of _group_block channels over grouped_filter weights
+      _group_convs            the remaining groups > 1 (channel multiplier > 1 with one input channel per group,
+                              shapes outside _grouped_fits): one NewConv2d per group
     Only this class reads these flags: forward() and the int8 pipeline run the layer through _quantize / _run /
     _run_add."""
 
-    # class-level default: a model pickled before the depthwise kernel existed has _group_convs set and no _depthwise
+    # class-level defaults: a model pickled before the depthwise / grouped kernels existed has _group_convs set and
+    # neither attribute
     _depthwise = False
+    _group_block = 0
 
     def __init__(self, conv_module, quantize_infor):
         super().__init__()
@@ -223,6 +229,7 @@ class NewConv2d(_IntSimBase):
         self._fuses_add = False
         self._group_convs = None
         self._smallc = self._s2d = self._explicit_im2col = self._depthwise = False
+        self._group_block = 0
         if conv.groups != 1:
             if _depthwise_fits(conv):
                 # one stencil kernel over the int8 NHWC image; weights [R][S][C_pad], channel-fastest
@@ -232,6 +239,12 @@ class NewConv2d(_IntSimBase):
                 w_rsc = torch.zeros((R, S, self._payload_channels), dtype=torch.int8, device=wq.device)
                 w_rsc[..., :K] = wq[:, 0].permute(1, 2, 0).to(torch.int8)
                 self.register_buffer("_w_rsc", w_rsc.contiguous())
+                return
+            if _grouped_fits(conv):
+                # one launch of the GEMM kernel over the whole layer; the weight layout depends on the tile width
+                self._group_block = _group_block(conv)
+                self._payload_channels = conv.in_channels
+                self.register_buffer("_w_krsc", grouped_filter(wq, conv.groups, self._group_block))
                 return
             self._build_groups(conv, wq)
             return
@@ -343,9 +356,11 @@ class NewConv2d(_IntSimBase):
                                         self.output_bit, want_f32=want_f32, want_s8=want_s8, relu=relu,
                                         dilation=self._dilation, channels=conv.out_channels)
         if self._payload_channels is not None:
+            grouped = self._group_block != 0
             return _native.conv2d_s8(operand, self._w_krsc, self._bias_i32, conv.stride, conv.padding, self.rs_bit,
                                      self.output_bit, want_f32=want_f32, want_s8=want_s8, c_real=conv.in_channels,
-                                     relu=relu, dilation=self._dilation)
+                                     relu=relu, dilation=self._dilation, groups=conv.groups if grouped else 1,
+                                     group_block=self._group_block)
         t = operand[0]
         N, K, P, Q = self._out_shape(operand)
         if self._explicit_im2col:
@@ -384,6 +399,53 @@ def _depthwise_fits(conv):
     (R, S), (sh, sw), (ph, pw), (dh, dw) = conv.kernel_size, conv.stride, conv.padding, conv.dilation
     return (conv.groups == conv.in_channels == conv.out_channels and R <= 7 and S <= 7 and sh in (1, 2)
             and sw in (1, 2) and dh in (1, 2) and dw in (1, 2) and 0 <= ph <= (R - 1) * dh and 0 <= pw <= (S - 1) * dw)
+
+
+def _plain(conv):
+    """A 1x1 stride-1 unpadded convolution: the kernel runs it as a plain GEMM over the NHWC image."""
+    return tuple(conv.kernel_size) == (1, 1) and tuple(conv.stride) == (1, 1) and tuple(conv.padding) == (0, 0)
+
+
+def _group_block(conv):
+    """The output-channel tile width of the grouped kernel for this layer, or None when no width is legal
+    (include/pq_sm100.h): the one that wastes the fewest tensor-core operations (max(1, width / Kg) times the useful
+    work), the widest among those (fewer re-reads of the input window)."""
+    G, C, K = conv.groups, conv.in_channels, conv.out_channels
+    Cg, Kg = C // G, K // G
+    box = 16 if _plain(conv) else 32
+    best = None
+    for b in (256, 128, 64, 32):
+        wb = _native.group_window(C, K, G, b)
+        if (b % Kg and Kg % b) or K % b or wb % box:
+            continue
+        if best is None or max(1, b // Kg) < max(1, best // Kg):
+            best = b
+    return best
+
+
+def _grouped_fits(conv):
+    """A grouped convolution the GEMM kernel runs in one launch: >= 2 input channels per group (one channel per group
+    is depthwise or a channel multiplier), unpadded channels in whole TMA boxes (C % 32 == 0; 16 for a 1x1 stride-1
+    GEMM) and a legal tile width."""
+    G, C, K = conv.groups, conv.in_channels, conv.out_channels
+    return (G > 1 and C % G == 0 and K % G == 0 and C // G >= 2 and C % (16 if _plain(conv) else 32) == 0
+            and _group_block(conv) is not None)
+
+
+def grouped_filter(wq, groups, group_block):
+    """Integer filter [K][Cg][R][S] of a grouped convolution -> int8 [K][R][S][Wb], the layout pq_conv2d_s8 reads for
+    output-channel tiles of group_block channels: the tile starting at channel n0 reads the input-channel window that
+    starts at (n0 // Kg) * Cg, Wb = Cg * max(1, group_block // Kg) channels wide, and row k holds its group's Cg
+    channels at that group's offset inside the window, zeros elsewhere."""
+    K, Cg, R, S = wq.shape
+    Kg = K // groups
+    wb = Cg * max(1, group_block // Kg)
+    k = torch.arange(K, device=wq.device)
+    off = (k // Kg) * Cg - (k // group_block * group_block // Kg) * Cg          # group origin - window origin
+    idx = (off[:, None] + torch.arange(Cg, device=wq.device))[:, None, None, :].expand(K, R, S, Cg)
+    w = torch.zeros((K, R, S, wb), dtype=torch.int8, device=wq.device)
+    w.scatter_(3, idx, wq.permute(0, 2, 3, 1).to(torch.int8))
+    return w.contiguous()
 
 
 def s2d_filter(wq, padding):

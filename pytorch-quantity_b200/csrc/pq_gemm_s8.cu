@@ -361,6 +361,10 @@ struct GemmParams {
     const uint32_t *bias_hl;   // PQ_FLAG_BIAS_FOLDED: [N/2] s16x2 pairs 127 + min(b, 0), then [N/2] pairs -128 + max(b, 0)
     float *out_f32;            // optional
     int8_t *out_s8;            // optional, [M][N]
+    // Grouped convolution (modes 0 and 1): n tile t reads the input channels [(t / g_tpg) * g_wb, + g_wb), the
+    // channel window of the groups it covers; the weights are stored block-diagonally over that window, so the K loop
+    // is over g_wb bytes.  g_wb = 0: a dense layer (window origin 0).
+    int g_wb, g_tpg;
 };
 
 // Accumulator stages in TMEM (<= 512 columns) == groups of epilogue warps working on different tiles.
@@ -918,13 +922,14 @@ __device__ __forceinline__ void produce_a(const GemmParams &p, const CUtensorMap
     const uint32_t a_base = smem_u32(smem_a), full_base = smem_u32(full_bar);
     // Tile -> coordinate divisions are done 32 tiles at a time, one tile per lane, and handed to the
     // (warp-uniform) issue loop with shuffles: the divisions were 40 % of this warp's instruction stream.
-    int l_m0 = 0, l_nb = 0, l_hp = 0, l_wq = 0;
+    int l_m0 = 0, l_nb = 0, l_hp = 0, l_wq = 0, l_c0 = 0;
     int it = 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
         if ((it & 31) == 0) {
             const int t = tile + lane * (int)gridDim.x;            // tiles beyond the end are never fetched
             const int mt = n_tiles == 1 ? t : t / n_tiles;
             l_m0 = mt * kBM;
+            if (MODE != 2 && p.g_wb) l_c0 = ((t - mt * n_tiles) / p.g_tpg) * p.g_wb;   // grouped: channel window
             if (MODE == 1) {                   // first output pixel of the tile -> input coords
                 l_nb = l_m0 / pq;
                 const int rem = l_m0 - l_nb * pq;
@@ -940,6 +945,7 @@ __device__ __forceinline__ void produce_a(const GemmParams &p, const CUtensorMap
             }
         }
         const int m0 = __shfl_sync(0xffffffffu, l_m0, it & 31);
+        const int c0 = (MODE != 2 && p.g_wb) ? __shfl_sync(0xffffffffu, l_c0, it & 31) : 0;
         int wq = 0, hp = 0, nb = 0;
         if (MODE != 0) {
             nb = __shfl_sync(0xffffffffu, l_nb, it & 31);
@@ -959,10 +965,10 @@ __device__ __forceinline__ void produce_a(const GemmParams &p, const CUtensorMap
                     if (MODE == 2)             // filter row kb: padded input row = p * stride_h + kb
                         tma_load_5d_a(tmap_a, bar, dst, 0, wq, hp + kb / p.stride_h, kb % p.stride_h, nb);
                     else if (MODE == 1)
-                        tma_load_im2col_4d_a(tmap_a, bar, dst, cb * BK, w0, h0, nb, (uint16_t)(s * p.dil_w),
+                        tma_load_im2col_4d_a(tmap_a, bar, dst, c0 + cb * BK, w0, h0, nb, (uint16_t)(s * p.dil_w),
                                              (uint16_t)(r * p.dil_h));
                     else
-                        tma_load_2d_a(tmap_a, bar, dst, kb * BK, m0);
+                        tma_load_2d_a(tmap_a, bar, dst, c0 + kb * BK, m0);
                 }
                 if (MODE == 1) { if (++cb == p.cblocks) { cb = 0; if (++s == p.S) { s = 0; ++r; } } }
             }
@@ -1576,8 +1582,15 @@ int apply_add(pq::GemmParams &p, const pq_add_desc *add, int conv_ob)
     return PQ_OK;
 }
 
+// a grouped layer, validated by conv_impl: K loop over wb bytes (the weights' row length), n tiles of `block` output
+// channels, tile t reading the input channels [(t / tpg) * wb, + wb) (GemmParams::g_wb)
+struct Grouping {
+    int wb, tpg, block;
+};
+
 int gemm_impl(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, int N, int K, int rs, int ob, int hw,
-              int flags, float *out_f32, int8_t *out_s8, const pq_add_desc *add, pq_stream_t stream)
+              int flags, float *out_f32, int8_t *out_s8, const pq_add_desc *add, pq_stream_t stream,
+              const Grouping *grp = nullptr)
 {
     if (M <= 0 || N <= 0 || K <= 0 || hw <= 0) return PQ_EINVAL;
     if (!a || !w || !bias_q || (!out_f32 && !out_s8)) return PQ_EINVAL;
@@ -1586,14 +1599,18 @@ int gemm_impl(const int8_t *a, const int8_t *w, const int32_t *bias_q, int M, in
     if ((uintptr_t)bias_q & 15) return PQ_EALIGN;
     int rc = load_driver_entry_points();
     if (rc != PQ_OK) return rc;
-    const int bk = K >= 128 ? 128 : (K >= 64 ? 64 : 32);
-    int bn = pick_bn(M, N);
+    // grouped: the K tail of a window is zero-filled in the weights' map only; the A bytes it reads (the next group's
+    // channels) meet zero weights
+    const int kw = grp ? grp->wb : K;
+    const int bk = kw >= 128 ? 128 : (kw >= 64 ? 64 : 32);
+    int bn = grp ? grp->block : pick_bn(M, N);
     if (add && bn < 64) bn = 64;                 // the fused-add pass works on 64-column slabs
     CUtensorMap ta, tb;
     if ((rc = encode_2d(&ta, a, K, M, K, bk, pq::kBM)) != PQ_OK) return rc;
-    if ((rc = encode_2d(&tb, w, K, N, K, bk, bn)) != PQ_OK) return rc;
+    if ((rc = encode_2d(&tb, w, kw, N, kw, bk, bn)) != PQ_OK) return rc;
     pq::GemmParams p = {};
-    p.M = M; p.N = N; p.num_kb = (K + bk - 1) / bk; p.a_im2col = 0;
+    p.M = M; p.N = N; p.num_kb = (kw + bk - 1) / bk; p.a_im2col = 0;
+    if (grp) { p.g_wb = grp->wb; p.g_tpg = grp->tpg; }
     set_epilogue(p, bias_q, rs, ob, hw, flags, out_f32, out_s8);
     if ((rc = apply_add(p, add, ob)) != PQ_OK) return rc;
     return launch(ta, tb, p, bk, bn, (cudaStream_t)stream);
@@ -1616,16 +1633,30 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
     if ((uintptr_t)bias_q & 15) return PQ_EALIGN;
     const long long M = (long long)d.N * d.P * d.Q;
     if (M > 0x7fffffffLL) return PQ_EUNSUPPORTED;
-    if (d.R == 1 && d.S == 1 && d.stride_h == 1 && d.stride_w == 1 && d.pad_h == 0 && d.pad_w == 0)
+    const bool plain = d.R == 1 && d.S == 1 && d.stride_h == 1 && d.stride_w == 1 && d.pad_h == 0 && d.pad_w == 0;
+    Grouping grp = {0, 1, 0};
+    const bool grouped = d.groups > 1;
+    if (d.groups < 0) return PQ_EINVAL;
+    if (grouped) {                                                   // weights [K][R][S][Wb], see the header
+        if (add) return PQ_EUNSUPPORTED;
+        if (d.C % d.groups || d.K % d.groups) return PQ_EINVAL;
+        const int cg = d.C / d.groups, kg = d.K / d.groups, b = d.group_block;
+        if ((b != 32 && b != 64 && b != 128 && b != 256) || (b % kg && kg % b) || d.K % b) return PQ_EUNSUPPORTED;
+        grp.wb = cg * (b > kg ? b / kg : 1);
+        grp.tpg = kg > b ? kg / b : 1;
+        grp.block = b;
+        if (grp.wb % (plain ? 16 : 32)) return PQ_EUNSUPPORTED;     // box width of the path below
+    }
+    if (plain)                                                       // 1x1 stride-1: a plain GEMM over NHWC
         return gemm_impl(x_nhwc, w_krsc, bias_q, (int)M, d.K, d.C, d.rs, d.ob, d.P * d.Q, flags, out_f32_nchw,
-                         out_s8_nhwc, add, stream);                  // 1x1 stride-1: a plain GEMM over NHWC
+                         out_s8_nhwc, add, stream, grouped ? &grp : nullptr);
     if (d.C & 31) return PQ_EUNSUPPORTED;                            // im2col path: channel blocks of >= 32
     int rc = load_driver_entry_points();
     if (rc != PQ_OK) return rc;
     // 3x3 / stride 1 / pad 1 with one K block per tap and one n tile (ResNet: C = 64 at 56x56, C = 128 at 28x28): patch
     // windows (GemmParams, a_im2col == 3).  The im2col gather re-reads every input byte nine times out of L2 and bounds
     // these layers at ~9.5 TB/s of L2 -> SM traffic; the window box is read (TH + 2) / TH times.
-    if (!add && !(flags & PQ_FLAG_NO_WINDOWS) && d.R == 3 && d.S == 3 && d.stride_h == 1 && d.stride_w == 1 &&
+    if (!add && !grouped && !(flags & PQ_FLAG_NO_WINDOWS) && d.R == 3 && d.S == 3 && d.stride_h == 1 && d.stride_w == 1 &&
         d.pad_h == 1 && d.pad_w == 1 && d.dil_h == 1 && d.dil_w == 1 &&
         ((d.C == 64 && d.K <= 64) || (d.C == 128 && d.K > 64 && d.K <= 128)) && d.W + 2 <= 64) {
         const int tw_shift = d.W + 2 <= 16 ? 4 : (d.W + 2 <= 32 ? 5 : 6);
@@ -1655,15 +1686,17 @@ int conv_impl(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias_q,
                              : launch_cfg<128, 128, 3, 9>(ta, tb, p, (cudaStream_t)stream);
         }
     }
-    const int bk = (d.C % 128 == 0) ? 128 : ((d.C % 64 == 0) ? 64 : 32);
-    int bn = pick_bn(M, d.K);
+    const int cw = grouped ? grp.wb : d.C;       // input channels one output channel reads, per tap
+    const int bk = (cw % 128 == 0) ? 128 : ((cw % 64 == 0) ? 64 : 32);
+    int bn = grouped ? grp.block : pick_bn(M, d.K);
     if (add && bn < 64) bn = 64;                 // the fused-add pass works on 64-column slabs
     CUtensorMap ta, tb;
     if ((rc = encode_im2col(&ta, x_nhwc, d, bk)) != PQ_OK) return rc;
-    const uint64_t ktot = (uint64_t)d.R * d.S * d.C;
+    const uint64_t ktot = (uint64_t)d.R * d.S * cw;
     pq::GemmParams p = {};
     p.M = (int)M; p.N = d.K; p.a_im2col = 1;
-    p.R = d.R; p.S = d.S; p.C = d.C; p.cblocks = d.C / bk; p.num_kb = d.R * d.S * p.cblocks;
+    p.R = d.R; p.S = d.S; p.C = d.C; p.cblocks = cw / bk; p.num_kb = d.R * d.S * p.cblocks;
+    p.g_wb = grp.wb; p.g_tpg = grp.tpg;
     // short K blocks (<= 64 bytes of K: ~70 cycles of tensor work per block at BN = 64) are bound by the producers'
     // per-stage mbarrier round trip, not by TMA or the tensor pipe: move three K blocks per stage
     p.tps = (bk <= 64 && p.num_kb % 3 == 0) ? 3 : 1;

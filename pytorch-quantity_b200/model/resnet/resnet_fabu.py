@@ -18,8 +18,8 @@ import torch.nn as nn
 from common.quantity import Eltwise, View
 
 
-def _conv_bn(cin, cout, k, stride, pad):
-    return [nn.Conv2d(cin, cout, kernel_size=k, stride=stride, padding=pad, bias=False),
+def _conv_bn(cin, cout, k, stride, pad, groups=1):
+    return [nn.Conv2d(cin, cout, kernel_size=k, stride=stride, padding=pad, groups=groups, bias=False),
             nn.BatchNorm2d(cout)]
 
 
@@ -45,16 +45,18 @@ class BasicUnit(nn.Module):
 
 class BottleneckUnit(BasicUnit):
     """1x1 -> 3x3(stride) -> 1x1 residual unit (ResNet-50/101), stride on the 3x3 like
-    quantity/model/resnet/ResNet.py:31-61."""
+    quantity/model/resnet/ResNet.py:31-61.  With groups > 1 it is the ResNeXt unit: the 3x3 is a grouped convolution
+    of width * base_width / 64 * groups channels (torchvision's ResNeXt definition)."""
     expansion = 4
 
-    def __init__(self, cin, width, stride):
+    def __init__(self, cin, width, stride, groups=1, base_width=64):
         nn.Module.__init__(self)
         cout = width * self.expansion
+        mid = width * base_width // 64 * groups
         self.left = nn.Sequential(
-            *_conv_bn(cin, width, 1, 1, 0), nn.ReLU(False),
-            *_conv_bn(width, width, 3, stride, 1), nn.ReLU(False),
-            *_conv_bn(width, cout, 1, 1, 0))
+            *_conv_bn(cin, mid, 1, 1, 0), nn.ReLU(False),
+            *_conv_bn(mid, mid, 3, stride, 1, groups), nn.ReLU(False),
+            *_conv_bn(mid, cout, 1, 1, 0))
         self.shortcut = nn.Sequential()
         if stride != 1 or cin != cout:
             self.shortcut = nn.Sequential(*_conv_bn(cin, cout, 1, stride, 0))
@@ -63,7 +65,7 @@ class BottleneckUnit(BasicUnit):
 
 
 class FabuResNet(nn.Module):
-    def __init__(self, unit, depths, num_classes=1000, in_hw=224):
+    def __init__(self, unit, depths, num_classes=1000, in_hw=224, **unit_kw):
         super().__init__()
         self.stem = nn.Sequential(*_conv_bn(3, 64, 7, 2, 3), nn.ReLU(False))
         self.maxpool = nn.MaxPool2d(kernel_size=3, stride=2, padding=1)
@@ -71,7 +73,7 @@ class FabuResNet(nn.Module):
         for i, (width, n) in enumerate(zip((64, 128, 256, 512), depths)):
             units = []
             for j in range(n):
-                units.append(unit(cin, width, (1 if i == 0 else 2) if j == 0 else 1))
+                units.append(unit(cin, width, (1 if i == 0 else 2) if j == 0 else 1, **unit_kw))
                 cin = width * unit.expansion
             stages.append(nn.Sequential(*units))
         self.layer1, self.layer2, self.layer3, self.layer4 = stages
@@ -91,6 +93,10 @@ def resnet18_fabu(num_classes=1000, in_hw=224):
 
 def resnet50_fabu(num_classes=1000, in_hw=224):
     return FabuResNet(BottleneckUnit, (3, 4, 6, 3), num_classes, in_hw)
+
+
+def resnext50_32x4d_fabu(num_classes=1000, in_hw=224):
+    return FabuResNet(BottleneckUnit, (3, 4, 6, 3), num_classes, in_hw, groups=32, base_width=4)
 
 
 def randomize_bn_(model, seed=0):
