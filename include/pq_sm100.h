@@ -149,7 +149,8 @@ int pq_quantize_nchw_to_nhwc_s8(const float *x, int8_t *q, int N, int C, int H, 
 /* ---- a12 for convolutions with very few input channels (the ResNet stem): Quantity.forward fused
  * with an explicit im2col, a[m][k] = q(x[n][c][p*sh-ph+r][q*sw-pw+s]) for k = (r*S+s)*C + c, zero for
  * padding and for k in [R*S*C, kp); m = (n*P + p)*Q + q, row pitch kp bytes (multiple of 16).  The
- * result feeds pq_gemm_s8 with weights laid out [K][R][S][C] and zero-padded to kp. */
+ * result feeds pq_gemm_s8 with weights laid out [K][R][S][C] and zero-padded to kp.  A filter larger than the
+ * padded input (H + 2*pad_h < R or W + 2*pad_w < S) is PQ_EINVAL. */
 int pq_quantize_im2col_s8(const float *x, int8_t *a, int N, int C, int H, int W, int R, int S,
                           int stride_h, int stride_w, int pad_h, int pad_w, int kp, int ib,
                           pq_stream_t stream);
@@ -268,7 +269,9 @@ int pq_avgpool_global_nhwc_f32(const void *x, int is16, int bit, int relu, int N
 int pq_relu_s8(const int8_t *x, int8_t *y, size_t n, pq_stream_t stream);
 
 /* nn.MaxPool2d on int8 NHWC (max commutes with the monotone quantiser); relu != 0 also applies max(.,0).
- * Padding behaves like -inf, as in torch. */
+ * Padding behaves like -inf, as in torch.  Output P = (H + 2*pad - k) / stride + 1, Q alike; x and y 16-byte aligned.
+ * A window larger than the padded input (H + 2*pad < k or W + 2*pad < k) is PQ_EINVAL.  PQ_EUNSUPPORTED:
+ * C % 16 != 0, 2*pad > k (torch refuses that too), N > 65535, and one image of H*W*C >= 2^31 bytes. */
 int pq_maxpool_nhwc_s8(const int8_t *x, int8_t *y, int N, int H, int W, int C, int k, int stride, int pad,
                        int relu, pq_stream_t stream);
 

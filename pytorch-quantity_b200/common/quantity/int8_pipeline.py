@@ -305,6 +305,8 @@ def _maxpool(x, kernel_size, stride=None, padding=0, dilation=1, ceil_mode=False
     k, s, p = _pair(kernel_size), _pair(stride if stride is not None else kernel_size), _pair(padding)
     if k[0] != k[1] or s[0] != s[1] or p[0] != p[1] or _pair(dilation) != (1, 1) or ceil_mode or return_indices:
         return None
+    if 2 * p[0] > k[0] or min(x.shape[2], x.shape[3]) + 2 * p[0] < k[0]:
+        return None                                     # arguments torch refuses: let F.max_pool2d raise its own error
     if not x.has_q8() or x.channels % 16:               # payload channels == logical channels
         return None
     q8 = x.q8

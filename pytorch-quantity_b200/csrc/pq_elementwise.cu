@@ -519,8 +519,8 @@ extern "C" int pq_quantize_im2col_s8(const float *x, int8_t *a, int N, int C, in
     if (!x || !a || pad_h < 0 || pad_w < 0) return PQ_EINVAL;
     if (kp < R * S * C || (kp & 15) || ib < -126 || ib > 126) return PQ_EUNSUPPORTED;
     if (!aligned16(a)) return PQ_EALIGN;
+    if (H + 2 * pad_h < R || W + 2 * pad_w < S) return PQ_EINVAL;    // filter larger than the padded input
     const int P = (H + 2 * pad_h - R) / stride_h + 1, Q = (W + 2 * pad_w - S) / stride_w + 1;
-    if (P <= 0 || Q <= 0) return PQ_EINVAL;
     const long long M = (long long)N * P * Q;
     const size_t smem = (size_t)(pq::kIm2colWarps * 32 * ((kp >> 2) | 1)) * sizeof(unsigned int);
     if (smem > 200 * 1024) return PQ_EUNSUPPORTED;

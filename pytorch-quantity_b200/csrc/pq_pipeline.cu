@@ -442,11 +442,13 @@ extern "C" int pq_relu_s8(const int8_t *x, int8_t *y, size_t n, pq_stream_t stre
 extern "C" int pq_maxpool_nhwc_s8(const int8_t *x, int8_t *y, int N, int H, int W, int C, int k, int stride, int pad,
                                   int relu, pq_stream_t stream)
 {
-    if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || k <= 0 || stride <= 0 || pad < 0 || !x || !y) return PQ_EINVAL;
-    if ((C & 15) || pad >= k) return PQ_EUNSUPPORTED;
+    if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || k <= 0 || stride <= 0 || pad < 0) return PQ_EINVAL;
+    if ((long long)H * W * C >= (1LL << 31)) return PQ_EUNSUPPORTED;   // the k = 3 path addresses one image in int
+    if (!x || !y) return PQ_EINVAL;
+    if ((C & 15) || 2 * pad > k) return PQ_EUNSUPPORTED;              // torch: pad at most half the window
     if (!al16(x) || !al16(y)) return PQ_EALIGN;
+    if (H + 2 * pad < k || W + 2 * pad < k) return PQ_EINVAL;        // window larger than the padded input
     const int P = (H + 2 * pad - k) / stride + 1, Q = (W + 2 * pad - k) / stride + 1;
-    if (P <= 0 || Q <= 0) return PQ_EINVAL;
     if (N > 65535) return PQ_EUNSUPPORTED;
     pq::maxpool_nhwc_s8_kernel<<<dim3((unsigned)P, (unsigned)N), pq::kPipeThreads, 0, (cudaStream_t)stream>>>(
         x, y, N, H, W, C, k, stride, pad, P, Q, relu);
