@@ -56,7 +56,8 @@ const char *pq_error_string(int code);
 /* ---- a1: DistributionCollector.refresh_max_val, common/quantity/distribution_collector.py:70-78
  * max_bits[i] = max(max_bits[i], bits(|x|)) over tensor i, as the uint32 pattern of the
  * fp32 magnitude (monotone for non-NaN floats; reinterpret as float to read it).
- * xs_host / ns_host are HOST arrays of k device pointers / element counts. */
+ * xs_host / ns_host are HOST arrays of k device pointers / element counts (k <= PQ_MAX_SEGMENTS, else PQ_ETOOMANY;
+ * a table of more than 2^32 - 1 chunks of 8192 elements is PQ_EUNSUPPORTED; the histogram entry points share both limits). */
 int pq_absmax_multi_f32(const float *const *xs_host, const uint64_t *ns_host, int k,
                         uint32_t *max_bits, pq_stream_t stream);
 
@@ -87,7 +88,9 @@ int pq_eltwise_add_f32(const float *a, const float *b, float *z, size_t n, float
 
 /* ---- a3: DistributionCollector._add_to_distribution, distribution_collector.py:127-135
  * for every x != 0:  hist[i][min((int)trunc(fl32(|x| / interval_i)), 2047)] += 1
- * with a correctly rounded fp32 division.  hist is int64 [k][2048] (the reference's int32
+ * with a correctly rounded fp32 division, for any interval_i > 0 (subnormal ones included; 0, negative or NaN
+ * intervals are PQ_EINVAL).  A NaN x, or a NaN quotient (inf / inf), is counted in the top bin 2047
+ * wherever it sits in the tensor (the reference leaves NaN undefined).  hist is int64 [k][2048] (the reference's int32
  * would overflow at BASELINE.json's 8192-image config; the Python layer narrows to int32
  * when it fits).  intervals_host: HOST array of k fp32 bin widths (a2, :60-61). */
 int pq_hist2048_multi_f32(const float *const *xs_host, const uint64_t *ns_host,
@@ -109,10 +112,12 @@ int pq_kl_search_f64(const double *counts, int k, double *workspace, double *kl,
 /* ---- a3 / a5 / a6 for any INTERVAL_NUM (tools/configs.yml:23; DistributionCollector(interval_num=...),
  * common/quantity/distribution_collector.py:9-22, and `length = distribution.size` in
  * common/quantity/quantizer.py:98-103).  nbins == 2048 forwards to the specialised entry points above.
- * pq_hist_multi_f32: hist is int64 [k][nbins], 1 <= nbins <= PQ_HIST_BINS_MAX (else PQ_EUNSUPPORTED).
+ * pq_hist_multi_f32: hist is int64 [k][nbins], 1 <= nbins <= PQ_HIST_BINS_MAX (else PQ_EUNSUPPORTED); the top bin
+ * nbins - 1 takes every quotient >= nbins - 1 and every NaN, as above.
  * pq_kl_search_n_f64: counts fp64 [k][nbins], kl (optional) fp64 [k][nbins - 128], 128 < nbins <=
  * PQ_HIST_BINS_MAX (nbins <= 128: PQ_EINVAL -- the reference's candidate loop would be empty), default
- * threshold nbins - 1; workspace fp64 [k][pq_kl_workspace_doubles_n(nbins)]. */
+ * threshold nbins - 1; workspace fp64 [k][pq_kl_workspace_doubles_n(nbins)].  Both KL entry points take k <= 65535
+ * tensors per call (else PQ_EUNSUPPORTED); _native.kl_search splits larger batches. */
 int pq_hist_multi_f32(const float *const *xs_host, const uint64_t *ns_host, const float *intervals_host,
                       int k, int nbins, long long *hist, pq_stream_t stream);
 size_t pq_kl_workspace_doubles_n(int nbins);

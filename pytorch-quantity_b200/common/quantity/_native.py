@@ -19,6 +19,7 @@ HIST_BINS_MAX = 8192
 KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
+KL_MAX_ROWS = 65535          # tensors per pq_kl_search_n_f64 call (one grid row per tensor)
 PQ_VERSION = 203             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
@@ -264,20 +265,23 @@ def hist_multi(tensors, intervals, hist):
 
 
 def kl_search(counts_f64, want_curves=False):
-    """counts_f64: CUDA fp64 [k][nbins].  Returns (threshold int32 [k], kl fp64 [k][nbins - 128] or None)."""
+    """counts_f64: CUDA fp64 [k][nbins].  Returns (threshold int32 [k], kl fp64 [k][nbins - 128] or None).
+    More than KL_MAX_ROWS tensors are searched in blocks of KL_MAX_ROWS, one launch sequence each."""
     require_cuda(counts_f64, "kl_search")
     assert counts_f64.dtype == torch.float64 and counts_f64.dim() == 2
     nbins = int(counts_f64.shape[1])
     counts_f64 = counts_f64.contiguous()
     k = counts_f64.shape[0]
     dev = counts_f64.device
-    ws = torch.empty(k * lib().pq_kl_workspace_doubles_n(nbins), dtype=torch.float64, device=dev)
+    ws = torch.empty(min(k, KL_MAX_ROWS) * lib().pq_kl_workspace_doubles_n(nbins), dtype=torch.float64, device=dev)
     thr = torch.empty(k, dtype=torch.int32, device=dev)
     kl = torch.empty((k, max(nbins - KL_TARGET_BIN, 0)), dtype=torch.float64, device=dev) if want_curves else None
-    with _Timed("kl", 3, 8 * counts_f64.numel(), dev):
-        check(lib().pq_kl_search_n_f64(counts_f64.data_ptr(), k, nbins, ws.data_ptr(),
-                                       kl.data_ptr() if want_curves else None, thr.data_ptr(),
-                                       _stream(counts_f64)), "pq_kl_search_n_f64 (INTERVAL_NUM=%d)" % nbins)
+    for lo in range(0, k, KL_MAX_ROWS):
+        rows = min(k - lo, KL_MAX_ROWS)
+        with _Timed("kl", 3, 8 * rows * nbins, dev):
+            check(lib().pq_kl_search_n_f64(counts_f64[lo:].data_ptr(), rows, nbins, ws.data_ptr(),
+                                           kl[lo:].data_ptr() if want_curves else None, thr[lo:].data_ptr(),
+                                           _stream(counts_f64)), "pq_kl_search_n_f64 (INTERVAL_NUM=%d)" % nbins)
     return thr, kl
 
 

@@ -187,7 +187,7 @@ int main(int argc, char **argv)
         cudaMemset(mx, 0, 64);
         // production absmax through the ABI-level table
         SegTable t; t.k = 1; t.ptr[0] = x; t.n[0] = n; t.param[0] = 0.f;
-        t.chunk_end[0] = seg_num_chunks(x, n); t.total_chunks = t.chunk_end[0];
+        t.chunk_end[0] = (unsigned int)seg_num_chunks(x, n); t.total_chunks = t.chunk_end[0];
         float ms = time_ms([&] { absmax_multi_kernel<<<148 * 8, kStatThreads>>>(t, mx); });
         unsigned int bits; cudaMemcpy(&bits, mx, 4, cudaMemcpyDeviceToHost);
         float maxv; memcpy(&maxv, &bits, 4);

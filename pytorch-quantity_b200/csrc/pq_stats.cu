@@ -158,6 +158,25 @@ extern "C" int pq_eltwise_add_f32(const float *a, const float *b, float *z, size
     return launch_epilogue(p, pq::EPI_ADD, (cudaStream_t)stream);
 }
 
+namespace {
+// the reference-literal kernel (one IEEE division per element) for any bin count
+int launch_hist_generic(const pq::SegTable &t, int nbins, long long *hist, cudaStream_t stream)
+{
+    const size_t smem = (size_t)nbins * 4;
+    static bool attr_set = false;
+    if (!attr_set) {
+        PQ_CUDA_TRY(cudaFuncSetAttribute(pq::hist_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         PQ_HIST_BINS_MAX * 4));
+        attr_set = true;
+    }
+    int ctas_per_sm = (int)((200 * 1024) / (smem + 1024));
+    ctas_per_sm = ctas_per_sm < 1 ? 1 : (ctas_per_sm > 8 ? 8 : ctas_per_sm);
+    pq::hist_generic_kernel<<<grid_for(t.total_chunks, ctas_per_sm), pq::kStatThreads, smem, stream>>>(
+        t, nbins, reinterpret_cast<unsigned long long *>(hist));
+    return (int)cudaGetLastError();
+}
+}  // namespace
+
 extern "C" int pq_hist2048_multi_f32(const float *const *xs_host, const uint64_t *ns_host,
                                      const float *intervals_host, int k, long long *hist,
                                      pq_stream_t stream)
@@ -169,6 +188,9 @@ extern "C" int pq_hist2048_multi_f32(const float *const *xs_host, const uint64_t
     pq::SegTable t;
     int rc = build_table(t, xs_host, ns_host, intervals_host, k);
     if (rc != PQ_OK) return rc;
+    // the fast path multiplies by RN(1/interval), which overflows for subnormal intervals (pq_stats_kernels.cuh)
+    for (int i = 0; i < k; ++i)
+        if (intervals_host[i] < 0x1p-126f) return launch_hist_generic(t, PQ_HIST_BINS, hist, (cudaStream_t)stream);
     constexpr size_t smem = pq::hist_smem_bytes(kHistCopies);
     auto kern = pq::hist_multi_kernel<kHistCopies>;
     static bool attr_set = false;
@@ -195,16 +217,5 @@ extern "C" int pq_hist_multi_f32(const float *const *xs_host, const uint64_t *ns
     pq::SegTable t;
     int rc = build_table(t, xs_host, ns_host, intervals_host, k);
     if (rc != PQ_OK) return rc;
-    const size_t smem = (size_t)nbins * 4;
-    static bool attr_set = false;
-    if (!attr_set) {
-        PQ_CUDA_TRY(cudaFuncSetAttribute(pq::hist_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         PQ_HIST_BINS_MAX * 4));
-        attr_set = true;
-    }
-    int ctas_per_sm = (int)((200 * 1024) / (smem + 1024));
-    ctas_per_sm = ctas_per_sm < 1 ? 1 : (ctas_per_sm > 8 ? 8 : ctas_per_sm);
-    pq::hist_generic_kernel<<<grid_for(t.total_chunks, ctas_per_sm), pq::kStatThreads, smem, (cudaStream_t)stream>>>(
-        t, nbins, reinterpret_cast<unsigned long long *>(hist));
-    return (int)cudaGetLastError();
+    return launch_hist_generic(t, nbins, hist, (cudaStream_t)stream);
 }

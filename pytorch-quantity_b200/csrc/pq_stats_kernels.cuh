@@ -40,14 +40,15 @@ __device__ __forceinline__ SegGeom seg_geom(const SegTable &t, int s)
     return g;
 }
 
-__host__ __device__ inline unsigned int seg_num_chunks(const float *p, unsigned long long n)
+// 64-bit: the host sums these and refuses a table of more than 2^32 - 1 chunks, however large one segment is
+__host__ __device__ inline unsigned long long seg_num_chunks(const float *p, unsigned long long n)
 {
     unsigned long long addr = (unsigned long long)p;
     unsigned long long head = ((16ull - (addr & 15ull)) & 15ull) >> 2;
     if (head > n) head = n;
     unsigned long long nvec = (n - head) >> 2;
     unsigned long long c = (nvec + kChunkVecs - 1) / kChunkVecs;
-    return (unsigned int)(c ? c : 1);
+    return c ? c : 1;
 }
 
 // ------------------------------------------------------------------------------ absmax
@@ -393,11 +394,15 @@ epilogue_kernel(const EpiArgs p)
 //   u = RZ(min(q0, 2047.5) + 2048) holds trunc(q0) in mantissa bits [12,23) and the first 12
 //   fraction bits f below them.  If 4 <= f < 4092, q0 is >= 2^-10 = 9.8e-4 away from every
 //   integer, hence trunc(Q) == trunc(q0).
+//   This needs a finite r: for a subnormal d < 1/FLT_MAX, r = +inf files every non-zero element in the top bin and
+//   an exact zero too (0 * inf = NaN), so pq_hist2048_multi_f32 sends a call with any subnormal interval
+//   (d < 2^-126) to hist_generic_kernel, which divides literally.
 // Otherwise (0.2 % of elements, plus every exact zero) the element is "ambiguous": the hot loop
 // still counts it in bin trunc(q0) (no select, no branch), flags its float4, and the rare redo pass
 // takes that count back and files the element with the real IEEE division.  Values at or beyond
 // the top bin clamp to 2047.5 and are counted there directly (their true quotient is > 2047).
-// NaN inputs are undefined in the reference; here they land in the top bin.
+// NaN inputs are undefined in the reference; here they land in the top bin on every path (the fast path through
+// fminf, the exact paths through !(q < top)), so where a NaN sits in the tensor does not change its bin.
 struct HistDiv {
     float d;        // bin width
     float r;        // RN(1/d)
@@ -416,7 +421,7 @@ __device__ __forceinline__ void hist_add_exact(unsigned int *sh, float v, float 
 {
     if (v != 0.0f) {                                       // bins are (lo, hi]: zeros are skipped
         const float q = __fdiv_rn(fabsf(v), interval);     // IEEE division, as numpy float32 / float32
-        const int idx = q >= 2047.0f ? 2047 : (int)q;      // trunc + clamp (np.minimum(..., 2047))
+        const int idx = !(q < 2047.0f) ? 2047 : (int)q;    // trunc + clamp (np.minimum(..., 2047)); NaN: top bin
         atomicAdd(sh + idx, 1u);
     }
 }
@@ -629,7 +634,7 @@ __device__ __forceinline__ void hist_add_exact_n(unsigned int *sh, float v, floa
 {
     if (v != 0.0f) {
         const float q = __fdiv_rn(fabsf(v), interval);
-        const int idx = q >= (float)(nbins - 1) ? nbins - 1 : (int)q;     // np.minimum(int32(q), nbins - 1)
+        const int idx = !(q < (float)(nbins - 1)) ? nbins - 1 : (int)q;  // np.minimum(int32(q), nbins - 1); NaN: top
         atomicAdd(sh + idx, 1u);
     }
 }

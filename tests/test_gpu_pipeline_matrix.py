@@ -778,15 +778,15 @@ OTHER_KERNELS = {
     "gemm_s8_kernel": "test_gpu_epilogue_matrix.py",
     "conv_rows_s8_kernel": "test_gpu_epilogue_matrix.py",
     "dw_conv_s8_kernel": "test_gpu_depthwise.py",
-    "absmax_multi_kernel": "test_gpu_parity.py",
-    "absmax_per_channel_kernel": "test_gpu_parity.py",
-    "absmax_periodic_kernel": "test_gpu_parity.py",
-    "hist_multi_kernel": "test_gpu_parity.py",
-    "hist_generic_kernel": "test_gpu_parity.py",
-    "epilogue_kernel": "test_gpu_calib_fusion.py",
-    "kl_prepare_kernel": "test_gpu_parity.py",
-    "kl_candidate_kernel": "test_gpu_parity.py",
-    "kl_argmin_kernel": "test_gpu_parity.py",
+    "absmax_multi_kernel": "test_gpu_stats_matrix.py",
+    "absmax_per_channel_kernel": "test_gpu_stats_matrix.py",
+    "absmax_periodic_kernel": "test_gpu_stats_matrix.py",
+    "hist_multi_kernel": "test_gpu_stats_matrix.py",
+    "hist_generic_kernel": "test_gpu_stats_matrix.py",
+    "epilogue_kernel": "test_gpu_stats_matrix.py",
+    "kl_prepare_kernel": "test_gpu_stats_matrix.py",
+    "kl_candidate_kernel": "test_gpu_stats_matrix.py",
+    "kl_argmin_kernel": "test_gpu_stats_matrix.py",
 }
 ROW_KERNELS = ({r[-1] for r in NHWC_ROWS} | {"quantize_im2col_kernel"} | {r[-1] for r in PAD8_ROWS} |
                {r[-1] for r in S2D_ROWS} | {"concat_requant_%s_kernel" % r[-1] for r in CONCAT_ROWS})
