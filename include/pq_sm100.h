@@ -165,10 +165,15 @@ int pq_quantize_im2col_s8(const float *x, int8_t *a, int N, int C, int H, int W,
  *   q[n][h + pad_h][w + pad_w][c] = (int8) clamp(rint(x[n][c][h][w] * 2^ib)),  0 elsewhere   ([N][Hp][Wp][8])
  * so that the S taps of one filter row are 8*S contiguous bytes; pq_conv2d_smallc_s8 fetches them for a
  * patch of output pixels with one overlapping-stride tiled TMA per filter row (no im2col matrix in HBM).
- * desc.C must be 8; weights are [K][R][64] int8 = 8 tap slots x 8 channel slots per filter row, zero
- * where s >= S or c >= C.  Requires S <= 8, even stride_w, Hp % stride_h == 0,
- * Hp >= max((P-1)*stride_h + R, H + pad_h), Wp even, Wp >= max((Q-1)*stride_w + 8, W + pad_w).
- * desc.dil_h / dil_w must be 1 (else PQ_EUNSUPPORTED).  Epilogue, flags and outputs as pq_conv2d_s8. */
+ * Weights are [K][R][64] int8 = 8 tap slots x 8 channel slots per filter row, zero where s >= S or c >= C.
+ * The image is read as already padded (desc.pad_h / pad_w only size it).  Outside these limits the call returns
+ * PQ_EUNSUPPORTED and writes nothing (patches: N * ceil(P / TH) * ceil(Q / TW), TW = 4, 8 or 16 for Q < 8, < 16, else,
+ * TH = 128 / TW):
+ *   smallc limit: C == 8;  smallc limit: S <= 8;  smallc limit: even stride_w;  smallc limit: R <= 64;
+ *   smallc limit: Hp % stride_h == 0;  smallc limit: Hp >= (P-1)*stride_h + R;  smallc limit: Hp >= H + pad_h;
+ *   smallc limit: Wp even;  smallc limit: Wp >= (Q-1)*stride_w + 8;  smallc limit: Wp >= W + pad_w;
+ *   smallc limit: dilation 1;  smallc limit: patches*128 <= 2^31 - 1;
+ * Epilogue, flags and outputs as pq_conv2d_s8. */
 int pq_quantize_nchw_to_padded_nhwc8_s8(const float *x, int8_t *q, int N, int C, int H, int W, int pad_h,
                                         int pad_w, int Hp, int Wp, int ib, pq_stream_t stream);
 
@@ -187,6 +192,20 @@ int pq_quantize_nchw_to_padded_nhwc8_s8(const float *x, int8_t *q, int N, int C,
  * NewConv2d; the reference's weight path zero-stuffs such kernels for its target hardware,
  * tools/pytorch_quantizer.py:626-629,679-693) take the im2col-TMA path with the dilation as tap offsets, so no
  * multiply is wasted on stuffed zeros; a 1x1 filter ignores the dilation.
+ *
+ * Geometry limits of pq_conv2d_s8 and pq_conv2d_s8_add, per dimension (h with R, w with S), checked before any launch;
+ * a call outside them returns PQ_EUNSUPPORTED unless noted and writes nothing.  The im2col-TMA tensor map carries the
+ * padding as the corners of its bounding box, lower = -pad and upper = pad - (R-1)*dil, and cuda.h allows the corners
+ * of a rank-4 map only in [-128, 127]; those corner limits, not the footprint limit, bind for most dilated filters
+ * (3x3 with dil 65 and pad 0 is refused, 3x3 with dil 127 and pad 126 on a 3x3 image runs):
+ *   conv limit: stride <= 8;
+ *   conv limit: pad <= 128;
+ *   conv limit: pad - (R-1)*dil <= 127;
+ *   conv limit: (R-1)*dil - pad <= 128;
+ *   conv limit: (R-1)*dil + 1 <= 255;
+ *   conv limit: C % 16 == 0;  (else PQ_EALIGN)
+ *   conv limit: C % 32 == 0 off the plain path;  (the plain path: 1x1, stride 1, no padding)
+ *   conv limit: N*P*Q <= 2^31 - 1;
  *
  * Grouped convolutions (desc.groups = G > 1; nn.Conv2d(groups=G) wrapped by NewConv2d), Cg = C / G input and
  * Kg = K / G output channels per group, run in the same single launch: output-channel tile t of B = group_block
