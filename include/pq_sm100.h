@@ -262,7 +262,12 @@ int pq_conv2d_s8(const int8_t *x_nhwc, const int8_t *w_krsc, const int32_t *bias
  * Flags PQ_FLAG_RELU / PQ_FLAG_BIAS_FOLDED as for pq_conv2d_s8.  Outputs (either may be NULL, not both): fp32 NCHW
  * [N][K][P][Q], int8 NHWC [N][P][Q][K].  Supports 1 <= R, S <= 7, stride 1 or 2 and dilation 1 or 2 in each
  * dimension, 0 <= pad <= (R - 1) * dil; anything else is PQ_EUNSUPPORTED (and nothing is written).  x, w_rsc and
- * out_s8_nhwc 16-byte aligned. */
+ * out_s8_nhwc 16-byte aligned, bias_q and out_f32_nchw 4-byte aligned (else PQ_EALIGN).  One CTA covers 16 * G
+ * channels, G = 4, 2 or 1 for C % 64 == 0, C % 32 == 0 or neither, and the launch grid has at most 65535 of them, so
+ * C <= 16 * 65535 (G = 1), 32 * 65535 (G = 2) or 64 * 65535 (G = 4).  The limits, per dimension (h with R, w with S),
+ * checked before any launch:
+ *   dw limit: R, S <= 7;  dw limit: stride <= 2;  dw limit: dilation <= 2;  dw limit: pad <= (R-1)*dil;
+ *   dw limit: C % 16 == 0;  dw limit: C / (16*G) <= 65535;  dw limit: N*P*Q <= 2^31 - 1; */
 int pq_conv2d_dw_s8(const int8_t *x_nhwc, const int8_t *w_rsc, const int32_t *bias_q, const pq_conv_desc *desc_host,
                     int flags, float *out_f32_nchw, int8_t *out_s8_nhwc, pq_stream_t stream);
 

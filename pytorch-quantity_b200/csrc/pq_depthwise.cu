@@ -156,6 +156,8 @@ extern "C" int pq_conv2d_dw_s8(const int8_t *x_nhwc, const int8_t *w_rsc, const 
     if (d.ob < -100 || d.ob > 100 || d.rs > 24 || d.rs < -24) return PQ_EUNSUPPORTED;
     const long long M = (long long)d.N * d.P * d.Q;
     if (M > 0x7fffffffLL) return PQ_EUNSUPPORTED;
+    const int G = d.C % 64 == 0 ? 4 : (d.C % 32 == 0 ? 2 : 1);
+    if (d.C / (16 * G) > 65535) return PQ_EUNSUPPORTED;             // grid.y below: one CTA per 16 * G channels
     if ((((uintptr_t)x_nhwc | (uintptr_t)w_rsc | (uintptr_t)out_s8_nhwc) & 15) || (((uintptr_t)bias_q | (uintptr_t)out_f32_nchw) & 3))
         return PQ_EALIGN;
 
@@ -168,7 +170,6 @@ extern "C" int pq_conv2d_dw_s8(const int8_t *x_nhwc, const int8_t *w_rsc, const 
     p.dil_h = d.dil_h; p.dil_w = d.dil_w; p.P = d.P; p.Q = d.Q; p.rs = d.rs; p.ob = d.ob;
     p.relu = flags & PQ_FLAG_RELU;
     p.M = (int)M;
-    const int G = d.C % 64 == 0 ? 4 : (d.C % 32 == 0 ? 2 : 1);
     const int KS = (d.R == d.S && (d.R == 3 || d.R == 5)) ? d.R : 0;
     const long long pix_per_cta = (long long)pq::kDwThreads / G * pq::kDwPixIters;
     const dim3 grid((unsigned)((M + pix_per_cta - 1) / pix_per_cta), (unsigned)(d.C / (16 * G)));
