@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 203
+#define PQ_VERSION 204
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -49,6 +49,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 #define PQ_KL_TARGET_BIN 128 /* common/quantity/quantizer.py:98 target_bin */
 #define PQ_KL_CANDIDATES (PQ_HIST_BINS - PQ_KL_TARGET_BIN)
 #define PQ_MAX_SEGMENTS 256 /* tensors per multi-tensor launch */
+#define PQ_MAXPOOL_PLANE_BYTES (227 * 1024 - 1024) /* largest [H][W] plane of pq_conv_epilogue_maxpool_f32 */
 
 int pq_version(void); /* PQ_VERSION */
 const char *pq_error_string(int code);
@@ -85,6 +86,22 @@ int pq_conv_epilogue_f32(float *y, const float *bias, int N, int C, uint64_t hw,
                          uint32_t *max_slot, pq_stream_t stream);
 int pq_eltwise_add_f32(const float *a, const float *b, float *z, size_t n, float *relu_out, uint32_t *max_slot,
                        pq_stream_t stream);
+/* pq_conv_epilogue_add_f32: pq_conv_epilogue_f32 and the Eltwise that reads its output, in one pass, for the convolution
+ *   that completes the Eltwise's operands (the other operand, `other` [N][C][hw], already exists):
+ *   y += bias[c];  z = other + y when other_first, else y + other (the Eltwise's operand order);
+ *   relu_out = relu(z) when relu_out != NULL;  *max_slot takes max |y| and *max_z max |z| (each may be NULL).
+ *   other, z and relu_out 16-byte aligned, distinct from y and from each other; limits as pq_conv_epilogue_f32.
+ * pq_conv_epilogue_maxpool_f32: pq_conv_epilogue_f32 with relu_out (required) and the nn.MaxPool2d that reads it:
+ *   pool_out [N][C][OH][OW] = max_pool2d(relu_out, k, stride s, padding pad), OH = (H + 2 pad - k) / s + 1, as
+ *   ATen's max_pool2d bit for bit (NaN and signed-zero ties included).  Dilation 1, no ceil_mode, no indices.
+ *   k <= 3, s <= k, 2 pad <= k, H + 2 pad >= k, W + 2 pad >= k and H * W * 4 <= PQ_MAXPOOL_PLANE_BYTES (one plane
+ *   in shared memory), else PQ_EUNSUPPORTED.
+ *   y and relu_out 16-byte aligned, pool_out 4-byte aligned. */
+int pq_conv_epilogue_add_f32(float *y, const float *bias, int N, int C, uint64_t hw, const float *other,
+                             int other_first, float *z, float *relu_out, uint32_t *max_slot, uint32_t *max_z,
+                             pq_stream_t stream);
+int pq_conv_epilogue_maxpool_f32(float *y, const float *bias, int N, int C, int H, int W, float *relu_out,
+                                 float *pool_out, int k, int s, int pad, uint32_t *max_slot, pq_stream_t stream);
 
 /* ---- a3: DistributionCollector._add_to_distribution, distribution_collector.py:127-135
  * for every x != 0:  hist[i][min((int)trunc(fl32(|x| / interval_i)), 2047)] += 1

@@ -6,7 +6,8 @@ calibration-forward kernels against a copy peak measured in the same process.
 Workload: bench.py's (ResNet-50, BN folded, micro-batch 64, inputs resident in HBM), K batches through
 Quantity.activation_quantize after a warm-up job; pass 2 is served from the HBM activation cache.  The list gives
 every kernel's count, total time and share; then, per plane size, the algorithmic GB/s of pq::epilogue_kernel
-(conv epilogue: 8 bytes per element, 12 with the ReLU output; Eltwise: 12 / 16) and of absmax_multi_kernel, over the
+(conv epilogue: 8 bytes per element, 12 with the ReLU output; Eltwise: 12 / 16; conv epilogue with the Eltwise: 16 / 20;
+stem epilogue with the max-pool: 12 + 4 per pooled element) and of absmax_multi_kernel, over the
 copy peak: a CUDA-event-timed clone of a 4 GiB tensor (8 bytes per element moved).  A conv output is read back
 right after cuDNN wrote it, so part of it still comes from L2: the conv epilogue can exceed the copy peak.
 Profiler-traced, so the host side is slower than in bench.py: compare kernel times and shares, not the step time."""
@@ -65,8 +66,10 @@ def main():
     batches = [bench.make_batch(i, device="cuda") for i in range(args.steps)]
     cfg, user = bench.tool_configs(workdir, args.steps)
     q = tools.Quantity(net, config=cfg, user_config=user, verbose=False)     # the (unfused) tracing forward
-    rec, shapes = {}, {"conv_epilogue": [], "eltwise": []}
-    for kind, fname in (("conv_epilogue", "conv_epilogue"), ("eltwise", "eltwise_add")):
+    rec = {}
+    shapes = {"conv_epilogue": [], "eltwise": [], "conv_epilogue_add": [], "conv_epilogue_maxpool": []}
+    for kind, fname in (("conv_epilogue", "conv_epilogue"), ("eltwise", "eltwise_add"),
+                        ("conv_epilogue_add", "conv_epilogue_add"), ("conv_epilogue_maxpool", "conv_epilogue_maxpool")):
         def wrap(fn, kind=kind):                   # the tensor shape of every fused launch, in order
             def call(t, *a, **k):
                 shapes[kind].append(tuple(t.shape))
@@ -106,9 +109,13 @@ def main():
     lines.append("# copy peak, same process: clone of a 4 GiB fp32 tensor, %.1f GB/s" % peak)
     lines.append("%-44s %6s %10s %9s %8s" % ("pq kernel, tensor shape, bytes per launch", "count", "GB", "GB/s",
                                              "of copy"))
-    for kind, match in (("conv_epilogue", "epilogue_kernel<0>|epilogue_kernel<1>"), ("eltwise", "epilogue_kernel<2>"),
-                        ("absmax", "absmax_multi_kernel")):
-        ev = [e for e in kernels if any(m in e.name for m in match.split("|"))]
+    # the conv epilogue's overloads share its template ids and differ in their parameter lists
+    def plain(e):
+        return "AddendArgs" not in e.name and "PoolArgs" not in e.name
+    for kind, match, only in (("conv_epilogue", "epilogue_kernel<0>|epilogue_kernel<1>", plain),
+                              ("conv_epilogue_add", "AddendArgs", None), ("conv_epilogue_maxpool", "PoolArgs", None),
+                              ("eltwise", "epilogue_kernel<2>", None), ("absmax", "absmax_multi_kernel", None)):
+        ev = [e for e in kernels if any(m in e.name for m in match.split("|")) and (only is None or only(e))]
         recs = rec.get(kind, [])
         assert len(ev) == len(recs), (kind, len(ev), len(recs))
         groups = defaultdict(lambda: [0, 0, 0.0])

@@ -20,7 +20,8 @@ KL_TARGET_BIN = 128
 KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
 KL_MAX_ROWS = 65535          # tensors per pq_kl_search_n_f64 call (one grid row per tensor)
-PQ_VERSION = 203             # the header's PQ_VERSION: the entry points below match a library built from it
+MAXPOOL_PLANE_BYTES = 227 * 1024 - 1024   # PQ_MAXPOOL_PLANE_BYTES: largest plane pq_conv_epilogue_maxpool_f32 takes
+PQ_VERSION = 204             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -31,6 +32,8 @@ SYMBOLS = {
     "pq_absmax_per_channel_f32": (_i, [_vp, ctypes.c_uint64, _i, ctypes.c_uint64, _vp, _vp]),
     "pq_conv_epilogue_f32": (_i, [_vp, _vp, _i, _i, ctypes.c_uint64, _vp, _vp, _vp]),
     "pq_eltwise_add_f32": (_i, [_vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "pq_conv_epilogue_add_f32": (_i, [_vp, _vp, _i, _i, ctypes.c_uint64, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "pq_conv_epilogue_maxpool_f32": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "pq_hist2048_multi_f32": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "pq_kl_workspace_doubles": (_sz, []),
     "pq_kl_search_f64": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
@@ -88,6 +91,9 @@ _lib = None
 
 # ---- instrumentation used by bench.py: launch counts always; CUDA-event timing of each launch
 # on its launching stream when a profile dict is installed with set_profile().
+# LAUNCHES["total"] counts kernel launches; every other key counts the operations of its kind, so a launch that
+# performs two operations (conv_epilogue_add: a conv epilogue and an Eltwise) counts once under each of their keys
+# and once under "total".
 LAUNCHES = {"total": 0}
 _profile = None
 
@@ -100,12 +106,16 @@ def set_profile(store):
 
 
 class _Timed:
-    def __init__(self, name, kernels, alg_bytes, device):
+    """ops: the LAUNCHES keys the launch counts under besides "total" (default: its profile name)."""
+
+    def __init__(self, name, kernels, alg_bytes, device, ops=None):
         self.name, self.kernels, self.alg_bytes, self.device = name, kernels, alg_bytes, device
+        self.ops = ops if ops is not None else (name,)
 
     def __enter__(self):
         LAUNCHES["total"] += self.kernels
-        LAUNCHES[self.name] = LAUNCHES.get(self.name, 0) + self.kernels
+        for op in self.ops:
+            LAUNCHES[op] = LAUNCHES.get(op, 0) + self.kernels
         if _profile is not None:
             self.start = torch.cuda.Event(enable_timing=True)
             self.start.record(torch.cuda.current_stream(self.device))
@@ -229,6 +239,45 @@ def conv_epilogue(y, bias, relu=False, max_slot=None):
         check(lib().pq_conv_epilogue_f32(y.data_ptr(), bias.data_ptr(), N, C, H * W, r.data_ptr() if relu else None,
                                          max_slot, _stream(y)), "pq_conv_epilogue_f32")
     return r
+
+
+def conv_epilogue_add(y, bias, other, other_first, relu=False, max_slot=None, max_z=None):
+    """conv_epilogue and the Eltwise that reads y in one launch: y += bias[c] in place, z = other + y (other_first)
+    or y + other.  Returns (z, relu(z) or None); max_slot takes max |y|, max_z (a device address or None) max |z|."""
+    _require_f32_contiguous((y, bias, other), "conv_epilogue_add")
+    N, C, H, W = y.shape
+    if bias.numel() != C:
+        raise RuntimeError("conv_epilogue_add: %d bias values for %d channels" % (bias.numel(), C))
+    if other.shape != y.shape:
+        raise RuntimeError("conv_epilogue_add: shapes %s and %s differ" % (tuple(y.shape), tuple(other.shape)))
+    z = torch.empty_like(y)
+    r = torch.empty_like(y) if relu else None
+    with _Timed("conv_epilogue_add", 1, y.numel() * (20 if relu else 16), y.device, ("conv_epilogue", "eltwise")):
+        check(lib().pq_conv_epilogue_add_f32(y.data_ptr(), bias.data_ptr(), N, C, H * W, other.data_ptr(),
+                                             int(other_first), z.data_ptr(), r.data_ptr() if relu else None,
+                                             max_slot, max_z, _stream(y)), "pq_conv_epilogue_add_f32")
+    return z, r
+
+
+def conv_epilogue_maxpool(y, bias, kernel_size, stride, padding, max_slot=None):
+    """conv_epilogue with relu, and the max_pool2d(relu(y), kernel_size, stride, padding) that reads it, in one
+    launch (dilation 1, no ceil_mode).  Returns (relu(y), pooled), or None without touching y when the kernel does
+    not implement the geometry (see include/pq_sm100.h)."""
+    _require_f32_contiguous((y, bias), "conv_epilogue_maxpool")
+    N, C, H, W = y.shape
+    if bias.numel() != C:
+        raise RuntimeError("conv_epilogue_maxpool: %d bias values for %d channels" % (bias.numel(), C))
+    k, s, p = kernel_size, stride, padding
+    if not (0 < k <= 3 and 0 < s <= k and 0 <= 2 * p <= k and H + 2 * p >= k and W + 2 * p >= k
+            and H * W * 4 <= MAXPOOL_PLANE_BYTES):
+        return None
+    r = torch.empty_like(y)
+    pooled = y.new_empty((N, C, (H + 2 * p - k) // s + 1, (W + 2 * p - k) // s + 1))
+    with _Timed("conv_epilogue_maxpool", 1, y.numel() * 12 + pooled.numel() * 4, y.device, ("conv_epilogue",)):
+        check(lib().pq_conv_epilogue_maxpool_f32(y.data_ptr(), bias.data_ptr(), N, C, H, W, r.data_ptr(),
+                                                 pooled.data_ptr(), k, s, p, max_slot, _stream(y)),
+              "pq_conv_epilogue_maxpool_f32")
+    return r, pooled
 
 
 def eltwise_add(a, b, relu=False, max_slot=None):

@@ -102,7 +102,7 @@ extern "C" int pq_absmax_per_channel_f32(const float *x, uint64_t outer, int cha
 namespace {
 bool aligned16(const void *p) { return (((unsigned long long)p) & 15ull) == 0; }
 
-int launch_epilogue(pq::EpiArgs &p, int mode, cudaStream_t stream)
+int launch_epilogue(pq::EpiArgs &p, int mode, cudaStream_t stream, const pq::AddendArgs *q = nullptr)
 {
     const unsigned long long nvec = p.n >> 2;
     if (nvec >= (1ull << 31) || (mode == pq::EPI_BIAS1 && p.n >= (1ull << 31))) return PQ_EUNSUPPORTED;
@@ -112,10 +112,32 @@ int launch_epilogue(pq::EpiArgs &p, int mode, cudaStream_t stream)
     if (blocks > (unsigned long long)pq::kNumSMs * 8) blocks = (unsigned long long)pq::kNumSMs * 8;
     if (blocks == 0) blocks = 1;
     const unsigned int g = (unsigned int)blocks;
-    if (mode == pq::EPI_BIAS4) pq::epilogue_kernel<pq::EPI_BIAS4><<<g, pq::kStatThreads, 0, stream>>>(p);
+    if (q && mode == pq::EPI_BIAS4) pq::epilogue_kernel<pq::EPI_BIAS4><<<g, pq::kStatThreads, 0, stream>>>(p, *q);
+    else if (q) pq::epilogue_kernel<pq::EPI_BIAS1><<<g, pq::kStatThreads, 0, stream>>>(p, *q);
+    else if (mode == pq::EPI_BIAS4) pq::epilogue_kernel<pq::EPI_BIAS4><<<g, pq::kStatThreads, 0, stream>>>(p);
     else if (mode == pq::EPI_BIAS1) pq::epilogue_kernel<pq::EPI_BIAS1><<<g, pq::kStatThreads, 0, stream>>>(p);
     else pq::epilogue_kernel<pq::EPI_ADD><<<g, pq::kStatThreads, 0, stream>>>(p);
     return (int)cudaGetLastError();
+}
+
+// the conv epilogue's arguments and mode; PQ_OK or the error code
+int conv_epilogue_args(pq::EpiArgs &p, int &mode, float *y, const float *bias, int N, int C, uint64_t hw,
+                       float *relu_out, uint32_t *max_slot)
+{
+    if (!y || !bias || relu_out == y) return PQ_EINVAL;
+    if (!aligned16(y) || !aligned16(relu_out) || (((unsigned long long)bias) & 3ull)) return PQ_EALIGN;
+    if (hw >= (1ull << 31) || (uint64_t)N * (uint64_t)C >= (1ull << 31)) return PQ_EUNSUPPORTED;
+    p = {};
+    p.a = y;
+    p.b = bias;
+    p.out = y;
+    p.relu_out = relu_out;
+    p.max_slot = max_slot;
+    p.n = (uint64_t)N * (uint64_t)C * hw;
+    p.channels = (unsigned int)C;
+    mode = (hw & 3) == 0 ? pq::EPI_BIAS4 : pq::EPI_BIAS1;
+    p.hw = (unsigned int)(mode == pq::EPI_BIAS4 ? hw / 4 : hw);
+    return PQ_OK;
 }
 }  // namespace
 
@@ -124,20 +146,68 @@ extern "C" int pq_conv_epilogue_f32(float *y, const float *bias, int N, int C, u
 {
     if (N < 0 || C <= 0) return PQ_EINVAL;
     if (N == 0 || hw == 0) return PQ_OK;
-    if (!y || !bias || relu_out == y) return PQ_EINVAL;
-    if (!aligned16(y) || !aligned16(relu_out) || (((unsigned long long)bias) & 3ull)) return PQ_EALIGN;
-    if (hw >= (1ull << 31) || (uint64_t)N * (uint64_t)C >= (1ull << 31)) return PQ_EUNSUPPORTED;
-    pq::EpiArgs p = {};
-    p.a = y;
-    p.b = bias;
-    p.out = y;
+    pq::EpiArgs p;
+    int mode;
+    const int rc = conv_epilogue_args(p, mode, y, bias, N, C, hw, relu_out, max_slot);
+    return rc != PQ_OK ? rc : launch_epilogue(p, mode, (cudaStream_t)stream);
+}
+
+extern "C" int pq_conv_epilogue_add_f32(float *y, const float *bias, int N, int C, uint64_t hw, const float *other,
+                                        int other_first, float *z, float *relu_out, uint32_t *max_slot,
+                                        uint32_t *max_z, pq_stream_t stream)
+{
+    if (N < 0 || C <= 0) return PQ_EINVAL;
+    if (N == 0 || hw == 0) return PQ_OK;
+    if (!other || !z || z == y || z == other || other == y || relu_out == other || relu_out == z) return PQ_EINVAL;
+    if (!aligned16(other) || !aligned16(z)) return PQ_EALIGN;
+    pq::EpiArgs p;
+    int mode;
+    const int rc = conv_epilogue_args(p, mode, y, bias, N, C, hw, relu_out, max_slot);
+    if (rc != PQ_OK) return rc;
+    const pq::AddendArgs q = {other, z, max_z, other_first != 0};
+    return launch_epilogue(p, mode, (cudaStream_t)stream, &q);
+}
+
+extern "C" int pq_conv_epilogue_maxpool_f32(float *y, const float *bias, int N, int C, int H, int W, float *relu_out,
+                                            float *pool_out, int k, int s, int pad, uint32_t *max_slot,
+                                            pq_stream_t stream)
+{
+    if (N < 0 || C <= 0 || H <= 0 || W <= 0 || k <= 0 || s <= 0 || pad < 0) return PQ_EINVAL;
+    if (!y || !bias || !relu_out || !pool_out || relu_out == y || pool_out == y || pool_out == relu_out)
+        return PQ_EINVAL;
+    if (!aligned16(y) || !aligned16(relu_out) || (((unsigned long long)bias) & 3ull) ||
+        (((unsigned long long)pool_out) & 3ull))
+        return PQ_EALIGN;
+    if (k > 3 || s > k || 2 * pad > k || (uint64_t)H * W * 4 > (uint64_t)PQ_MAXPOOL_PLANE_BYTES || H + 2 * pad < k ||
+        W + 2 * pad < k || (uint64_t)N * C >= (1ull << 31))
+        return PQ_EUNSUPPORTED;
+    if (N == 0) return PQ_OK;
+    pq::PoolArgs p;
+    p.y = y;
+    p.bias = bias;
     p.relu_out = relu_out;
+    p.pool_out = pool_out;
     p.max_slot = max_slot;
-    p.n = (uint64_t)N * (uint64_t)C * hw;
     p.channels = (unsigned int)C;
-    const int mode = (hw & 3) == 0 ? pq::EPI_BIAS4 : pq::EPI_BIAS1;
-    p.hw = (unsigned int)(mode == pq::EPI_BIAS4 ? hw / 4 : hw);
-    return launch_epilogue(p, mode, (cudaStream_t)stream);
+    p.h = (unsigned int)H;
+    p.w = (unsigned int)W;
+    p.oh = (unsigned int)((H + 2 * pad - k) / s + 1);
+    p.ow = (unsigned int)((W + 2 * pad - k) / s + 1);
+    p.k = k;
+    p.s = s;
+    p.pad = pad;
+    const size_t smem = (size_t)H * W * 4;
+    void (*const vec)(const pq::PoolArgs) = pq::epilogue_kernel<pq::EPI_BIAS4>;
+    void (*const any)(const pq::PoolArgs) = pq::epilogue_kernel<pq::EPI_BIAS1>;
+    static bool attr_set = false;
+    if (!attr_set) {
+        PQ_CUDA_TRY(cudaFuncSetAttribute(vec, cudaFuncAttributeMaxDynamicSharedMemorySize, PQ_MAXPOOL_PLANE_BYTES));
+        PQ_CUDA_TRY(cudaFuncSetAttribute(any, cudaFuncAttributeMaxDynamicSharedMemorySize, PQ_MAXPOOL_PLANE_BYTES));
+        attr_set = true;
+    }
+    const bool whole = (((uint64_t)H * W) & 3) == 0;
+    (whole ? vec : any)<<<(unsigned int)(N * C), pq::kStatThreads, smem, (cudaStream_t)stream>>>(p);
+    return (int)cudaGetLastError();
 }
 
 extern "C" int pq_eltwise_add_f32(const float *a, const float *b, float *z, size_t n, float *relu_out,

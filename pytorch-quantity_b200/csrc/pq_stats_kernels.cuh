@@ -288,6 +288,9 @@ absmax_periodic_kernel(const float4 *__restrict__ x, unsigned int vec_per_img, u
 //   EPI_BIAS1 : the same for any plane size (7x7): the channel is found for the first element of the float4 and
 //               stepped for the other three (hw = elements per plane)
 //   EPI_ADD   : Eltwise, out = a + b out of place
+// With ADDEND (EPI_BIAS* only) the launch also runs the Eltwise that reads the conv output: z = first + second, in the
+// Eltwise's operand order, where one operand is the biased conv output and the other is `other` [n]; relu_out takes
+// relu(z) instead of relu(out), *max_slot max |out| and *max_z max |z|.
 // Grid-stride over float4 with kEpiUnroll float4 per operand in flight per thread; n % 4 tail scalars in CTA 0.
 enum EpiMode { EPI_BIAS4 = 0, EPI_BIAS1 = 1, EPI_ADD = 2 };
 constexpr int kEpiUnroll = 4;
@@ -304,8 +307,31 @@ struct EpiArgs {
     int s_hw, s_chan;
 };
 
+// ADDEND: the Eltwise that reads the conv output
+struct AddendArgs {
+    const float *other;         // the Eltwise's other operand [n]
+    float *z;                   // the Eltwise's output [n]
+    unsigned int *max_z;        // may be null
+    int other_first;            // z = other + out (else out + other)
+};
+
 // ATen's clamp_min(v, 0) (launch_clamp_scalar): NaN propagates, otherwise max(v, 0)
 __device__ __forceinline__ float relu_aten(float v) { return isnan(v) ? v : fmaxf(v, 0.0f); }
+
+__device__ __forceinline__ unsigned int absmax4(unsigned int m, const float4 &o)
+{
+    return max(max(m, max(absbits(o.x), absbits(o.y))), max(absbits(o.z), absbits(o.w)));
+}
+
+__device__ __forceinline__ float4 relu4(const float4 &o)
+{
+    return make_float4(relu_aten(o.x), relu_aten(o.y), relu_aten(o.z), relu_aten(o.w));
+}
+
+__device__ __forceinline__ float4 add4(const float4 &a, const float4 &b)
+{
+    return make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+}
 
 template <int MODE>
 __device__ __forceinline__ float4 epi_load_a(const EpiArgs &p, unsigned int i)
@@ -341,36 +367,47 @@ __device__ __forceinline__ float4 epi_load_b(const EpiArgs &p, unsigned int i)
     return make_float4(v[0], v[1], v[2], v[3]);
 }
 
-__device__ __forceinline__ void epi_store(const EpiArgs &p, unsigned int i, const float4 &a, const float4 &b,
-                                          unsigned int &m)
+template <bool ADDEND>
+__device__ __forceinline__ void epi_store(const EpiArgs &p, const AddendArgs &q, unsigned int i, const float4 &a,
+                                          const float4 &b, const float4 &other, unsigned int &m, unsigned int &mz)
 {
-    const float4 o = make_float4(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y), __fadd_rn(a.z, b.z), __fadd_rn(a.w, b.w));
+    const float4 o = add4(a, b);
     __stcs(reinterpret_cast<float4 *>(p.out) + i, o);
-    if (p.relu_out)
-        reinterpret_cast<float4 *>(p.relu_out)[i] = make_float4(relu_aten(o.x), relu_aten(o.y), relu_aten(o.z),
-                                                                relu_aten(o.w));
-    m = max(max(m, max(absbits(o.x), absbits(o.y))), max(absbits(o.z), absbits(o.w)));
+    m = absmax4(m, o);
+    if (ADDEND) {
+        const float4 z = q.other_first ? add4(other, o) : add4(o, other);
+        __stcs(reinterpret_cast<float4 *>(q.z) + i, z);
+        if (p.relu_out) reinterpret_cast<float4 *>(p.relu_out)[i] = relu4(z);
+        mz = absmax4(mz, z);
+    } else if (p.relu_out) {
+        reinterpret_cast<float4 *>(p.relu_out)[i] = relu4(o);
+    }
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(kStatThreads)
-epilogue_kernel(const EpiArgs p)
+template <int MODE, bool ADDEND>
+__device__ __forceinline__ void epilogue_body(const EpiArgs &p, const AddendArgs &q)
 {
     __shared__ unsigned int s_warp[kStatThreads / 32];
     const unsigned int nvec = (unsigned int)(p.n >> 2);
     const unsigned int stride = gridDim.x * kStatThreads;
+    const float4 *other4 = reinterpret_cast<const float4 *>(q.other);
+    const float4 none = make_float4(0.f, 0.f, 0.f, 0.f);
     unsigned int i = blockIdx.x * kStatThreads + threadIdx.x;
-    unsigned int m = 0;
+    unsigned int m = 0, mz = 0;
     for (; i + (kEpiUnroll - 1) * stride < nvec; i += kEpiUnroll * stride) {
-        float4 a[kEpiUnroll], b[kEpiUnroll];
+        float4 a[kEpiUnroll], b[kEpiUnroll], o[kEpiUnroll];
 #pragma unroll
         for (int u = 0; u < kEpiUnroll; ++u) a[u] = epi_load_a<MODE>(p, i + u * stride);
 #pragma unroll
+        for (int u = 0; u < kEpiUnroll; ++u) o[u] = ADDEND ? ld_stream_f4(other4 + i + u * stride) : none;
+#pragma unroll
         for (int u = 0; u < kEpiUnroll; ++u) b[u] = epi_load_b<MODE>(p, i + u * stride);
 #pragma unroll
-        for (int u = 0; u < kEpiUnroll; ++u) epi_store(p, i + u * stride, a[u], b[u], m);
+        for (int u = 0; u < kEpiUnroll; ++u) epi_store<ADDEND>(p, q, i + u * stride, a[u], b[u], o[u], m, mz);
     }
-    for (; i < nvec; i += stride) epi_store(p, i, epi_load_a<MODE>(p, i), epi_load_b<MODE>(p, i), m);
+    for (; i < nvec; i += stride)
+        epi_store<ADDEND>(p, q, i, epi_load_a<MODE>(p, i), epi_load_b<MODE>(p, i),
+                          ADDEND ? ld_stream_f4(other4 + i) : none, m, mz);
     const unsigned long long t = ((unsigned long long)nvec << 2) + blockIdx.x * kStatThreads + threadIdx.x;
     if (t < p.n) {                                         // the n % 4 tail: threads 0..2 of CTA 0
         float b;
@@ -378,8 +415,114 @@ epilogue_kernel(const EpiArgs p)
         else b = __ldg(p.b + (unsigned int)((t / (MODE == EPI_BIAS4 ? 4ull * p.hw : p.hw)) % p.channels));
         const float o = __fadd_rn(p.a[t], b);
         p.out[t] = o;
-        if (p.relu_out) p.relu_out[t] = relu_aten(o);
         m = max(m, absbits(o));
+        if (ADDEND) {
+            const float z = q.other_first ? __fadd_rn(q.other[t], o) : __fadd_rn(o, q.other[t]);
+            q.z[t] = z;
+            if (p.relu_out) p.relu_out[t] = relu_aten(z);
+            mz = max(mz, absbits(z));
+        } else if (p.relu_out) {
+            p.relu_out[t] = relu_aten(o);
+        }
+    }
+    if (p.max_slot) block_max_publish(m, s_warp, p.max_slot);
+    if (ADDEND && q.max_z) block_max_publish(mz, s_warp, q.max_z);
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(kStatThreads)
+epilogue_kernel(const EpiArgs p)
+{
+    epilogue_body<MODE, false>(p, AddendArgs{});
+}
+
+// the conv epilogue (MODE EPI_BIAS4 / EPI_BIAS1) with the Eltwise that reads its output
+template <int MODE>
+__global__ void __launch_bounds__(kStatThreads)
+epilogue_kernel(const EpiArgs p, const AddendArgs q)
+{
+    epilogue_body<MODE, true>(p, q);
+}
+
+// The stem's conv epilogue with the max-pool that follows its ReLU (nn.Conv2d -> nn.ReLU -> nn.MaxPool2d), MODE
+// EPI_BIAS4 for planes of whole float4 (H * W % 4 == 0), EPI_BIAS1 for any: one CTA
+// owns one [H][W] plane, so the whole plane is one channel (one bias value) and no other CTA reads it.  The CTA
+//   adds the bias in place (max |y| -> *max_slot), writes relu(y) to relu_out and keeps it in shared memory, then
+//   writes max_pool2d(relu(y), k, s, p) to pool_out [OH][OW].
+// The pool is ATen's max_pool_forward_nchw bit for bit: each window is scanned row-major from -inf and the running
+// maximum is replaced when `v > max || isnan(v)`, so the last NaN of the window wins with its payload and a tie keeps
+// the first value (+0 / -0).  Padding only ever shortens a window (p <= k / 2), it never empties one.
+struct PoolArgs {
+    float *y;
+    const float *bias;
+    float *relu_out, *pool_out;
+    unsigned int *max_slot;     // may be null
+    unsigned int channels, h, w, oh, ow;
+    int k, s, pad;
+};
+
+template <int MODE>
+__global__ void __launch_bounds__(kStatThreads)
+epilogue_kernel(const PoolArgs p)
+{
+    extern __shared__ float s_plane[];                     // relu(y) of the plane, [h][w]
+    __shared__ unsigned int s_warp[kStatThreads / 32];
+    const unsigned int hw = p.h * p.w;
+    const size_t base = (size_t)blockIdx.x * hw;
+    const float bias = __ldg(p.bias + blockIdx.x % p.channels);
+    unsigned int m = 0;
+    if (MODE == EPI_BIAS4) {
+        float4 *y4 = reinterpret_cast<float4 *>(p.y + base);
+        float4 *r4 = reinterpret_cast<float4 *>(p.relu_out + base);
+        const unsigned int nvec = hw >> 2;
+        const float4 b = make_float4(bias, bias, bias, bias);
+        unsigned int i = threadIdx.x;
+        for (; i + (kEpiUnroll - 1) * kStatThreads < nvec; i += kEpiUnroll * kStatThreads) {
+            float4 v[kEpiUnroll];
+#pragma unroll
+            for (int u = 0; u < kEpiUnroll; ++u) v[u] = __ldcs(y4 + i + u * kStatThreads);
+#pragma unroll
+            for (int u = 0; u < kEpiUnroll; ++u) {
+                const float4 o = add4(v[u], b);
+                const float4 r = relu4(o);
+                __stcs(y4 + i + u * kStatThreads, o);
+                __stcs(r4 + i + u * kStatThreads, r);
+                reinterpret_cast<float4 *>(s_plane)[i + u * kStatThreads] = r;
+                m = absmax4(m, o);
+            }
+        }
+        for (; i < nvec; i += kStatThreads) {
+            const float4 o = add4(__ldcs(y4 + i), b);
+            const float4 r = relu4(o);
+            __stcs(y4 + i, o);
+            __stcs(r4 + i, r);
+            reinterpret_cast<float4 *>(s_plane)[i] = r;
+            m = absmax4(m, o);
+        }
+    } else {
+        for (unsigned int i = threadIdx.x; i < hw; i += kStatThreads) {
+            const float o = __fadd_rn(p.y[base + i], bias);
+            const float r = relu_aten(o);
+            p.y[base + i] = o;
+            p.relu_out[base + i] = r;
+            s_plane[i] = r;
+            m = max(m, absbits(o));
+        }
+    }
+    __syncthreads();
+    const unsigned int ohw = p.oh * p.ow;
+    float *dst = p.pool_out + (size_t)blockIdx.x * ohw;
+    for (unsigned int o = threadIdx.x; o < ohw; o += kStatThreads) {
+        const int oy = (int)(o / p.ow), ox = (int)(o - (unsigned int)oy * p.ow);
+        const int y0 = oy * p.s - p.pad, x0 = ox * p.s - p.pad;
+        const int y1 = min(y0 + p.k, (int)p.h), x1 = min(x0 + p.k, (int)p.w);
+        float mx = -INFINITY;
+        for (int yy = max(y0, 0); yy < y1; ++yy)
+            for (int xx = max(x0, 0); xx < x1; ++xx) {
+                const float v = s_plane[yy * (int)p.w + xx];
+                if (v > mx || isnan(v)) mx = v;
+            }
+        __stcs(dst + o, mx);
     }
     if (p.max_slot) block_max_publish(m, s_warp, p.max_slot);
 }

@@ -15,8 +15,9 @@ What is different from the reference, by design (B200-first):
     tables are bit-identical for any rank count;
   * the KL threshold search for all tensors is one GPU launch sequence;
   * during calibration the bias add after every cuDNN convolution, each Eltwise and the out-of-place nn.ReLU that
-    follows either run as one native kernel that also takes the pass-1 max-abs (plan_calibration_fusion), with
-    bit-identical results;
+    follows either run as one native kernel that also takes the pass-1 max-abs (plan_calibration_fusion); the
+    convolution that completes an Eltwise's operands also computes the Eltwise, and the stem's convolution the
+    max-pool after its ReLU (plan_calibration_handover), all with bit-identical results;
   * producer/consumer links are traced by tensor identity instead of a value hash.
 """
 import json
@@ -93,30 +94,106 @@ def plan_calibration_fusion(net, modules, inplace_modified):
     return plan
 
 
+def plan_calibration_handover(net, modules, plan):
+    """The hand-overs between the fused ops of ``plan`` (plan_calibration_fusion), from the same trace.  Returns
+    (eltwise, pools):
+      * eltwise: {Eltwise tracer name: (producer, other, producer_first)} for every planned Eltwise whose two operands
+        come from two traced modules, where ``producer`` -- the operand producer that fires last -- is a planned
+        convolution without a fused ReLU.  Its fused forward also computes the Eltwise (pq_conv_epilogue_add_f32)
+        when the traced tensor ``other`` of the other operand exists unmodified; ``producer_first``: the producer's
+        output is the Eltwise's first operand.
+      * pools: {convolution tracer name: MaxPool2d tracer name} for every planned
+        convolution whose fused ReLU's only consumer is a plain nn.MaxPool2d without indices, dilation or ceil_mode
+        that fired once: its fused forward also computes the pooled output (pq_conv_epilogue_maxpool_f32)."""
+    calls = Counter(id(m) for m in modules.values())
+    consumers = {}
+    for name, info in net.items():
+        for src in info["inputs"]:
+            consumers.setdefault(src, []).append(name)
+    name_of = {id(m): n for n, m in modules.items()}
+
+    def pos(name):
+        return int(name.rsplit("_", 1)[1])
+
+    eltwise = OrderedDict()
+    for name, (m, _relu) in plan.items():
+        srcs = net[name]["inputs"]
+        if type(m) is not Eltwise or len(srcs) != 2 or srcs[0] == srcs[1]:
+            continue
+        last = max(srcs, key=pos)
+        if last in plan and isinstance(plan[last][0], nn.Conv2d) and plan[last][1] is None:
+            eltwise[name] = (last, srcs[1] if last == srcs[0] else srcs[0], last == srcs[0])
+
+    def pair(v):
+        return tuple(v) if isinstance(v, (tuple, list)) else (v, v)
+
+    pools = OrderedDict()
+    for name, (m, relu) in plan.items():
+        if relu is None or not isinstance(m, nn.Conv2d):
+            continue
+        relu_name = name_of[id(relu)]
+        after = consumers.get(relu_name, [])
+        if len(after) != 1:
+            continue
+        pool = modules[after[0]]
+        if (type(pool) is nn.MaxPool2d and calls[id(pool)] == 1 and "forward" not in vars(pool)
+                and not pool.return_indices and not pool.ceil_mode and pair(pool.dilation) == (1, 1)
+                and len(set(pair(pool.kernel_size))) == 1 and len(set(pair(pool.stride))) == 1
+                and len(set(pair(pool.padding))) == 1):
+            pools[name] = after[0]
+    return eltwise, pools
+
+
 class _CalibrationFusion:
-    """The fused forwards of a plan (plan_calibration_fusion) for one activation_quantize call: install() sets them as
-    instance attributes, remove() restores the modules.
+    """The fused forwards of a plan (plan_calibration_fusion) and its hand-overs (plan_calibration_handover) for one
+    activation_quantize call: install() sets them as instance attributes, remove() restores the modules.
 
     Each fused op is one native launch on the stream current at the call.  While ``collect`` is set (pass 1) a fused
     op whose output the collector observes (``slots``: tensor name -> its max_bits slot) also takes the max |x| of
     that output into the slot, provided it runs at its traced position in the forward (the calibration hooks' count),
-    and adds the name to ``reduced``; refresh_max_val then skips those tensors.  A fused op that also computed its
-    consumer ReLU's output hands it over only if that ReLU is called with the very tensor, unmodified; any other
-    call runs the ReLU's own forward."""
+    and adds the name to ``reduced``; refresh_max_val then skips those tensors.
 
-    def __init__(self, plan, hook_state, slots, device):
+    A fused op may also compute a consumer's output speculatively: the convolution its ReLU's (and the stem's
+    max-pool's), the convolution that completes an Eltwise's operands the Eltwise's.  The consumer returns it only if
+    it is called with the very tensors, unmodified; any other call runs the consumer's own forward.  Every module's
+    output is complete when the module returns.  A speculated Eltwise takes its max |z| into a pending slot; fold()
+    moves it to max_bits only when the Eltwise took z at its traced position."""
+
+    def __init__(self, plan, handover, modules, hook_state, slots, max_bits, device):
         self.collect = False
         self.reduced = set()
         self._state = hook_state
         self._device = device
+        eltwise, pools = handover
+        name_of = {id(m): n for n, m in modules.items()}
+        # Per forward (begin() clears them): the outputs of fused ops and of handed-over ReLUs / max-pools that an
+        # Eltwise hand-over reads as its other operand (tracer name -> (tensor, _version)), and the speculated Eltwise
+        # outputs (tracer name -> (a, a._version, b, b._version, z, relu(z) or None)).
+        self._others = {other for _, other, _ in eltwise.values()}
+        self._outputs = {}
+        self._speculated = {}
+        # max |z| of a speculated Eltwise: pending[i] for max_bits[i], folded in once the hand-over is confirmed
+        self._max_bits = max_bits
+        self._pending = torch.zeros_like(max_bits) if max_bits is not None and eltwise else None
+        self._published = set()     # pending indices written this forward
+        self._confirmed = set()     # ... and confirmed
         self._forwards = []         # (module, fused forward), all built before any module is touched
         for name, (m, relu) in plan.items():
-            stash = [None] if relu is not None else None
+            relu_stash = [None] if relu is not None else None
             pos = int(name.rsplit("_", 1)[1])
-            make = self._conv if isinstance(m, nn.Conv2d) else self._eltwise
-            self._forwards.append((m, make(m, name, pos, slots.get(name), stash)))
+            if isinstance(m, nn.Conv2d):
+                adds = [(e, other, first, slots.get(e), plan[e][1] is not None)
+                        for e, (producer, other, first) in eltwise.items() if producer == name]
+                pool = None
+                if name in pools:
+                    pool = (modules[pools[name]], [None])
+                    self._forwards.append((pool[0], self._pool(pool[0], pools[name], pool[1])))
+                fwd = self._conv(m, name, pos, slots.get(name), relu_stash, adds[0] if adds else None, pool)
+            else:
+                fwd = self._eltwise(m, name, pos, slots.get(name), relu_stash)
+            self._forwards.append((m, fwd))
             if relu is not None:
-                self._forwards.append((relu, self._relu(relu, stash)))
+                self._forwards.append((relu, self._relu(relu, name_of[id(relu)], relu_stash)))
         self._patched = []
 
     def install(self):
@@ -128,18 +205,44 @@ class _CalibrationFusion:
         for m in self._patched:
             del m.forward
         self._patched = []
+        self.begin()
+
+    def begin(self):
+        """A forward begins: nothing the last one computed can be handed over any more."""
+        self._outputs.clear()
+        self._speculated.clear()
+
+    def fold(self):
+        """Pass 1, after a forward: the confirmed speculative maxima into max_bits (an integer max, order-free like
+        the kernels' atomicMax), the others dropped, the pending slots cleared for the next forward."""
+        if not self._published:
+            return
+        for i in self._published - self._confirmed:
+            self._pending[i] = 0
+        if self._confirmed:
+            torch.maximum(self._max_bits, self._pending, out=self._max_bits)
+        self._pending.zero_()
+        self._published.clear()
+        self._confirmed.clear()
 
     def _fusable(self, t):
         return (isinstance(t, torch.Tensor) and t.device == self._device and t.dtype == torch.float32
                 and t.is_contiguous() and t.data_ptr() % 16 == 0)
 
+    def _at_position(self, pos):
+        return self.collect and self._state["idx"] == pos - 1
+
     def _slot(self, name, pos, slot):
-        if slot is not None and self.collect and self._state["idx"] == pos - 1:
+        if slot is not None and self._at_position(pos):
             self.reduced.add(name)
             return slot
         return None
 
-    def _conv(self, m, name, pos, slot, stash):
+    def _output(self, name, t):
+        if name in self._others:
+            self._outputs[name] = (t, t._version)
+
+    def _conv(self, m, name, pos, slot, relu_stash, add, pool):
         own = m.forward
         cudnn = {}                  # input shape -> does cuDNN run this convolution (bias included)?
 
@@ -152,6 +255,35 @@ class _CalibrationFusion:
                                                      (0, 0), m.groups) == torch._C._ConvBackend.Cudnn
             except (TypeError, RuntimeError):
                 return False
+
+        def epilogue(y):
+            max_slot = self._slot(name, pos, slot)
+            if add is not None:
+                elt, other_name, first, elt_slot, elt_relu = add
+                got = self._outputs.get(other_name)
+                if got is not None and got[0]._version == got[1] and self._fusable(got[0]) \
+                        and got[0].shape == y.shape:
+                    other = got[0]
+                    i = max_z = None
+                    if elt_slot is not None and self.collect:
+                        i = (elt_slot - self._max_bits.data_ptr()) // 4
+                        max_z = self._pending.data_ptr() + 4 * i
+                        self._published.add(i)
+                    z, r = _native.conv_epilogue_add(y, m.bias, other, not first, elt_relu, max_slot, max_z)
+                    a, b = (y, other) if first else (other, y)
+                    self._speculated[elt] = (a, a._version, b, b._version, z, r, i)
+                    return
+            if pool is not None:
+                k, s, p = (v if isinstance(v, int) else v[0]
+                           for v in (pool[0].kernel_size, pool[0].stride, pool[0].padding))
+                got = _native.conv_epilogue_maxpool(y, m.bias, k, s, p, max_slot)
+                if got is not None:
+                    relu_stash[0] = (y, y._version, got[0])
+                    pool[1][0] = (got[0], got[0]._version, got[1])
+                    return
+            r = _native.conv_epilogue(y, m.bias, relu_stash is not None, max_slot)
+            if relu_stash is not None:
+                relu_stash[0] = (y, y._version, r)
 
         def forward(x):
             # under autocast the convolution runs in 16 bits with the bias cast alongside: the module's own forward
@@ -166,32 +298,49 @@ class _CalibrationFusion:
             y = F.conv2d(x, m.weight, None, m.stride, m.padding, m.dilation, m.groups)
             if y.dtype != torch.float32 or not y.is_contiguous():     # (a channels_last weight) ATen's own bias add
                 return y.add_(m.bias.reshape(1, -1, 1, 1))
-            r = _native.conv_epilogue(y, m.bias, stash is not None, self._slot(name, pos, slot))
-            if stash is not None:
-                stash[0] = (y, y._version, r)
+            epilogue(y)
+            self._output(name, y)
             return y
         return forward
 
-    def _eltwise(self, m, name, pos, slot, stash):
+    def _eltwise(self, m, name, pos, slot, relu_stash):
         own = m.forward
 
         def forward(a, b):
-            # (torch.add is not an autocast op: fp32 operands give the fp32 sum with autocast on or off)
-            if torch.is_grad_enabled() or not (self._fusable(a) and self._fusable(b)) or a.shape != b.shape:
-                return own(a, b)
-            z, r = _native.eltwise_add(a, b, stash is not None, self._slot(name, pos, slot))
-            if stash is not None:
-                stash[0] = (z, z._version, r)
+            spec = self._speculated.pop(name, None)
+            if spec is not None and a is spec[0] and a._version == spec[1] and b is spec[2] and b._version == spec[3]:
+                z, r, i = spec[4], spec[5], spec[6]
+                if i is not None and self._slot(name, pos, slot) is not None:
+                    self._confirmed.add(i)
+            else:
+                # (torch.add is not an autocast op: fp32 operands give the fp32 sum with autocast on or off)
+                if torch.is_grad_enabled() or not (self._fusable(a) and self._fusable(b)) or a.shape != b.shape:
+                    return own(a, b)
+                z, r = _native.eltwise_add(a, b, relu_stash is not None, self._slot(name, pos, slot))
+            if relu_stash is not None:
+                relu_stash[0] = (z, z._version, r)
+            self._output(name, z)
             return z
         return forward
 
-    @staticmethod
-    def _relu(relu, stash):
+    def _relu(self, relu, name, stash):
         own = relu.forward
 
         def forward(x):
             st, stash[0] = stash[0], None
             if st is not None and x is st[0] and x._version == st[1]:
+                self._output(name, st[2])
+                return st[2]
+            return own(x)
+        return forward
+
+    def _pool(self, pool, name, stash):
+        own = pool.forward
+
+        def forward(x):
+            st, stash[0] = stash[0], None
+            if st is not None and x is st[0] and x._version == st[1]:
+                self._output(name, st[2])
                 return st[2]
             return own(x)
         return forward
@@ -299,6 +448,8 @@ class Quantity(object):
         # exactly these tensors (and only these) to record the same values.
         self._inplace_modified = {n for n, t, v in observed if t._version != v}
         self._fusion_plan = plan_calibration_fusion(net, modules, self._inplace_modified)
+        self._handover_plan = plan_calibration_handover(net, modules, self._fusion_plan)
+        self._traced_modules = modules
         keep = [n for n, info in net.items() if info["type"] in self._cared_op_type]
         return self.prune_net_info(net, keep)
 
@@ -510,15 +661,19 @@ class Quantity(object):
         plan = self._fusion_plan if self._fuse_calibration else {}
         # max slots only for the tensors the collector observes (CARE_OP_TYPE); the other fused ops take no max
         slots = {n: collector._max_slot(n) for n in plan if n in top_feat_names}
-        fusion = _CalibrationFusion(plan, self._feat_state, slots, self.cuda_device)
+        handover = self._handover_plan if self._fuse_calibration else ({}, {})
+        fusion = _CalibrationFusion(plan, handover, self._traced_modules, self._feat_state, slots,
+                                    collector.device_state()[0] if slots else None, self.cuda_device)
         try:
             fusion.install()
             fusion.collect = True
             for i, img in self._device_batches(images_files):                    # pass 1  (:379-390)
                 fusion.reduced.clear()
+                fusion.begin()
                 self._forward_device(self.model, img)
                 self._check_unmodified(named_feats)
                 feats = {n: named_feats[n] for n in top_feat_names}
+                fusion.fold()
                 collector._refresh_max_val_except(feats, fusion.reduced)
                 nbytes = sum(t.numel() * t.element_size() for t in feats.values())
                 if cached_bytes + nbytes <= budget:
@@ -552,6 +707,7 @@ class Quantity(object):
                 if img is None:
                     feats = cache.pop(i)
                 else:
+                    fusion.begin()
                     self._forward_device(self.model, img)
                     self._check_unmodified(named_feats)
                     feats = {n: named_feats[n] for n in top_feat_names}
