@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 204
+#define PQ_VERSION 205
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -350,6 +350,34 @@ typedef struct pq_concat_src {
 } pq_concat_src;
 int pq_concat_requant_s8(const pq_concat_src *srcs_host, int k, size_t pixels, int q_bit, int c_out_pad,
                          int8_t *out, pq_stream_t stream);
+
+/* Nearest-neighbour upsampling (nn.UpsamplingNearest2d, nn.Upsample, F.interpolate(mode='nearest'); listed in the
+ * tracer's tools/configs.yml:21-22) read through index tables instead of being written: output pixel (n, p, q) reads
+ * source pixel (n, map_h[p], map_w[q]).  The tables are int32 [P] and [Q], built from ATen's own nearest rule.  A
+ * gather commutes exactly with the quantiser, with ReLU and with the exact int16 sum, so both entry points below
+ * equal their same-resolution counterparts applied to the gathered operand.
+ * pq_add_requant_nearest: pq_add_requant (flags, bit ranges, relu on load, either output NULL) on a, out16 and out8
+ *   [N][P][Q][C], with operand b an int8 or int16 [N][Hb][Wb][C] tensor read through the tables.  16-byte aligned.
+ * pq_concat_requant_nearest_s8: pq_concat_requant_s8 producing [N][P][Q][c_out_pad], where source i is
+ *   [N][H][W][channels] read through its own tables, or at the same pixel when both are NULL (then H == P, W == Q,
+ *   else PQ_EINVAL).  The vector path needs every channel count and c_out_pad % 16 == 0 and 16-byte aligned buffers;
+ *   anything else takes the scalar path.
+ * Precondition (not checked): 0 <= map_h[p] < Hb (H) and 0 <= map_w[q] < Wb (W).  Outside these limits the call
+ * returns PQ_EUNSUPPORTED and writes nothing:
+ *   nearest limit: C % 16 == 0;  (pq_add_requant_nearest)
+ *   nearest limit: N*P*Q <= 2^31 - 1; */
+typedef struct pq_concat_nearest_src {
+    const void *ptr;
+    int is16, channels, bit, relu;   /* as pq_concat_src */
+    int H, W;                        /* source height / width */
+    const int32_t *map_h, *map_w;    /* [P] / [Q] source row / column, or both NULL */
+} pq_concat_nearest_src;
+int pq_add_requant_nearest(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16, int b_bit,
+                           int b_relu, int N, int P, int Q, int C, int Hb, int Wb, const int32_t *map_h,
+                           const int32_t *map_w, int flags, int16_t *out16, int8_t *out8, int q_bit,
+                           pq_stream_t stream);
+int pq_concat_requant_nearest_s8(const pq_concat_nearest_src *srcs_host, int k, int N, int P, int Q, int q_bit,
+                                 int c_out_pad, int8_t *out, pq_stream_t stream);
 
 /* NewConv2d + NewAdd (+ the nn.ReLU after the Eltwise) in ONE kernel: the conv / GEMM epilogue adds the
  * shortcut operand and writes the exact int16 sum and its int8 requantisation, exactly as pq_add_requant

@@ -21,7 +21,7 @@ KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
 KL_MAX_ROWS = 65535          # tensors per pq_kl_search_n_f64 call (one grid row per tensor)
 MAXPOOL_PLANE_BYTES = 227 * 1024 - 1024   # PQ_MAXPOOL_PLANE_BYTES: largest plane pq_conv_epilogue_maxpool_f32 takes
-PQ_VERSION = 204             # the header's PQ_VERSION: the entry points below match a library built from it
+PQ_VERSION = 205             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -59,6 +59,8 @@ SYMBOLS = {
     "pq_add_requant": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _sz, _i, _vp, _vp, _i, _vp]),
     "pq_concat_requant_s8": (_i, [_vp, _i, _sz, _i, _i, _vp, _vp]),
     "pq_bias_fold_s32": (_i, [_vp, _i, _i, _vp, _vp]),
+    "pq_add_requant_nearest": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i] + [_i] * 6 + [_vp, _vp, _i, _vp, _vp, _i, _vp]),
+    "pq_concat_requant_nearest_s8": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
 }
 FLAG_RELU = 1
 FLAG_BIAS_FOLDED = 2
@@ -83,6 +85,13 @@ class ConcatSrc(ctypes.Structure):
     """struct pq_concat_src"""
     _fields_ = [("ptr", ctypes.c_void_p), ("is16", ctypes.c_int), ("channels", ctypes.c_int),
                 ("bit", ctypes.c_int), ("relu", ctypes.c_int)]
+
+
+class ConcatNearestSrc(ctypes.Structure):
+    """struct pq_concat_nearest_src"""
+    _fields_ = [("ptr", ctypes.c_void_p), ("is16", ctypes.c_int), ("channels", ctypes.c_int), ("bit", ctypes.c_int),
+                ("relu", ctypes.c_int), ("H", ctypes.c_int), ("W", ctypes.c_int), ("map_h", ctypes.c_void_p),
+                ("map_w", ctypes.c_void_p)]
 
 
 CONCAT_MAX_SOURCES = 8
@@ -678,4 +687,60 @@ def concat_requant_s8(sources, q_bit, c_out_pad=None):
     with _Timed("concat_requant", 1, nbytes + out.numel(), first.device):
         check(lib().pq_concat_requant_s8(arr, k, N * H * W, int(q_bit), c_out_pad, out.data_ptr(), _stream(first)),
               "pq_concat_requant_s8")
+    return out
+
+
+def add_requant_nearest(a, a_bit, a_relu, b, b_bit, b_relu, map_h, map_w, q_bit, want16=True, want8=True,
+                        out_relu=False):
+    """add_requant with operand b an int8 / int16 NHWC [N][Hb][Wb][C] tensor read at (n, map_h[p], map_w[q]) for
+    output pixel (n, p, q) of a's [N][P][Q][C] (nearest-neighbour upsampling, never written at full resolution).
+    map_h / map_w: int32 CUDA [P] / [Q] with values in [0, Hb) / [0, Wb)."""
+    require_cuda(a, "add_requant_nearest")
+    N, P, Q, C = a.shape
+    Nb, Hb, Wb, Cb = b.shape
+    assert (Nb, Cb) == (N, C) and a.is_contiguous() and b.is_contiguous()
+    assert map_h.dtype == map_w.dtype == torch.int32 and map_h.numel() == P and map_w.numel() == Q
+    out16 = torch.empty(a.shape, dtype=torch.int16, device=a.device) if want16 else None
+    out8 = torch.empty(a.shape, dtype=torch.int8, device=a.device) if want8 else None
+    nbytes = a.numel() * (a.element_size() + (2 if want16 else 0) + (1 if want8 else 0)) + b.numel() * b.element_size()
+    with _Timed("add_requant_nearest", 1, nbytes, a.device):
+        check(lib().pq_add_requant_nearest(a.data_ptr(), 1 if a.dtype == torch.int16 else 0, int(a_bit),
+                                           1 if a_relu else 0, b.data_ptr(), 1 if b.dtype == torch.int16 else 0,
+                                           int(b_bit), 1 if b_relu else 0, N, P, Q, C, Hb, Wb, map_h.data_ptr(),
+                                           map_w.data_ptr(), FLAG_RELU if out_relu else 0,
+                                           out16.data_ptr() if want16 else None, out8.data_ptr() if want8 else None,
+                                           int(q_bit), _stream(a)), "pq_add_requant_nearest")
+    return out16, out8
+
+
+def concat_requant_nearest_s8(sources, out_hw, q_bit, c_out_pad=None):
+    """concat_requant_s8 at output resolution out_hw = (P, Q) where each source may be read through nearest-neighbour
+    tables.  sources: list of (payload int8 / int16 [N][H_i][W_i][C_i], bit, relu, maps), maps = (map_h, map_w) int32
+    CUDA [P] / [Q] or None (same resolution).  Returns int8 [N][P][Q][c_out_pad]."""
+    first = sources[0][0]
+    require_cuda(first, "concat_requant_nearest_s8")
+    N = first.shape[0]
+    P, Q = out_hw
+    k = len(sources)
+    if k > CONCAT_MAX_SOURCES:
+        raise RuntimeError("concat_requant_nearest_s8: at most %d sources" % CONCAT_MAX_SOURCES)
+    arr = (ConcatNearestSrc * k)()
+    c_sum = nbytes = 0
+    for i, (t, bit, relu, maps) in enumerate(sources):
+        assert t.is_contiguous() and t.shape[0] == N and t.dtype in (torch.int8, torch.int16)
+        if maps is None:
+            assert tuple(t.shape[1:3]) == (P, Q)
+        else:
+            assert maps[0].dtype == maps[1].dtype == torch.int32 and (maps[0].numel(), maps[1].numel()) == (P, Q)
+        arr[i] = ConcatNearestSrc(t.data_ptr(), 1 if t.dtype == torch.int16 else 0, t.shape[3], int(bit),
+                                  1 if relu else 0, t.shape[1], t.shape[2],
+                                  maps[0].data_ptr() if maps is not None else None,
+                                  maps[1].data_ptr() if maps is not None else None)
+        c_sum += t.shape[3]
+        nbytes += t.numel() * t.element_size()
+    c_out_pad = c_sum if c_out_pad is None else c_out_pad
+    out = torch.empty((N, P, Q, c_out_pad), dtype=torch.int8, device=first.device)
+    with _Timed("concat_requant_nearest", 1, nbytes + out.numel(), first.device):
+        check(lib().pq_concat_requant_nearest_s8(arr, k, N, P, Q, int(q_bit), c_out_pad, out.data_ptr(),
+                                                 _stream(first)), "pq_concat_requant_nearest_s8")
     return out

@@ -14,6 +14,10 @@ layers hand each other int8 NHWC payloads wrapped in a lazy ``QTensor``:
     Concat(QTensor, QTensor) / torch.cat(dim=1)     lazy: the consuming NewConv2d asks for the concatenation at
                                                     ITS input bit and one bandwidth kernel (pq_concat_requant_s8)
                                                     writes the channel-padded int8 NHWC operand directly
+    F.interpolate(QTensor, mode='nearest')          lazy view (nn.UpsamplingNearest2d, nn.Upsample): never written;
+                                                    its consumer reads the source through row / column index tables
+                                                    (a Concat or NewConv2d: pq_concat_requant_nearest_s8; a NewAdd:
+                                                    pq_add_requant_nearest)
     anything else (AvgPool2d, user code)            the QTensor de-quantises itself to fp32 NCHW first
 
 so the final output is bit-identical to the fp32-boundary model while HBM traffic drops ~4x.
@@ -93,7 +97,15 @@ class _LazyAdd:
             x, y = self.x, self.y
             if not self._fusable(x) and self._fusable(y):
                 x, y = y, x
-            if self._fusable(x):                       # conv + add (+ relu) in one kernel (always writes int8)
+            if y._upsample is not None or x._upsample is not None:
+                if x._upsample is not None:
+                    x, y = y, x
+                t, extra, tables = y._lazy_cat.view_source()      # b = the view's source, read through the tables
+                (a, abit, arelu), (b, bbit, brelu) = _operand(x), _operand(t)
+                s16, q8 = _native.add_requant_nearest(a, abit, arelu, b, bbit, brelu or extra or
+                                                      (y.relu_pending and not y.nonneg), tables.map_h, tables.map_w,
+                                                      self.q_bit, want16=want16, want8=want8, out_relu=relu)
+            elif self._fusable(x):                       # conv + add (+ relu) in one kernel (always writes int8)
                 lc = x._lazy_conv
                 sc, sc_bit, sc_relu = _operand(y)
                 s16, q8 = lc.mod._run_add(lc.operand, sc, sc_bit, sc_relu, self.q_bit, relu, want16)
@@ -116,34 +128,59 @@ class _LazyCat:
     """torch.cat(members, 1) that has not run yet.  The reference leaves Concat in fp32
     (tools/reconstruction.py:219-238) and the consumer's Quantity(ib) quantises the result, so the exact
     int8 operand is ``clamp(rint(member * 2^ib))`` per member -- computed here from the members' most
-    exact integer payloads once the consumer (and so ib and its channel padding) is known."""
+    exact integer payloads once the consumer (and so ib and its channel padding) is known.
+
+    A member may be read through nearest-neighbour tables (an upsampled tensor, see _upsample); a lazy nearest view
+    is itself a one-member _LazyCat with tables, so a NewConv2d reads ``Up(x)`` as a one-source concatenation."""
 
     def __init__(self, members):
-        self.members = []                              # (QTensor, extra_relu), nested concatenations flattened
+        self.parts = list(members)                     # the tensors torch.cat received (fp32 evaluation)
+        self.members = []                              # (QTensor, extra_relu, tables or None), nested cats flattened
         for m in members:
             if m._lazy_cat is not None:
-                self.members += [(t, r or m.relu_pending) for t, r in m._lazy_cat.members]
+                self.members += [(t, r or m.relu_pending, mp) for t, r, mp in m._lazy_cat.members]
             else:
-                self.members.append((m, False))
+                self.members.append((m, False, None))
+        self.hw = tuple(members[0].shape[2:]) if members else None
         self.done = {}
 
+    @classmethod
+    def upsampled(cls, x, tables):
+        """The lazy view Up(x): x's members (or x itself) read through `tables` composed with their own."""
+        view = cls([])
+        if x._lazy_cat is not None:
+            view.members = [(t, r or x.relu_pending, _compose(mp, tables)) for t, r, mp in x._lazy_cat.members]
+        else:
+            view.members = [(x, False, tables)]
+        view.hw = (tables.map_h.numel(), tables.map_w.numel())
+        return view
+
+    def view_source(self):
+        """(QTensor, extra_relu, tables) when this is a single upsampled tensor, else None."""
+        return self.members[0] if len(self.members) == 1 and self.members[0][2] is not None else None
+
     def supported(self, q_bit):
+        if any(mp is not None for _, _, mp in self.members) and \
+                self.members[0][0].shape[0] * self.hw[0] * self.hw[1] > NEAREST_MAX_PIXELS:
+            return False                               # beyond pq_concat_requant_nearest_s8's pixel limit
         return len(self.members) <= _native.CONCAT_MAX_SOURCES and all(
-            t.exact_bit() is not None and abs(q_bit - t.exact_bit()) <= 15 for t, _ in self.members)
+            t.exact_bit() is not None and abs(q_bit - t.exact_bit()) <= 15 for t, _, _ in self.members)
 
     def get(self, q_bit, c_pad, relu):
         key = (q_bit, c_pad, relu)
         if key not in self.done:
             srcs = []
-            for t, extra in self.members:
+            for t, extra, mp in self.members:
                 payload, bit, r = _operand(t)
-                srcs.append((payload, bit, r or extra or relu))
-            self.done[key] = _native.concat_requant_s8(srcs, q_bit, c_pad)
+                srcs.append((payload, bit, r or extra or relu, mp and (mp.map_h, mp.map_w)))
+            if any(mp is not None for _, _, _, mp in srcs):
+                self.done[key] = _native.concat_requant_nearest_s8(srcs, self.hw, q_bit, c_pad)
+            else:
+                self.done[key] = _native.concat_requant_s8([s[:3] for s in srcs], q_bit, c_pad)
         return self.done[key]
 
     def dequantize(self):
-        parts = [torch.relu(t.dequantize()) if extra else t.dequantize() for t, extra in self.members]
-        return torch.cat(parts, 1)
+        return torch.cat([t.dequantize() for t in self.parts], 1)
 
 
 class QTensor(torch.Tensor):
@@ -155,7 +192,7 @@ class QTensor(torch.Tensor):
                                                    requires_grad=False)
 
     def __init__(self, shape, device, q8=None, q8_bit=None, s16=None, s16_bit=None, relu_pending=False,
-                 nonneg=False, lazy=None, lazy_conv=None, lazy_cat=None):
+                 nonneg=False, lazy=None, lazy_conv=None, lazy_cat=None, upsample=None):
         self.channels = int(shape[1])                  # plain attribute: tensor.shape on a subclass costs a dispatch
         self._q8, self.q8_bit = q8, q8_bit             # int8 NHWC, value = q8 / 2^q8_bit (after pending relu)
         self._s16, self.s16_bit = s16, s16_bit         # int16 NHWC exact value (outputs of NewAdd)
@@ -164,10 +201,13 @@ class QTensor(torch.Tensor):
         self._lazy = lazy                              # _LazyAdd: payloads appear on first use
         self._lazy_conv = lazy_conv                    # _LazyConv: the int8 payload appears on first use
         self._lazy_cat = lazy_cat                      # _LazyCat: payload exists per (consumer bit, padding)
+        self._upsample = upsample                      # (input, args, kwargs) of the F.interpolate this view is
         self._q8_relu = None
 
     def exact_bit(self):
-        """Fractional bit of the most exact payload, without materialising anything."""
+        """Fractional bit of the most exact payload, without materialising anything (a nearest view: its source's)."""
+        if self._upsample is not None and self._lazy_cat.view_source() is not None:
+            return self._lazy_cat.view_source()[0].exact_bit()
         return self.s16_bit if self.s16_bit is not None else self.q8_bit
 
     def _materialize(self, kind):
@@ -216,6 +256,10 @@ class QTensor(torch.Tensor):
 
     def dequantize(self):
         """fp32 NCHW, exactly what the fp32-boundary model would hold here (cold path: plain torch ops)."""
+        if self._upsample is not None:
+            x, args, kwargs = self._upsample
+            v = F.interpolate(x.dequantize(), *args, **kwargs)
+            return torch.relu(v) if self.relu_pending else v
         if self._lazy_cat is not None:
             v = self._lazy_cat.dequantize()
             return torch.relu(v) if self.relu_pending else v
@@ -232,7 +276,7 @@ class QTensor(torch.Tensor):
             return self
         return QTensor(self.shape, self.device, q8=self._q8, q8_bit=self.q8_bit, s16=self._s16,
                        s16_bit=self.s16_bit, relu_pending=True, lazy=self._lazy, lazy_conv=self._lazy_conv,
-                       lazy_cat=self._lazy_cat)
+                       lazy_cat=self._lazy_cat, upsample=self._upsample)
 
     # ---- dispatch -------------------------------------------------------------------------
     @classmethod
@@ -252,6 +296,10 @@ class QTensor(torch.Tensor):
                 return out
         if func is F.max_pool2d and isinstance(args[0], QTensor):
             out = _maxpool(args[0], *args[1:], **kwargs)
+            if out is not None:
+                return out
+        if func is F.interpolate and args and isinstance(args[0], QTensor):
+            out = _upsample(args[0], args[1:], kwargs)
             if out is not None:
                 return out
         if func is F.avg_pool2d and isinstance(args[0], QTensor):
@@ -299,6 +347,84 @@ def _concat(tensors, dim=0, out=None):
         return None
     shape = (first.shape[0], sum(t.shape[1] for t in tensors), first.shape[2], first.shape[3])
     return QTensor(shape, first.device, lazy_cat=lazy, nonneg=all(t.nonneg for t in tensors))
+
+
+class _Tables:
+    """Nearest-neighbour index tables: output row p reads source row map_h[p], output column q source column map_w[q]
+    (int32 tensors on the payload's device)."""
+
+    def __init__(self, key, map_h, map_w):
+        self.key, self.map_h, self.map_w = key, map_h, map_w
+
+
+_TABLES = {}                                           # geometry key -> _Tables (filled by the first forward)
+NEAREST_MAX_PIXELS = 2 ** 31 - 1                       # 'nearest limit: N*P*Q <= 2^31 - 1' (include/pq_sm100.h)
+
+
+def nearest_add_fits(shape):
+    """Whether pq_add_requant_nearest takes an NCHW output of `shape` (its 'nearest limit:' lines: C % 16 == 0 and
+    N*P*Q <= 2^31 - 1).  A NewAdd with an upsampled operand outside them takes the fp32 path, as without the pipeline."""
+    N, C, P, Q = (int(v) for v in shape)
+    return C % 16 == 0 and N * P * Q <= NEAREST_MAX_PIXELS
+
+
+def nearest_request(ndim, size=None, scale_factor=None, mode="nearest", align_corners=None,
+                    recompute_scale_factor=None, antialias=False):
+    """The F.interpolate arguments that fix a nearest view's tables -- (size, scale_factor, recompute_scale_factor),
+    lists made tuples -- or None when the pipeline leaves the call to ATen: any mode but 'nearest' ('nearest-exact',
+    the linear modes, 'area'), antialias, align_corners (torch refuses it for 'nearest') and inputs that are not 4-D."""
+    if mode != "nearest" or antialias or align_corners is not None or ndim != 4:
+        return None
+    tup = lambda v: tuple(v) if isinstance(v, (list, tuple)) else v
+    return tup(size), tup(scale_factor), recompute_scale_factor
+
+
+def nearest_tables(hw, request, device):
+    """_Tables of F.interpolate(mode='nearest') for an input of height / width hw, taken from ATen's own rule: two
+    [1][1][H][W] float32 images holding each pixel's row and column index (exact in fp32) are interpolated with the
+    caller's arguments.  Cached per geometry, so a CUDA-graph capture allocates and launches nothing for them."""
+    key = (tuple(hw), request, str(device))
+    t = _TABLES.get(key)
+    if t is None:
+        H, W = hw
+        size, scale_factor, rsf = request
+        rows = torch.arange(H, dtype=torch.float32, device=device).view(1, 1, H, 1).expand(1, 1, H, W).contiguous()
+        cols = torch.arange(W, dtype=torch.float32, device=device).view(1, 1, 1, W).expand(1, 1, H, W).contiguous()
+        kw = dict(size=size, scale_factor=scale_factor, mode="nearest", recompute_scale_factor=rsf)
+        r, c = F.interpolate(rows, **kw), F.interpolate(cols, **kw)
+        t = _Tables(key, r[0, 0, :, 0].to(torch.int32).contiguous(), c[0, 0, 0, :].to(torch.int32).contiguous())
+        _TABLES[key] = t
+    return t
+
+
+def _compose(inner, outer):
+    """Tables of Up_outer(Up_inner(x)): map_outer read through map_inner (inner None: outer alone)."""
+    if inner is None:
+        return outer
+    key = ("compose", inner.key, outer.key)
+    t = _TABLES.get(key)
+    if t is None:
+        t = _Tables(key, inner.map_h[outer.map_h.long()].contiguous(), inner.map_w[outer.map_w.long()].contiguous())
+        _TABLES[key] = t
+    return t
+
+
+def _upsample(x, args, kwargs):
+    """F.interpolate(x, mode='nearest') on a 4-D QTensor: a lazy view (x's payload read through index tables by its
+    consumer), or None to leave the call to ATen on the de-quantised tensor."""
+    try:
+        request = nearest_request(x.dim(), *args, **kwargs)
+    except TypeError:
+        return None                                     # not a valid call: let F.interpolate raise its own error
+    if request is None or (x._lazy_cat is None and x.exact_bit() is None):
+        return None
+    try:
+        tables = nearest_tables(x.shape[2:], request, x.device)
+    except (RuntimeError, ValueError, TypeError):
+        return None                                     # arguments ATen refuses: it raises on the fallback path
+    lazy = _LazyCat.upsampled(x, tables)
+    shape = (x.shape[0], x.shape[1]) + lazy.hw
+    return QTensor(shape, x.device, lazy_cat=lazy, nonneg=x.nonneg, upsample=(x, tuple(args), dict(kwargs)))
 
 
 def _maxpool(x, kernel_size, stride=None, padding=0, dilation=1, ceil_mode=False, return_indices=False):
@@ -370,6 +496,9 @@ def add_forward(mod, x, y):
     """NewAdd.forward in pipeline mode; returns None when the operands are not both quantised."""
     if not (isinstance(x, QTensor) and isinstance(y, QTensor)) or x.shape != y.shape:
         return None
+    views = sum(t._upsample is not None for t in (x, y))
+    if views == 2 or (views == 1 and not nearest_add_fits(x.shape)):
+        return None                                     # two nearest views, or outside the kernel's limits: fp32 path
     q_bit = getattr(mod, "output_bit", None)
     abit, bbit = x.exact_bit(), y.exact_bit()
     if q_bit is None or abit is None or bbit is None:
@@ -399,7 +528,9 @@ class GraphedForward:
     collapse into one graph launch.  The arithmetic is the captured kernels', so outputs are unchanged.
 
         fwd = GraphedForward(model, example_batch);  y = fwd(batch)      # y is overwritten by the next call
-    """
+
+    An output that is still a lazy QTensor (a model ending in an upsample or a convolution) is de-quantised inside the
+    capture, so every replay recomputes it."""
 
     def __init__(self, model, example, warmup=2):
         if not example.is_cuda:
@@ -411,13 +542,13 @@ class GraphedForward:
             side.wait_stream(torch.cuda.current_stream(example.device))
             with torch.cuda.stream(side):
                 for _ in range(warmup):                # lazy one-time setup must not land in the capture
-                    model(self.static_in)
+                    _plain_tree(model(self.static_in))
             torch.cuda.current_stream(example.device).wait_stream(side)
             torch.cuda.synchronize(example.device)
             self.graph = torch.cuda.CUDAGraph()
             l0 = _native.LAUNCHES["total"]
             with torch.cuda.graph(self.graph):
-                self.static_out = model(self.static_in)
+                self.static_out = _plain_tree(model(self.static_in))
             self.launches = _native.LAUNCHES["total"] - l0     # kernels of this library inside the graph
 
     def __call__(self, x):

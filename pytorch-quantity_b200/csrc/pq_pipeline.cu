@@ -340,6 +340,65 @@ add_requant_kernel(const AddParams p, size_t n)
     }
 }
 
+// pq_add_requant_nearest: the same sum with operand b read through nearest-neighbour index tables, so an upsampled
+// operand is never written at full resolution.  a and the outputs are [N][P][Q][C]; b is [N][Hb][Wb][C], read at
+// (n, map_h[p], map_w[q]) for output pixel (n, p, q).
+struct AddNearestParams {
+    AddParams add;
+    const int *map_h, *map_w;      // [P], [Q]: source row / column of each output row / column
+    int P, Q, Hb, Wb;
+    unsigned int groups;           // C / 16
+};
+
+// One thread per (pixel, 16-channel group), channel group fastest, so a warp reads and writes contiguous runs.  The
+// pixel -> (n, p, q) -> source pixel arithmetic runs once per 16 elements (two 32-bit divisions: N*P*Q < 2^31), and
+// a thread's (pixel, group) advances by a constant per grid-stride trip without a division.
+template <bool A16, bool B16, bool RELU_IN, bool QDOWN>
+__global__ void __launch_bounds__(kPipeThreads)
+add_requant_kernel(const AddNearestParams np, size_t total)
+{
+    const AddParams &p = np.add;
+    const unsigned int G = np.groups;
+    const size_t stride = (size_t)gridDim.x * kPipeThreads;
+    size_t t = (size_t)blockIdx.x * kPipeThreads + threadIdx.x;
+    if (t >= total) return;
+    unsigned int pix = (unsigned int)(t / G), cg = (unsigned int)(t - (size_t)pix * G);
+    const unsigned int dpix = (unsigned int)(stride / G), dcg = (unsigned int)(stride - (size_t)dpix * G);
+    const int a_mul = 1 << p.a_shift, b_mul = 1 << p.b_shift;
+    const int a_lo = p.a_relu ? 0 : -32768, b_lo = p.b_relu ? 0 : -32768;
+    const int d = QDOWN ? -p.q_shift : 0;
+    const int rc = QDOWN ? (1 << (d - 1)) - 1 : 0;
+    for (; t < total; t += stride) {
+        const unsigned int row = pix / (unsigned int)np.Q, q = pix - row * (unsigned int)np.Q;
+        const unsigned int n = row / (unsigned int)np.P, pp = row - n * (unsigned int)np.P;
+        const size_t src = ((size_t)n * np.Hb + __ldg(np.map_h + pp)) * np.Wb + __ldg(np.map_w + q);
+        int av[16], bv[16], num[16], qv[16];
+        add_load16<A16>(p.a, t, av);
+        add_load16<B16>(p.b, src * G + cg, bv);
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+            int x = av[j], y = bv[j];
+            if (RELU_IN) { x = max(x, a_lo); y = max(y, b_lo); }
+            num[j] = max(p.lo, min(p.hi, x * a_mul + y * b_mul));
+            if (QDOWN) qv[j] = (num[j] + rc + ((num[j] >> d) & 1)) >> d;
+            else qv[j] = max(-128, min(127, num[j])) << p.q_shift;
+        }
+        if (p.out16) {
+            uint32_t o16[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) o16[j] = __byte_perm((uint32_t)num[2 * j], (uint32_t)num[2 * j + 1], 0x5410);
+            uint4 *d0 = reinterpret_cast<uint4 *>(p.out16) + 2 * t;
+            d0[0] = make_uint4(o16[0], o16[1], o16[2], o16[3]);
+            d0[1] = make_uint4(o16[4], o16[5], o16[6], o16[7]);
+        }
+        if (p.out8)
+            reinterpret_cast<uint4 *>(p.out8)[t] =
+                make_uint4(pack4_sat_s8(qv[0], qv[1], qv[2], qv[3]), pack4_sat_s8(qv[4], qv[5], qv[6], qv[7]),
+                           pack4_sat_s8(qv[8], qv[9], qv[10], qv[11]), pack4_sat_s8(qv[12], qv[13], qv[14], qv[15]));
+        pix += dpix; cg += dcg;
+        if (cg >= G) { cg -= G; ++pix; }
+    }
+}
 
 // Concat + the consumer's input quantiser on quantised operands (pq_concat_requant_s8).  HBM-bound:
 // 1 (int8) or 2 (int16) bytes read + 1 byte written per element.
@@ -399,6 +458,79 @@ concat_requant_scalar_kernel(const ConcatParams p, size_t pixels, int8_t *__rest
         out[t] = (int8_t)q;
     }
 }
+
+// pq_concat_requant_nearest_s8: the output is [N][P][Q][c_out_pad]; source i is [N][H_i][W_i][channels_i], read at
+// (n, map_h_i[p], map_w_i[q]), or at (n, p, q) when its tables are NULL (then H_i == P and W_i == Q).
+struct ConcatNearestParams {
+    ConcatParams c;
+    const int *map_h[PQ_CONCAT_MAX_SOURCES], *map_w[PQ_CONCAT_MAX_SOURCES];
+    int H[PQ_CONCAT_MAX_SOURCES], W[PQ_CONCAT_MAX_SOURCES];
+    int P, Q;
+};
+
+// source pixel of output pixel pix (< 2^31) in member i
+__device__ __forceinline__ size_t nearest_src(const ConcatNearestParams &p, int i, unsigned int pix)
+{
+    if (p.map_h[i] == nullptr) return pix;
+    const unsigned int row = pix / (unsigned int)p.Q, q = pix - row * (unsigned int)p.Q;
+    const unsigned int n = row / (unsigned int)p.P, pp = row - n * (unsigned int)p.P;
+    return ((size_t)n * p.H[i] + __ldg(p.map_h[i] + pp)) * p.W[i] + __ldg(p.map_w[i] + q);
+}
+
+// one thread per (pixel, 16 output channels), as the same-resolution kernel; the source pixel is found once per thread
+__global__ void __launch_bounds__(kPipeThreads)
+concat_requant_vec_kernel(const ConcatNearestParams np, size_t pixels, int8_t *__restrict__ out)
+{
+    const ConcatParams &p = np.c;
+    const unsigned int groups = (unsigned int)p.c_out_pad >> 4;
+    const size_t total = pixels * groups;
+    for (size_t t = (size_t)blockIdx.x * kPipeThreads + threadIdx.x; t < total; t += (size_t)gridDim.x * kPipeThreads) {
+        const unsigned int pix = (unsigned int)(t / groups);
+        const int c0 = (int)(t - (size_t)pix * groups) << 4;
+        uint4 o = make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll 1
+        for (int i = 0; i < p.k; ++i) {
+            const int c = c0 - p.off[i];
+            if (c < 0 || c >= p.channels[i]) continue;
+            const size_t v = (nearest_src(np, i, pix) * (size_t)p.channels[i] + c) >> 4;
+            int x[16];
+            if (p.is16[i]) add_load16<true>(p.ptr[i], v, x); else add_load16<false>(p.ptr[i], v, x);
+            const int lo = p.relu[i] ? 0 : -32768, sh = p.sh[i];
+            int q[16];
+#pragma unroll
+            for (int j = 0; j < 16; ++j) q[j] = requant_rne(max(x[j], lo), sh);
+            o = make_uint4(pack4_sat_s8(q[0], q[1], q[2], q[3]), pack4_sat_s8(q[4], q[5], q[6], q[7]),
+                           pack4_sat_s8(q[8], q[9], q[10], q[11]), pack4_sat_s8(q[12], q[13], q[14], q[15]));
+            break;
+        }
+        reinterpret_cast<uint4 *>(out)[t] = o;
+    }
+}
+
+// any channel counts: one warp per output pixel, lanes across its channels, so the source pixels are found once per
+// lane and pixel and the stores stay contiguous
+__global__ void __launch_bounds__(kPipeThreads)
+concat_requant_scalar_kernel(const ConcatNearestParams np, size_t pixels, int8_t *__restrict__ out)
+{
+    const ConcatParams &p = np.c;
+    const unsigned int lane = threadIdx.x & 31u;
+    const size_t warps = (size_t)gridDim.x * (kPipeThreads / 32);
+    for (size_t w = (size_t)blockIdx.x * (kPipeThreads / 32) + (threadIdx.x >> 5); w < pixels; w += warps) {
+        const unsigned int pix = (unsigned int)w;
+        int8_t *o = out + w * (unsigned int)p.c_out_pad;
+        for (int i = 0; i < p.k; ++i) {
+            const size_t base = nearest_src(np, i, pix) * (size_t)p.channels[i];
+            for (int c = (int)lane; c < p.channels[i]; c += 32) {
+                int x = add_load(p.ptr[i], p.is16[i], base + c);
+                if (p.relu[i]) x = max(x, 0);
+                o[p.off[i] + c] = (int8_t)requant_rne(x, p.sh[i]);
+            }
+        }
+        const int used = p.k > 0 ? p.off[p.k - 1] + p.channels[p.k - 1] : 0;
+        for (int c = used + (int)lane; c < p.c_out_pad; c += 32) o[c] = 0;
+    }
+}
+
 __global__ void bias_fold_kernel(const int32_t *__restrict__ b, int n, int rs, int32_t *__restrict__ out)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -534,6 +666,85 @@ extern "C" int pq_concat_requant_s8(const pq_concat_src *srcs_host, int k, size_
     else
         pq::concat_requant_scalar_kernel<<<pipe_grid(pixels * (size_t)c_out_pad), pq::kPipeThreads, 0, st>>>(
             p, pixels, out);
+    return (int)cudaGetLastError();
+}
+
+extern "C" int pq_add_requant_nearest(const void *a, int a_is16, int a_bit, int a_relu, const void *b, int b_is16,
+                                      int b_bit, int b_relu, int N, int P, int Q, int C, int Hb, int Wb,
+                                      const int32_t *map_h, const int32_t *map_w, int flags, int16_t *out16,
+                                      int8_t *out8, int q_bit, pq_stream_t stream)
+{
+    if (N <= 0 || P <= 0 || Q <= 0 || C <= 0 || Hb <= 0 || Wb <= 0) return PQ_EINVAL;
+    if (!a || !b || !map_h || !map_w || (!out16 && !out8)) return PQ_EINVAL;
+    if ((C & 15) || (long long)N * P * Q > 0x7fffffffLL) return PQ_EUNSUPPORTED;
+    if (!al16(a) || !al16(b) || (out16 && !al16(out16)) || (out8 && !al16(out8))) return PQ_EALIGN;
+    const int o_bit = a_bit > b_bit ? a_bit : b_bit;
+    const int span = o_bit - (a_bit < b_bit ? a_bit : b_bit);
+    if (span > 7 || o_bit < 0 || o_bit > 7 || q_bit - o_bit > 15 || o_bit - q_bit > 15) return PQ_EUNSUPPORTED;
+    pq::AddNearestParams np;
+    pq::AddParams &p = np.add;
+    p.a = a; p.b = b; p.a_is16 = a_is16; p.b_is16 = b_is16; p.a_relu = a_relu; p.b_relu = b_relu;
+    p.a_shift = o_bit - a_bit; p.b_shift = o_bit - b_bit;
+    p.out_relu = flags & PQ_FLAG_RELU;
+    p.lo = p.out_relu ? 0 : -128 * (1 << o_bit); p.hi = 127 * (1 << o_bit);
+    p.q_shift = q_bit - o_bit; p.out16 = out16; p.out8 = out8;
+    np.map_h = map_h; np.map_w = map_w; np.P = P; np.Q = Q; np.Hb = Hb; np.Wb = Wb;
+    np.groups = (unsigned int)(C >> 4);
+    const size_t total = (size_t)N * P * Q * np.groups;
+    const unsigned int grid = pipe_grid(total);
+    cudaStream_t s = (cudaStream_t)stream;
+    const int variant = (a_is16 ? 8 : 0) | (b_is16 ? 4 : 0) | ((a_relu || b_relu) ? 2 : 0) | (p.q_shift < 0 ? 1 : 0);
+#define PQ_ADD_CASE(V, A, B, R, Q) \
+    case V: pq::add_requant_kernel<A, B, R, Q><<<grid, pq::kPipeThreads, 0, s>>>(np, total); break;
+    switch (variant) {
+        PQ_ADD_CASE(0, false, false, false, false) PQ_ADD_CASE(1, false, false, false, true)
+        PQ_ADD_CASE(2, false, false, true, false) PQ_ADD_CASE(3, false, false, true, true)
+        PQ_ADD_CASE(4, false, true, false, false) PQ_ADD_CASE(5, false, true, false, true)
+        PQ_ADD_CASE(6, false, true, true, false) PQ_ADD_CASE(7, false, true, true, true)
+        PQ_ADD_CASE(8, true, false, false, false) PQ_ADD_CASE(9, true, false, false, true)
+        PQ_ADD_CASE(10, true, false, true, false) PQ_ADD_CASE(11, true, false, true, true)
+        PQ_ADD_CASE(12, true, true, false, false) PQ_ADD_CASE(13, true, true, false, true)
+        PQ_ADD_CASE(14, true, true, true, false) PQ_ADD_CASE(15, true, true, true, true)
+    }
+#undef PQ_ADD_CASE
+    return (int)cudaGetLastError();
+}
+
+extern "C" int pq_concat_requant_nearest_s8(const pq_concat_nearest_src *srcs_host, int k, int N, int P, int Q,
+                                            int q_bit, int c_out_pad, int8_t *out, pq_stream_t stream)
+{
+    if (k < 0 || c_out_pad < 0 || N < 0 || P < 0 || Q < 0 || (k > 0 && !srcs_host)) return PQ_EINVAL;
+    if (k > PQ_CONCAT_MAX_SOURCES) return PQ_ETOOMANY;
+    if ((long long)N * P * Q > 0x7fffffffLL) return PQ_EUNSUPPORTED;
+    const size_t pixels = (size_t)N * P * Q;
+    if (pixels == 0 || c_out_pad == 0) return PQ_OK;
+    if (!out) return PQ_EINVAL;
+    pq::ConcatNearestParams np;
+    pq::ConcatParams &p = np.c;
+    p.k = k; p.c_out_pad = c_out_pad;
+    np.P = P; np.Q = Q;
+    int off = 0;
+    bool vec = (c_out_pad & 15) == 0 && al16(out);
+    for (int i = 0; i < k; ++i) {
+        const pq_concat_nearest_src &s = srcs_host[i];
+        if (s.channels < 0 || (s.channels > 0 && !s.ptr)) return PQ_EINVAL;
+        if (!s.map_h != !s.map_w) return PQ_EINVAL;
+        if (s.map_h ? (s.H <= 0 || s.W <= 0) : (s.H != P || s.W != Q)) return PQ_EINVAL;
+        if (q_bit - s.bit > 15 || s.bit - q_bit > 15) return PQ_EUNSUPPORTED;
+        if (s.is16 && (((unsigned long long)s.ptr) & 1ull)) return PQ_EALIGN;
+        p.ptr[i] = s.ptr; p.is16[i] = s.is16 ? 1 : 0; p.channels[i] = s.channels; p.off[i] = off;
+        p.sh[i] = q_bit - s.bit; p.relu[i] = s.relu ? 1 : 0;
+        np.map_h[i] = s.map_h; np.map_w[i] = s.map_w; np.H[i] = s.H; np.W[i] = s.W;
+        vec = vec && (s.channels & 15) == 0 && al16(s.ptr);
+        off += s.channels;
+    }
+    if (off > c_out_pad) return PQ_EINVAL;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (vec)
+        pq::concat_requant_vec_kernel<<<pipe_grid(pixels * (size_t)(c_out_pad >> 4)), pq::kPipeThreads, 0, st>>>(
+            np, pixels, out);
+    else
+        pq::concat_requant_scalar_kernel<<<pipe_grid(pixels * 32), pq::kPipeThreads, 0, st>>>(np, pixels, out);
     return (int)cudaGetLastError();
 }
 

@@ -22,6 +22,7 @@ MODELS = {
                                            fromlist=["resnext50_32x4d_fabu"]).resnext50_32x4d_fabu(), (3, 224, 224)),
     "mobilenetv2": (lambda: __import__("model.mobilenet.mobilenetv2_fabu",
                                        fromlist=["mobilenetv2_fabu"]).mobilenetv2_fabu(), (3, 224, 224)),
+    "fpn_r50": (lambda: __import__("model.fpn.fpn_fabu", fromlist=["fpn_r50_fabu"]).fpn_r50_fabu(), (3, 512, 512)),
 }
 
 
