@@ -36,7 +36,7 @@ typedef void *pq_stream_t; /* cudaStream_t */
 
 /* pq_version() of a library built from this header.  Bump it whenever an entry point changes its parameters: ctypes
  * binds by name only, so a stale build would otherwise be called with the wrong arguments without any error. */
-#define PQ_VERSION 205
+#define PQ_VERSION 206
 
 #define PQ_OK 0
 #define PQ_EINVAL (-1)       /* null pointer, negative size, bad enum */
@@ -310,6 +310,35 @@ int pq_conv2d_smallc_s8(const int8_t *xp, const int8_t *w_krs8, const int32_t *b
  * View -> NewLinear).  C % 8 == 0. */
 int pq_avgpool_global_nhwc_f32(const void *x, int is16, int bit, int relu, int N, int HW, int C, float *out,
                                pq_stream_t stream);
+
+/* Windowed average pool (nn.AvgPool2d / F.avg_pool2d; listed in the tracer's tools/configs.yml:21) followed by the
+ * consumer's input quantiser, on a quantised payload: x is int8 or int16 NHWC [N][H][W][C] at fractional bit `bit`;
+ * out is the consumer's int8 NHWC operand [N][P][Q][c_out_pad] at q_bit, channels C .. c_out_pad-1 zero-filled:
+ *   out = Quantity(q_bit)(F.avg_pool2d(DeQuantity(x), ...)) bit for bit
+ *       = clamp(rint(fl(fl(S) * 2^-bit / (float)d) * 2^q_bit), -128, 127),   S the integer window sum,
+ * where d is divisor_override, or with count_include_pad the window area before clipping to the image (its end
+ * clipped to H + pad_h, W + pad_w only), else the clipped window's area -- ATen's rule; P and Q follow ATen's
+ * ceil_mode rule (the last window starts inside the image or the left padding).  relu & 1 applies max(., 0) on load
+ * (a pending ReLU before the pool), relu & 2 to the pooled value (a ReLU after it; it commutes with the quantiser).
+ * x and out 16-byte aligned (else PQ_EALIGN).  A kernel size or stride <= 0, a negative pad, an empty output,
+ * c_out_pad < C or relu & ~3 is PQ_EINVAL.  2*pad > k, which torch refuses too, is the one such argument reported as
+ * PQ_EUNSUPPORTED instead, as pq_maxpool_nhwc_s8 reports it.  Any H, W, Q and c_out_pad inside the limits below are
+ * taken: a row of the output may hold more than 2^31 bytes.  Outside these limits (per dimension, k with pad) the call returns
+ * PQ_EUNSUPPORTED and writes nothing:
+ *   avgpool limit: kh*kw*(32768 | 128) < 2^24;  (int16 | int8 payload: the fp32 window sum is exact)
+ *   avgpool limit: 2*pad <= k;  (torch refuses more)
+ *   avgpool limit: C % 8 == 0;
+ *   avgpool limit: c_out_pad % 16 == 0;
+ *   avgpool limit: N*P*Q <= 2^31 - 1;
+ *   avgpool limit: |bit| <= 31;
+ *   avgpool limit: |q_bit| <= 31; */
+typedef struct pq_pool_desc {
+    int kh, kw, sh, sw, ph, pw;
+    int ceil_mode, count_include_pad;
+    int divisor_override;    /* 0: none */
+} pq_pool_desc;
+int pq_avgpool_requant_s8(const void *x, int is16, int bit, int relu, int N, int H, int W, int C,
+                          const pq_pool_desc *desc, int q_bit, int c_out_pad, int8_t *out, pq_stream_t stream);
 
 /* y = max(x, 0) on int8 (nn.ReLU on a quantised tensor: relu commutes with the input quantiser). */
 int pq_relu_s8(const int8_t *x, int8_t *y, size_t n, pq_stream_t stream);

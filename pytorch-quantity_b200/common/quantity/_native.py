@@ -21,7 +21,7 @@ KL_CANDIDATES = HIST_BINS - KL_TARGET_BIN
 MAX_SEGMENTS = 256
 KL_MAX_ROWS = 65535          # tensors per pq_kl_search_n_f64 call (one grid row per tensor)
 MAXPOOL_PLANE_BYTES = 227 * 1024 - 1024   # PQ_MAXPOOL_PLANE_BYTES: largest plane pq_conv_epilogue_maxpool_f32 takes
-PQ_VERSION = 205             # the header's PQ_VERSION: the entry points below match a library built from it
+PQ_VERSION = 206             # the header's PQ_VERSION: the entry points below match a library built from it
 
 # every symbol include/pq_sm100.h declares: (restype, argtypes)
 _vp, _i, _sz, _f = ctypes.c_void_p, ctypes.c_int, ctypes.c_size_t, ctypes.c_float
@@ -61,6 +61,7 @@ SYMBOLS = {
     "pq_bias_fold_s32": (_i, [_vp, _i, _i, _vp, _vp]),
     "pq_add_requant_nearest": (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i] + [_i] * 6 + [_vp, _vp, _i, _vp, _vp, _i, _vp]),
     "pq_concat_requant_nearest_s8": (_i, [_vp, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "pq_avgpool_requant_s8": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp]),
 }
 FLAG_RELU = 1
 FLAG_BIAS_FOLDED = 2
@@ -94,7 +95,15 @@ class ConcatNearestSrc(ctypes.Structure):
                 ("map_w", ctypes.c_void_p)]
 
 
+class PoolDesc(ctypes.Structure):
+    """struct pq_pool_desc"""
+    _fields_ = [(n, ctypes.c_int) for n in
+                ("kh", "kw", "sh", "sw", "ph", "pw", "ceil_mode", "count_include_pad", "divisor_override")]
+
+
 CONCAT_MAX_SOURCES = 8
+AVGPOOL_MAX_BIT = 31         # 'avgpool limit: |bit| <= 31' and '|q_bit| <= 31' (include/pq_sm100.h)
+MAX_PIXELS = 2 ** 31 - 1     # 'avgpool limit: N*P*Q <= 2^31 - 1'
 
 _lib = None
 
@@ -647,6 +656,46 @@ def avgpool_global_nhwc(x, bit, relu=False):
         check(lib().pq_avgpool_global_nhwc_f32(x.data_ptr(), 1 if is16 else 0, int(bit), 1 if relu else 0, N, H * W, C,
                                                y.data_ptr(), _stream(x)), "pq_avgpool_global_nhwc_f32")
     return y
+
+
+_POOL_OUT = {}                                         # ((H, W), window) -> (P, Q)
+
+
+def avgpool_out_size(hw, window):
+    """(P, Q) of F.avg_pool2d on an H x W plane with `window` = (kh, kw, sh, sw, ph, pw, ceil_mode, count_include_pad,
+    divisor_override or 0), taken from ATen itself (a meta tensor, so nothing runs) and cached per geometry.  Raises
+    ATen's own error for arguments it refuses."""
+    key = (tuple(int(v) for v in hw), tuple(window))
+    out = _POOL_OUT.get(key)
+    if out is None:
+        kh, kw, sh, sw, ph, pw, ceil_mode, count_include_pad, divisor = window
+        y = torch.nn.functional.avg_pool2d(torch.empty((1, 1) + key[0], device="meta"), (kh, kw), (sh, sw), (ph, pw),
+                                           bool(ceil_mode), bool(count_include_pad), divisor or None)
+        out = _POOL_OUT[key] = (int(y.shape[2]), int(y.shape[3]))
+    return out
+
+
+def avgpool_requant_s8(x, bit, relu, window, q_bit, c_out_pad, out_relu=False):
+    """int8 / int16 NHWC payload [N][H][W][C] at fractional bit `bit` -> int8 NHWC [N][P][Q][c_out_pad] =
+    Quantity(q_bit)(F.avg_pool2d(de-quantised x, window)), channels C.. zero-filled (pq_avgpool_requant_s8).  `window`
+    as avgpool_out_size takes it; relu applies a pending ReLU on load, out_relu a ReLU after the pool.  None when the
+    exactness, channel, pixel or bit limits of the entry point do not hold."""
+    require_cuda(x, "avgpool_requant_s8")
+    N, H, W, C = x.shape
+    is16 = x.dtype == torch.int16
+    kh, kw = window[0], window[1]
+    if (C % 8 or c_out_pad % 16 or c_out_pad < C or kh * kw * (32768 if is16 else 128) >= (1 << 24)
+            or max(abs(int(bit)), abs(int(q_bit))) > AVGPOOL_MAX_BIT or not x.is_contiguous()):
+        return None
+    P, Q = avgpool_out_size((H, W), window)
+    if N * P * Q > MAX_PIXELS:
+        return None
+    out = torch.empty((N, P, Q, c_out_pad), dtype=torch.int8, device=x.device)
+    with _Timed("avgpool_requant", 1, x.numel() * x.element_size() + out.numel(), x.device):
+        check(lib().pq_avgpool_requant_s8(x.data_ptr(), 1 if is16 else 0, int(bit), (1 if relu else 0) |
+                                          (2 if out_relu else 0), N, H, W, C, ctypes.byref(PoolDesc(*window)),
+                                          int(q_bit), c_out_pad, out.data_ptr(), _stream(x)), "pq_avgpool_requant_s8")
+    return out
 
 
 def add_requant(a, a_bit, a_relu, b, b_bit, b_relu, q_bit, want16=True, want8=True, out_relu=False):

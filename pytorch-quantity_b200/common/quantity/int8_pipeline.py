@@ -18,7 +18,13 @@ layers hand each other int8 NHWC payloads wrapped in a lazy ``QTensor``:
                                                     its consumer reads the source through row / column index tables
                                                     (a Concat or NewConv2d: pq_concat_requant_nearest_s8; a NewAdd:
                                                     pq_add_requant_nearest)
-    anything else (AvgPool2d, user code)            the QTensor de-quantises itself to fp32 NCHW first
+    F.avg_pool2d(QTensor) over the whole plane      fp32 [N][C][1][1] straight from the most exact payload
+                                                    (pq_avgpool_global_nhwc_f32; ResNet's pool before the classifier)
+    F.avg_pool2d(QTensor), any other window         lazy pooled view (nn.AvgPool2d): a NewConv2d reading it gets its
+                                                    int8 operand from pq_avgpool_requant_s8, which pools the most exact
+                                                    payload (a NewAdd's int16 sum) and applies ITS input quantiser;
+                                                    every other consumer gets ATen's pool of the de-quantised source
+    anything else (user code)                       the QTensor de-quantises itself to fp32 NCHW first
 
 so the final output is bit-identical to the fp32-boundary model while HBM traffic drops ~4x.
 ``enable_int8_pipeline(model)`` turns it on for a model built by ``Reconstruction.ReconModel``.
@@ -183,6 +189,35 @@ class _LazyCat:
         return torch.cat([t.dequantize() for t in self.parts], 1)
 
 
+class _LazyPool:
+    """F.avg_pool2d(src, *args, **kwargs) that has not run yet.  The fp32-boundary model pools the de-quantised tensor
+    and the consumer's Quantity(ib) quantises the result, so the exact int8 operand depends on the consumer: it is
+    computed from src's most exact payload (a NewAdd's int16 sum, never its int8 requantisation) once the consumer, and
+    so ib, its channel padding and any ReLU in between, is known.  `window` is the kernel's form of the arguments."""
+
+    def __init__(self, src, window, args, kwargs):
+        self.src, self.window, self.args, self.kwargs = src, window, args, kwargs
+        self.done = {}
+
+    def supported(self, q_bit, c_pad):
+        """Whether the consumer's operand (input bit q_bit, c_pad channels) is inside pq_avgpool_requant_s8's limits.
+        Decided before the source's payload is materialised: every pipeline payload holds exactly the tensor's
+        (logical) channel count, so self.src.channels is the payload's.  The binding checks the payload itself again
+        for its direct callers."""
+        return abs(q_bit) <= _native.AVGPOOL_MAX_BIT and c_pad % 16 == 0 and c_pad >= self.src.channels
+
+    def get(self, q_bit, c_pad, relu):
+        key = (q_bit, c_pad, relu)
+        if key not in self.done:
+            payload, bit, src_relu = _operand(self.src)
+            self.done[key] = _native.avgpool_requant_s8(payload, bit, src_relu, self.window, q_bit, c_pad,
+                                                        out_relu=relu)
+        return self.done[key]
+
+    def dequantize(self):
+        return F.avg_pool2d(self.src.dequantize(), *self.args, **self.kwargs)
+
+
 class QTensor(torch.Tensor):
     """A float32 NCHW tensor that exists only as quantised payloads until somebody needs the floats."""
 
@@ -192,7 +227,7 @@ class QTensor(torch.Tensor):
                                                    requires_grad=False)
 
     def __init__(self, shape, device, q8=None, q8_bit=None, s16=None, s16_bit=None, relu_pending=False,
-                 nonneg=False, lazy=None, lazy_conv=None, lazy_cat=None, upsample=None):
+                 nonneg=False, lazy=None, lazy_conv=None, lazy_cat=None, upsample=None, lazy_pool=None):
         self.channels = int(shape[1])                  # plain attribute: tensor.shape on a subclass costs a dispatch
         self._q8, self.q8_bit = q8, q8_bit             # int8 NHWC, value = q8 / 2^q8_bit (after pending relu)
         self._s16, self.s16_bit = s16, s16_bit         # int16 NHWC exact value (outputs of NewAdd)
@@ -202,6 +237,7 @@ class QTensor(torch.Tensor):
         self._lazy_conv = lazy_conv                    # _LazyConv: the int8 payload appears on first use
         self._lazy_cat = lazy_cat                      # _LazyCat: payload exists per (consumer bit, padding)
         self._upsample = upsample                      # (input, args, kwargs) of the F.interpolate this view is
+        self._lazy_pool = lazy_pool                    # _LazyPool: payload exists per (consumer bit, padding, ReLU)
         self._q8_relu = None
 
     def exact_bit(self):
@@ -263,6 +299,9 @@ class QTensor(torch.Tensor):
         if self._lazy_cat is not None:
             v = self._lazy_cat.dequantize()
             return torch.relu(v) if self.relu_pending else v
+        if self._lazy_pool is not None:
+            v = self._lazy_pool.dequantize()
+            return torch.relu(v) if self.relu_pending else v
         if self.s16_bit is not None:
             v = self.s16.to(torch.float32) * (2.0 ** -self.s16_bit)
         else:
@@ -276,7 +315,7 @@ class QTensor(torch.Tensor):
             return self
         return QTensor(self.shape, self.device, q8=self._q8, q8_bit=self.q8_bit, s16=self._s16,
                        s16_bit=self.s16_bit, relu_pending=True, lazy=self._lazy, lazy_conv=self._lazy_conv,
-                       lazy_cat=self._lazy_cat, upsample=self._upsample)
+                       lazy_cat=self._lazy_cat, upsample=self._upsample, lazy_pool=self._lazy_pool)
 
     # ---- dispatch -------------------------------------------------------------------------
     @classmethod
@@ -442,7 +481,68 @@ def _maxpool(x, kernel_size, stride=None, padding=0, dilation=1, ceil_mode=False
     return QTensor((N, x.shape[1], P, Q), x.device, q8=y, q8_bit=x.q8_bit, nonneg=x.nonneg or relu)
 
 
-def _avgpool(x, kernel_size, stride=None, padding=0, ceil_mode=False, count_include_pad=True, divisor_override=None):
+def pool_window(ndim, kernel_size, stride=None, padding=0, ceil_mode=False, count_include_pad=True,
+                divisor_override=None):
+    """F.avg_pool2d's arguments as pq_avgpool_requant_s8's window (kh, kw, sh, sw, ph, pw, ceil_mode,
+    count_include_pad, divisor_override or 0), or None when the pipeline leaves the call to ATen: inputs that are not
+    4-D, and arguments that are not integers or sequences of one or two of them, or a divisor 0 or outside int32 (ATen
+    raises or truncates).  Values torch refuses pass here; avgpool_out_size raises for them."""
+    def two(v):
+        v = (v, v) if isinstance(v, int) else tuple(v)
+        v = v * 2 if len(v) == 1 else v
+        if len(v) != 2 or not all(isinstance(e, int) and not isinstance(e, bool) for e in v):
+            raise TypeError
+        return v
+    if ndim != 4:
+        return None
+    try:
+        k, p = two(kernel_size), two(padding)
+        s = two(stride) if stride is not None and (isinstance(stride, int) or len(stride)) else k
+    except TypeError:
+        return None
+    if divisor_override is not None and (not isinstance(divisor_override, int) or divisor_override == 0
+                                         or not -2 ** 31 <= divisor_override < 2 ** 31):
+        return None
+    return k + s + p + (int(bool(ceil_mode)), int(bool(count_include_pad)), divisor_override or 0)
+
+
+def _avgpool(x, *args, **kwargs):
+    """F.avg_pool2d on a QTensor: over the whole plane the fp32 result straight from the payload (_avgpool_global),
+    any other window a lazy pooled view (_avgpool_view); None leaves the call to ATen on the de-quantised tensor."""
+    try:
+        whole = x.dim() == 4 and _pair(args[0] if args else kwargs["kernel_size"]) == (x.shape[2], x.shape[3])
+    except (KeyError, TypeError):
+        return None                                     # not a valid call: let F.avg_pool2d raise its own error
+    return _avgpool_global(x, *args, **kwargs) if whole else _avgpool_view(x, args, kwargs)
+
+
+def _avgpool_view(x, args, kwargs):
+    """The lazy view F.avg_pool2d(x, *args, **kwargs): a NewConv2d reads it through pq_avgpool_requant_s8, anything
+    else gets ATen's pool of x de-quantised.  None (ATen) outside the kernel's limits, for arguments torch refuses
+    (ATen raises its own error) and for a source that is itself a lazy concatenation, nearest or pooled view."""
+    try:
+        window = pool_window(x.dim(), *args, **kwargs)
+    except TypeError:
+        return None                                     # not a valid call: let F.avg_pool2d raise its own error
+    if window is None or x._lazy_cat is not None or x._lazy_pool is not None:
+        return None
+    bit = x.exact_bit()
+    N, C, H, W = x.shape
+    is16 = x.s16_bit is not None
+    if bit is None or abs(bit) > _native.AVGPOOL_MAX_BIT or C % 8 or \
+            window[0] * window[1] * (32768 if is16 else 128) >= 1 << 24:
+        return None
+    try:
+        P, Q = _native.avgpool_out_size((H, W), window)
+    except RuntimeError:
+        return None                                     # arguments ATen refuses: it raises on the fallback path
+    if N * P * Q > _native.MAX_PIXELS:
+        return None
+    return QTensor((N, C, P, Q), x.device, lazy_pool=_LazyPool(x, window, tuple(args), dict(kwargs)))
+
+
+def _avgpool_global(x, kernel_size, stride=None, padding=0, ceil_mode=False, count_include_pad=True,
+                    divisor_override=None):
     """F.avg_pool2d over the WHOLE plane (ResNet's AvgPool2d before the classifier) straight from the most exact
     payload: fp32 [N][C][1][1], bit-identical to pooling the de-quantised tensor (pq_avgpool_global_nhwc_f32)."""
     k = _pair(kernel_size)
@@ -471,6 +571,9 @@ def conv_forward(mod, x):
         if x._lazy_cat is not None:
             if c is not None and x.channels <= c and x._lazy_cat.supported(mod.input_bit):
                 operand = x._lazy_cat.get(mod.input_bit, c, x.relu_pending and not x.nonneg)  # Concat + Quantity(ib)
+        elif x._lazy_pool is not None:
+            if c is not None and x._lazy_pool.supported(mod.input_bit, c):
+                operand = x._lazy_pool.get(mod.input_bit, c, x.relu_pending and not x.nonneg)  # AvgPool + Quantity(ib)
         elif c is not None and x.has_q8() and x.q8_bit == mod.input_bit and x.channels == c:
             operand = x.int8_payload()                           # Quantity(ib) is the identity here
     if operand is None:
@@ -529,8 +632,8 @@ class GraphedForward:
 
         fwd = GraphedForward(model, example_batch);  y = fwd(batch)      # y is overwritten by the next call
 
-    An output that is still a lazy QTensor (a model ending in an upsample or a convolution) is de-quantised inside the
-    capture, so every replay recomputes it."""
+    An output that is still a lazy QTensor (a model ending in an upsample, a pool or a convolution) is de-quantised
+    inside the capture, so every replay recomputes it."""
 
     def __init__(self, model, example, warmup=2):
         if not example.is_cuda:

@@ -531,6 +531,75 @@ concat_requant_scalar_kernel(const ConcatNearestParams np, size_t pixels, int8_t
     }
 }
 
+// pq_avgpool_requant_s8: a windowed nn.AvgPool2d of the de-quantised payload followed by the consumer's Quantity(q_bit),
+// written as the consumer's int8 NHWC operand [N][P][Q][c_out_pad].  As in the global overload, the fp32 window sum of
+// ATen is exact (kh*kw*max|x| < 2^24, checked by the caller), so with S the integer window sum
+//   out = clamp(rint(fl(fl(S) * 2^-bit / (float)d) * 2^q_bit), lo, 127),   one IEEE division by ATen's divisor d;
+// every product is by a power of two and stays a normal fp32 number for |bit|, |q_bit| <= 31, so it is exact.
+struct AvgPoolParams {
+    const void *x;
+    int8_t *out;
+    int H, W, C, P, Q, c_out_pad;
+    int kh, kw, sh, sw, ph, pw;
+    int count_include_pad, divisor_override;       // divisor_override 0: none
+    int relu_in;                                   // max(., 0) on load (a pending ReLU before the pool)
+    int lo;                                        // -128, or 0 for a ReLU after the pool
+    float scale, q_scale;                          // 2^-bit, 2^q_bit
+};
+
+// grid = (N * P output rows); as the max-pool, the threads of a block walk the (output column, 8-channel group) pairs of
+// one output row, channel group fastest, so a warp reads contiguous runs of each input row and nothing is divided per
+// element.  Groups at or beyond C / 8 write the zero channel padding.  A row may hold more than 2^31 such pairs (Q up
+// to 2^31 - 1 columns of c_out_pad / 8 groups), so the walk stops on the column, an unsigned that cannot wrap
+// (q < Q + 257 < 2^32), and the window ends, which may pass INT_MAX (W + pad), are taken in 64 bits.
+template <bool IS16>
+__global__ void __launch_bounds__(kPipeThreads)
+avgpool_global_kernel(const AvgPoolParams p)
+{
+    const unsigned int row = blockIdx.x, n = row / (unsigned int)p.P;
+    const int pp = (int)(row - n * (unsigned int)p.P);
+    const int G = p.c_out_pad >> 3, Gin = p.C >> 3;
+    // ATen's window: the divisor with count_include_pad takes the end before it is clipped to the image
+    const long long h0 = (long long)pp * p.sh - p.ph, h1 = min(h0 + p.kh, (long long)p.H + p.ph);
+    const int hs = (int)max(h0, 0LL), he = (int)min(h1, (long long)p.H);
+    const size_t img = (size_t)n * p.H;
+    int8_t *yrow = p.out + (size_t)row * p.Q * p.c_out_pad;
+    unsigned int q = threadIdx.x / (unsigned int)G;
+    int g = (int)(threadIdx.x - q * (unsigned int)G);
+    const int dq = kPipeThreads / G, dg = kPipeThreads - dq * G;   // advance of (q, g) per loop trip
+    while (q < (unsigned int)p.Q) {
+        uint2 o = make_uint2(0u, 0u);
+        if (g < Gin) {
+            const long long w0 = (long long)q * p.sw - p.pw, w1 = min(w0 + p.kw, (long long)p.W + p.pw);
+            const int ws = (int)max(w0, 0LL), we = (int)min(w1, (long long)p.W);
+            int acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+            // unrolled by two in each dimension, so the four loads of the usual 2 x 2 window are in flight together
+#pragma unroll 2
+            for (int iy = hs; iy < he; ++iy) {
+                const size_t e0 = ((img + iy) * p.W) * p.C + (size_t)g * 8;
+#pragma unroll 2
+                for (int ix = ws; ix < we; ++ix) {
+                    int v[8];
+                    add_load8<IS16>(p.x, e0 + (size_t)ix * p.C, v);
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) acc[j] += p.relu_in ? max(v[j], 0) : v[j];
+                }
+            }
+            const int d = p.divisor_override ? p.divisor_override
+                        : p.count_include_pad ? (int)((h1 - h0) * (w1 - w0)) : (he - hs) * (we - ws);
+            const float divisor = (float)d;
+            int r[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j)
+                r[j] = max(p.lo, __float2int_rn(__fmul_rn(__fdiv_rn(__fmul_rn((float)acc[j], p.scale), divisor), p.q_scale)));
+            o = make_uint2(pack4_sat_s8(r[0], r[1], r[2], r[3]), pack4_sat_s8(r[4], r[5], r[6], r[7]));
+        }
+        *reinterpret_cast<uint2 *>(yrow + (size_t)q * p.c_out_pad + (size_t)g * 8) = o;
+        q += dq; g += dg;
+        if (g >= G) { g -= G; ++q; }
+    }
+}
+
 __global__ void bias_fold_kernel(const int32_t *__restrict__ b, int n, int rs, int32_t *__restrict__ out)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -599,6 +668,48 @@ extern "C" int pq_avgpool_global_nhwc_f32(const void *x, int is16, int bit, int 
     const dim3 grid((unsigned)((C / 8 + pq::kPipeThreads - 1) / pq::kPipeThreads), (unsigned)N);
     if (is16) pq::avgpool_global_kernel<true><<<grid, pq::kPipeThreads, 0, (cudaStream_t)stream>>>(x, out, HW, C, relu, scale, divisor);
     else pq::avgpool_global_kernel<false><<<grid, pq::kPipeThreads, 0, (cudaStream_t)stream>>>(x, out, HW, C, relu, scale, divisor);
+    return (int)cudaGetLastError();
+}
+
+namespace {
+// ATen's pooling_output_shape: floor or ceil division, and in ceil mode the last window must start inside the image
+// or the left padding
+long long pool_out_size(long long in, long long k, long long s, long long pad, bool ceil_mode)
+{
+    const long long num = in + 2 * pad - k + (ceil_mode ? s - 1 : 0);
+    long long out = (num >= 0 ? num / s : -((-num + s - 1) / s)) + 1;
+    if (ceil_mode && (out - 1) * s >= in + pad) --out;
+    return out;
+}
+}  // namespace
+
+extern "C" int pq_avgpool_requant_s8(const void *x, int is16, int bit, int relu, int N, int H, int W, int C,
+                                     const pq_pool_desc *desc, int q_bit, int c_out_pad, int8_t *out,
+                                     pq_stream_t stream)
+{
+    if (!x || !out || !desc || (relu & ~3)) return PQ_EINVAL;
+    const pq_pool_desc d = *desc;
+    if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || c_out_pad < C) return PQ_EINVAL;
+    if (d.kh <= 0 || d.kw <= 0 || d.sh <= 0 || d.sw <= 0 || d.ph < 0 || d.pw < 0) return PQ_EINVAL;
+    if (2 * (long long)d.ph > d.kh || 2 * (long long)d.pw > d.kw) return PQ_EUNSUPPORTED;   // torch refuses it too
+    const long long P = pool_out_size(H, d.kh, d.sh, d.ph, d.ceil_mode != 0);
+    const long long Q = pool_out_size(W, d.kw, d.sw, d.pw, d.ceil_mode != 0);
+    if (P <= 0 || Q <= 0) return PQ_EINVAL;                               // torch: output size too small
+    // exactness of the fp32 window sum the reference performs (see the kernel): |sum| < 2^24 payload units, i.e.
+    // kh*kw < 2^24 / 32768 or 2^24 / 128 (kh*kw itself fits in 62 bits; times the unit it would not)
+    if ((long long)d.kh * d.kw >= (1LL << 24) / (is16 ? 32768 : 128)) return PQ_EUNSUPPORTED;
+    if ((C & 7) || (c_out_pad & 15) || (long long)N * P * Q > 0x7fffffffLL) return PQ_EUNSUPPORTED;
+    if (bit < -31 || bit > 31 || q_bit < -31 || q_bit > 31) return PQ_EUNSUPPORTED;
+    if (!al16(x) || !al16(out)) return PQ_EALIGN;
+    pq::AvgPoolParams p;
+    p.x = x; p.out = out; p.H = H; p.W = W; p.C = C; p.P = (int)P; p.Q = (int)Q; p.c_out_pad = c_out_pad;
+    p.kh = d.kh; p.kw = d.kw; p.sh = d.sh; p.sw = d.sw; p.ph = d.ph; p.pw = d.pw;
+    p.count_include_pad = d.count_include_pad != 0; p.divisor_override = d.divisor_override;
+    p.relu_in = relu & 1; p.lo = (relu & 2) ? 0 : -128;
+    p.scale = ldexpf(1.0f, -bit); p.q_scale = ldexpf(1.0f, q_bit);
+    const unsigned int grid = (unsigned int)(N * P);                      // <= N*P*Q <= 2^31 - 1
+    if (is16) pq::avgpool_global_kernel<true><<<grid, pq::kPipeThreads, 0, (cudaStream_t)stream>>>(p);
+    else pq::avgpool_global_kernel<false><<<grid, pq::kPipeThreads, 0, (cudaStream_t)stream>>>(p);
     return (int)cudaGetLastError();
 }
 

@@ -46,10 +46,12 @@ class BasicUnit(nn.Module):
 class BottleneckUnit(BasicUnit):
     """1x1 -> 3x3(stride) -> 1x1 residual unit (ResNet-50/101), stride on the 3x3 like
     quantity/model/resnet/ResNet.py:31-61.  With groups > 1 it is the ResNeXt unit: the 3x3 is a grouped convolution
-    of width * base_width / 64 * groups channels (torchvision's ResNeXt definition)."""
+    of width * base_width / 64 * groups channels (torchvision's ResNeXt definition).  With avg_down it is the ResNet-D
+    unit (He et al., "Bag of Tricks for Image Classification with Convolutional Neural Networks", 2019): a stride-2
+    shortcut averages 2 x 2 blocks first and then applies a stride-1 1x1 convolution, so no activation is skipped."""
     expansion = 4
 
-    def __init__(self, cin, width, stride, groups=1, base_width=64):
+    def __init__(self, cin, width, stride, groups=1, base_width=64, avg_down=False):
         nn.Module.__init__(self)
         cout = width * self.expansion
         mid = width * base_width // 64 * groups
@@ -58,16 +60,23 @@ class BottleneckUnit(BasicUnit):
             *_conv_bn(mid, mid, 3, stride, 1, groups), nn.ReLU(False),
             *_conv_bn(mid, cout, 1, 1, 0))
         self.shortcut = nn.Sequential()
-        if stride != 1 or cin != cout:
+        if avg_down and stride != 1:
+            self.shortcut = nn.Sequential(nn.AvgPool2d(stride, stride, ceil_mode=True, count_include_pad=False),
+                                          *_conv_bn(cin, cout, 1, 1, 0))
+        elif stride != 1 or cin != cout:
             self.shortcut = nn.Sequential(*_conv_bn(cin, cout, 1, stride, 0))
         self.Eltwise = Eltwise()
         self.relu = nn.ReLU(False)
 
 
 class FabuResNet(nn.Module):
-    def __init__(self, unit, depths, num_classes=1000, in_hw=224, **unit_kw):
+    def __init__(self, unit, depths, num_classes=1000, in_hw=224, deep_stem=False, **unit_kw):
         super().__init__()
-        self.stem = nn.Sequential(*_conv_bn(3, 64, 7, 2, 3), nn.ReLU(False))
+        if deep_stem:       # ResNet-C / -D: three 3x3 convolutions in place of the 7x7
+            self.stem = nn.Sequential(*_conv_bn(3, 32, 3, 2, 1), nn.ReLU(False), *_conv_bn(32, 32, 3, 1, 1),
+                                      nn.ReLU(False), *_conv_bn(32, 64, 3, 1, 1), nn.ReLU(False))
+        else:
+            self.stem = nn.Sequential(*_conv_bn(3, 64, 7, 2, 3), nn.ReLU(False))
         self.maxpool = nn.MaxPool2d(kernel_size=3, stride=2, padding=1)
         stages, cin = [], 64
         for i, (width, n) in enumerate(zip((64, 128, 256, 512), depths)):
@@ -93,6 +102,12 @@ def resnet18_fabu(num_classes=1000, in_hw=224):
 
 def resnet50_fabu(num_classes=1000, in_hw=224):
     return FabuResNet(BottleneckUnit, (3, 4, 6, 3), num_classes, in_hw)
+
+
+def resnet50d_fabu(num_classes=1000, in_hw=224):
+    """ResNet-50-D: the deep stem and avg-down shortcuts (AvgPool2d(2, 2, ceil_mode=True, count_include_pad=False)
+    -> 1x1 conv -> BN) on every stride-2 unit."""
+    return FabuResNet(BottleneckUnit, (3, 4, 6, 3), num_classes, in_hw, deep_stem=True, avg_down=True)
 
 
 def resnext50_32x4d_fabu(num_classes=1000, in_hw=224):

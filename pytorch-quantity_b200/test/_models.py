@@ -18,6 +18,8 @@ MODELS = {
                  (3, 224, 224)),
     "resnet50": (lambda: __import__("model.resnet.resnet_fabu", fromlist=["resnet50_fabu"]).resnet50_fabu(),
                  (3, 224, 224)),
+    "resnet50d": (lambda: __import__("model.resnet.resnet_fabu", fromlist=["resnet50d_fabu"]).resnet50d_fabu(),
+                  (3, 224, 224)),
     "resnext50_32x4d": (lambda: __import__("model.resnet.resnet_fabu",
                                            fromlist=["resnext50_32x4d_fabu"]).resnext50_32x4d_fabu(), (3, 224, 224)),
     "mobilenetv2": (lambda: __import__("model.mobilenet.mobilenetv2_fabu",
